@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py — Snake env-steps/sec on B200 (BASELINE.json metric), one JSON line on stdout.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs E]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--envs E] [--dump-outputs DIR]
 
 Workload (config.workload): BASELINE config 3 — E = 1,048,576 batched envs PER GPU (weak scaling: envs are
 independent, each rank owns its own shard, no collective on the step path), every step = ONE fused kernel
@@ -28,10 +28,12 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark leaves the tree as it found it (it may be read-only)
 
 BYTES_PER_STEP_CONFIG3 = 876   # SURVEY.md §8(d): 50 state + 1 action + 4 reward + 1 done + 3 mask + 800 obs + 12 q + 4 u + 1 ridx
 BYTES_PER_STEP_CONFIG2 = 859
 REF_SAMPLE_ENVS = 32768        # env count of the CPU arm's bounded sample (independent of the host's thread count)
+DUMP_MAX_ENVS = 65536          # --dump-outputs: 824 bytes of float32 per env
 METRIC = "snake_env_steps_per_sec"
 UNIT = "env-steps/s"
 
@@ -212,18 +214,21 @@ def run_ours(args):
         env.step_fused(q=qs[j], eps=eps, u=us[j], ridx=rs[j], out=out)
 
     # clocks are sampled from BEFORE the warm-up to the end of the timed region (a 20-step region lasts 3 ms, one
-    # nvidia-smi period is 20 ms): the warm-up is stretched with extra untimed steps until the sampler has delivered
+    # nvidia-smi period is 20 ms): the warm-up is preceded by extra untimed steps until the sampler has delivered.
+    # Their number depends on how soon it delivers, so the envs restart from the initial state after them: with the same
+    # arguments, every run's timed steps compute the same outputs from the same inputs.
     sampler = ClockSampler(local)
     if rank == 0:
         sampler.start()
-    for i in range(W):
-        one_step(i)
     extra, t_w = 0, time.perf_counter()
     while rank == 0 and len(sampler.rows) < 8 and time.perf_counter() - t_w < 1.5 and sampler.proc is not None:
         for i in range(50):
-            one_step(W + extra + i)
+            one_step(extra + i)
         torch.cuda.synchronize()
         extra += 50
+    env.reset()
+    for i in range(W):
+        one_step(i)
     barrier()
     use_graph = E < 400_000       # a shard this small takes < 60 us per step: launch through a CUDA graph of R steps
     if not use_graph:
@@ -265,6 +270,8 @@ def run_ours(args):
     total_ms = max_over_ranks(total_ms)
     kern_ms = max_over_ranks(kern_ms)
     value = world * E * K / (total_ms * 1e-3)
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     n_err = env.count_errors()
 
     # ---- the same fused step with the other observation formats (SURVEY 8(d): report all three byte counts)
@@ -475,6 +482,21 @@ def run_ours(args):
     if world > 1:
         dist.destroy_process_group()
     return 0
+
+
+def dump_outputs(path, out, max_envs=DUMP_MAX_ENVS):
+    """Writes what the last timed step returned to its caller as float32 `path`/<name>.npy: act_idx (E,), reward (E,),
+    done (E,), mask (E, 3), obs (E, 2, 10, 10).  Above max_envs envs only a fixed seeded sample of envs is written, the
+    same for every run with the same --envs; env_index.npy (float64) lists the envs written."""
+    import numpy as np
+    import torch
+    E = out["reward"].numel()
+    idx = np.arange(E) if E <= max_envs else np.sort(np.random.default_rng(0).choice(E, max_envs, replace=False))
+    sel = torch.from_numpy(idx).to(out["reward"].device)
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "env_index.npy"), idx.astype(np.float64))
+    for name in ("act_idx", "reward", "done", "mask", "obs"):
+        np.save(os.path.join(path, name + ".npy"), out[name].index_select(0, sel).float().cpu().numpy())
 
 
 def bench_config4(S, dev, local, n=65536, steps=20):
@@ -777,6 +799,9 @@ def main():
     ap.add_argument("--gram-rows", type=int, default=6250, help="rows of J per GPU in the row-sharded Gram (config 5b: 6,250)")
     ap.add_argument("--skip-config4", action="store_true")
     ap.add_argument("--skip-variants", action="store_true", help="skip the int8-observation / no-observation timings")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32, at most %d envs: "
+                         "about 54 MB)" % DUMP_MAX_ENVS)
     args = ap.parse_args()
     if args.impl == "reference":
         return run_reference(args)

