@@ -166,6 +166,17 @@ SNK_API int snk_rollout_fused(snk_handle h, const uint8_t *act_TxN, int64_t T, i
 SNK_API int snk_debug_rollout_timing(long long *device_buf);
 SNK_API int snk_host_alloc(void **p, size_t bytes);   /* pinned host memory */
 SNK_API int snk_host_free(void *p);
+/* device memory for the outputs of the fused step.  With SNK_ALLOC_COMPRESSIBLE, on a device that supports it
+ * (snk_compression_supported), the memory is created with generic L2 compression (cuMemCreate, CU_MEM_ALLOCATION_COMP_GENERIC,
+ * size rounded up to the allocation granularity, 2 MB on B200): lossless, every kernel and copy sees the same bytes, but lines
+ * of few distinct words - the Float32 observations - cross the DRAM bus compressed, so k_step writing into it is faster.
+ * Otherwise, or when the driver hands out memory that is not compressible, it is cudaMalloc memory.  *compressible (may be
+ * NULL) reports which one it is.  snk_device_free synchronises the device before it unmaps compressible memory: not for use
+ * inside a CUDA graph capture. */
+#define SNK_ALLOC_COMPRESSIBLE 1u
+SNK_API int snk_device_alloc(void **p, size_t bytes, int device, uint32_t flags, int *compressible);
+SNK_API int snk_device_free(void *p);
+SNK_API int snk_compression_supported(int device, int *yes);
 
 /* ---- assemble_state! / assemble_states_vector  utils.jl:135-149 --------------------------- */
 /* current two-frame state (board_{t-1}, board_t) of every env, in obs_fmt */

@@ -12,6 +12,7 @@ entry point raises.
 """
 import ctypes as C
 import os
+import warnings
 
 import torch
 
@@ -94,6 +95,8 @@ def lib():
         "snk_step_fused_host": [vp, vp, f32, vp, vp, vp, vp, vp, vp, i32, vp, vp, vp],
         "snk_rollout_fused": [vp, vp, i64, i32, vp, vp, vp, i32, vp, vp, vp],
         "snk_host_alloc": [C.POINTER(vp), C.c_size_t], "snk_host_free": [vp],
+        "snk_device_alloc": [C.POINTER(vp), C.c_size_t, i32, u32, C.POINTER(i32)], "snk_device_free": [vp],
+        "snk_compression_supported": [i32, C.POINTER(i32)],
         "snk_state": [vp, vp, i32], "snk_losing_mask": [vp, vp],
         "snk_state_host": [vp, vp, i32], "snk_losing_mask_host": [vp, vp], "snk_available_actions_host": [vp, vp],
         "snk_patch_reset_obs": [vp, vp, vp, i32],
@@ -170,6 +173,67 @@ def _ptr(t, dtype=None, numel=None, device=None):
     if device is not None and t.device != device:
         raise ValueError("tensor on %s, env on %s" % (t.device, device))
     return C.c_void_p(t.data_ptr())
+
+
+ALLOC_COMPRESSIBLE = 1
+_compression = {}            # device index -> snk_compression_supported
+_compressible = set()        # base pointers of the live compressible allocations
+_deferred = []               # pointers whose free had to wait: freed by the next allocation or free outside a graph capture
+
+
+def _free_deferred():
+    while _deferred and not torch.cuda.is_current_stream_capturing():
+        p = _deferred[-1]
+        if lib().snk_device_free(C.c_void_p(p)) != 0:
+            warnings.warn("snk_device_free: %s" % lib().snk_last_error().decode())
+            return
+        _deferred.pop()
+        _compressible.discard(p)
+
+
+class _DeviceBuffer:
+    """Owns one snk_device_alloc allocation; torch.as_tensor() views it through __cuda_array_interface__ and keeps this
+    object alive as long as any tensor sharing the memory lives.  The memory is freed with it."""
+
+    def __init__(self, nbytes, device):
+        p, comp = C.c_void_p(), C.c_int(0)
+        _check(lib().snk_device_alloc(C.byref(p), nbytes, device, ALLOC_COMPRESSIBLE, C.byref(comp)))
+        self.ptr = p.value
+        if comp.value:
+            _compressible.add(self.ptr)
+        self.__cuda_array_interface__ = {"shape": (nbytes,), "typestr": "|u1", "data": (self.ptr, False), "version": 3,
+                                         "strides": None, "stream": None}
+
+    def __del__(self):
+        # freeing synchronises the device, which a CUDA graph capture does not allow: a buffer that dies while one runs on
+        # this thread's current stream is freed later; a free that fails stays queued with a warning
+        try:
+            _deferred.append(self.ptr)
+            _free_deferred()
+        except Exception:              # interpreter shutdown: module globals may already be gone
+            pass
+
+
+def compressible_empty(shape, dtype, device):
+    """torch.empty(shape, dtype, device) in device memory with generic L2 compression (snk_device_alloc): lossless, but
+    data of few distinct words crosses the DRAM bus compressed.  Plain torch.empty where the device has no compression."""
+    device = torch.device(device)
+    idx = device.index if device.index is not None else torch.cuda.current_device()
+    if idx not in _compression:
+        yes = C.c_int(0)
+        _check(lib().snk_compression_supported(idx, C.byref(yes)))
+        _compression[idx] = bool(yes.value)
+    if not _compression[idx]:
+        return torch.empty(shape, dtype=dtype, device=device)
+    _free_deferred()
+    n = torch.Size(shape).numel() * torch.empty((), dtype=dtype).element_size()
+    raw = torch.as_tensor(_DeviceBuffer(max(n, 1), idx), device=torch.device("cuda", idx))
+    return raw[:n].view(dtype).view(shape)
+
+
+def is_compressible(t):
+    """True when tensor t lives in compressible device memory (compressible_empty / alloc_outputs)."""
+    return t.untyped_storage().data_ptr() in _compressible
 
 
 def default_food_list():
@@ -254,19 +318,24 @@ class SnakeGame:
         return r, d
 
     # -- the fused rollout step -----------------------------------------------------------------
-    def alloc_outputs(self, obs="f32", mask=True, ep_stats=False, act=False):
-        out = {"reward": self._new((self.n,), torch.float32), "done": self._new((self.n,), torch.uint8)}
+    def alloc_outputs(self, obs="f32", mask=True, ep_stats=False, act=False, compressible=True):
+        """Output buffers of step_fused, to be reused step after step.  compressible: in device memory with generic L2
+        compression (compressible_empty) - the same values, but the Float32 step writes fewer DRAM bytes and runs faster.
+        Allocate them outside CUDA graph captures: allocating and freeing such memory synchronises the device.  (A buffer
+        that is garbage-collected during a capture on the current stream is freed after it.)"""
+        new = (lambda shape, dt: compressible_empty(shape, dt, self.device)) if compressible else self._new
+        out = {"reward": new((self.n,), torch.float32), "done": new((self.n,), torch.uint8)}
         if obs:
             _, dt, per = _OBS[obs]
-            out["obs"] = self._new((self.n, 2, 10, 10) if per == 200 else (self.n, per), dt)
+            out["obs"] = new((self.n, 2, 10, 10) if per == 200 else (self.n, per), dt)
             out["obs_fmt"] = obs
         if mask:
-            out["mask"] = self._new((self.n, 3), torch.uint8)
+            out["mask"] = new((self.n, 3), torch.uint8)
         if ep_stats:
-            out["ep_return"] = self._new((self.n,), torch.float32)
-            out["ep_score"] = self._new((self.n,), torch.int32)
+            out["ep_return"] = new((self.n,), torch.float32)
+            out["ep_score"] = new((self.n,), torch.int32)
         if act:
-            out["act_idx"] = self._new((self.n,), torch.uint8)
+            out["act_idx"] = new((self.n,), torch.uint8)
         return out
 
     def step_fused(self, act_idx=None, q=None, eps=0.0, u=None, ridx=None, out=None, obs="f32", replay=None):
@@ -276,8 +345,8 @@ class SnakeGame:
         (reward, done, obs, mask, ...); pass a dict from alloc_outputs() to reuse buffers.
         replay: a ReplayBuffer — every env's transition is store!d (utils.jl:267-277) by the same kernel.
         """
-        if out is None:
-            out = self.alloc_outputs(obs=obs, act=q is not None)
+        if out is None:            # buffers for one call: torch's caching allocator hands them out without a driver call
+            out = self.alloc_outputs(obs=obs, act=q is not None, compressible=False)
         fmt = _OBS[out["obs_fmt"]][0] if out.get("obs") is not None else OBS_NONE
         dev = self.device
         if q is not None:

@@ -25,11 +25,16 @@
 #include <string.h>
 
 #include <new>
+#include <mutex>
+#include <unordered_map>
+
+#include <cuda.h>
 
 #include "common.h"
 
 // how phase B stores the observation: 0 = st.global.cs (streaming), 1 = plain st.global (default), 2 = st.global.wt.
-// Measured at 2^20 envs on B200: 166.5 us with .cs, 162.8 us with plain or .wt stores (87.4 % of the HBM copy peak).
+// Measured at 2^20 envs on B200: 166.5 us with .cs, 162.8 us with plain or .wt stores (87.4 % of the HBM copy peak); into
+// compressible outputs (snk_device_alloc) 118.0 / 117.8 / 117.8 us.
 #ifndef SNK_OBS_STORE_MODE
 #define SNK_OBS_STORE_MODE 1
 #endif
@@ -55,13 +60,19 @@ int fail(int code, const char *fmt, ...) {
 
 // ------------------------------------------------------------------------------------------------
 #ifndef SNK_TPB
-#define SNK_TPB 256            // measured on B200 at 2^20 envs: 256 threads ~1-2 % faster than 128, 64 and 512 slower
+#define SNK_TPB 256            // measured on B200 at 2^20 envs into plain memory: 256 threads ~1-2 % faster than 128, 64 and 512 slower
+                               // (Float32 into compressible outputs at unroll 2: 128 threads 114.7 us, 256 117.8; not adopted, the
+                               // small formats' occupancy also depends on it and they were not re-measured)
 #endif
 #ifndef SNK_MINB
 #define SNK_MINB 1
 #endif
 #ifndef SNK_UNROLL
-#define SNK_UNROLL 2
+#define SNK_UNROLL 4           // Float32 phase B into compressible outputs, 2^20 envs on B200: 1 / 2 / 4 -> 123.9 / 117.8 / 115.1 us;
+                               // into plain memory 151.1 / 150.4 / 150.2 us.  Against unroll 2 (bench.py, with compressible outputs):
+                               // config 2 at 4,096 envs 4.96 -> 4.98 G env-steps/s, the host-buffer Float32 step (e2e
+                               // full_f32_obs_variant) 6.81 -> 6.82e7; the rollout kernels pass their own unroll (5); the
+                               // stand-alone state kernel (snk_state) was not timed
 #endif
 constexpr int PHASE_B_UNROLL = SNK_UNROLL;
 constexpr int TPB = SNK_TPB;      // envs (= threads) per CTA (tuning knobs: -DSNK_TPB / -DSNK_MINB / -DSNK_UNROLL)
@@ -1190,6 +1201,116 @@ static cudaError_t ensure(T **p, size_t bytes) {
 #endif
 static long long *g_rollout_prof = nullptr;
 
+// ---- device memory with generic L2 compression (snk_device_alloc) ---------------------------------------------------
+// Blackwell's L2 compresses the lines of an allocation made with CU_MEM_ALLOCATION_COMP_GENERIC when it writes them back to
+// DRAM.  It is lossless: kernels and copies see the same bytes.  k_step's Float32 observations are mostly zeros and a few
+// repeated words; written into such memory, the step moves fewer bytes over the DRAM bus than it stores (DESIGN §3).
+// The driver API comes from cudaGetDriverEntryPoint: the library does not link libcuda.
+struct Vmm {
+    CUresult (*device_get)(CUdevice *, int);
+    CUresult (*get_attribute)(int *, CUdevice_attribute, CUdevice);
+    CUresult (*granularity)(size_t *, const CUmemAllocationProp *, CUmemAllocationGranularity_flags);
+    CUresult (*create)(CUmemGenericAllocationHandle *, size_t, const CUmemAllocationProp *, unsigned long long);
+    CUresult (*properties)(CUmemAllocationProp *, CUmemGenericAllocationHandle);
+    CUresult (*address_reserve)(CUdeviceptr *, size_t, size_t, CUdeviceptr, unsigned long long);
+    CUresult (*map)(CUdeviceptr, size_t, size_t, CUmemGenericAllocationHandle, unsigned long long);
+    CUresult (*set_access)(CUdeviceptr, size_t, const CUmemAccessDesc *, size_t);
+    CUresult (*unmap)(CUdeviceptr, size_t);
+    CUresult (*address_free)(CUdeviceptr, size_t);
+    CUresult (*release)(CUmemGenericAllocationHandle);
+};
+static int vmm_api(const Vmm **out) {
+    static Vmm api;
+    static int state = 0;                       // 0 = not loaded yet, 1 = loaded, -1 = an entry point is missing
+    static std::mutex mu;
+    std::lock_guard<std::mutex> lk(mu);
+    if (state == 0) {
+        struct { const char *name; void **slot; } want[] = {
+            {"cuDeviceGet", (void **)&api.device_get}, {"cuDeviceGetAttribute", (void **)&api.get_attribute},
+            {"cuMemGetAllocationGranularity", (void **)&api.granularity}, {"cuMemCreate", (void **)&api.create},
+            {"cuMemGetAllocationPropertiesFromHandle", (void **)&api.properties},
+            {"cuMemAddressReserve", (void **)&api.address_reserve}, {"cuMemMap", (void **)&api.map},
+            {"cuMemSetAccess", (void **)&api.set_access}, {"cuMemUnmap", (void **)&api.unmap},
+            {"cuMemAddressFree", (void **)&api.address_free}, {"cuMemRelease", (void **)&api.release}};
+        state = 1;
+        for (auto &w : want) {
+            cudaDriverEntryPointQueryResult q;
+            if (cudaGetDriverEntryPoint(w.name, w.slot, cudaEnableDefault, &q) != cudaSuccess || q != cudaDriverEntryPointSuccess ||
+                *w.slot == nullptr) {
+                cudaGetLastError();
+                state = -1;
+                return fail(SNK_ERR_CUDA, "driver entry point %s not available", w.name);
+            }
+        }
+    }
+    if (state < 0) return fail(SNK_ERR_CUDA, "driver virtual-memory entry points not available");
+    *out = &api;
+    return SNK_OK;
+}
+static int vmm_compression_supported(const Vmm &v, int device, int *yes) {
+    CUdevice d;
+    int vmm = 0, comp = 0;
+    CUresult r = v.device_get(&d, device);
+    if (r == CUDA_SUCCESS) r = v.get_attribute(&vmm, CU_DEVICE_ATTRIBUTE_VIRTUAL_MEMORY_MANAGEMENT_SUPPORTED, d);
+    if (r == CUDA_SUCCESS) r = v.get_attribute(&comp, CU_DEVICE_ATTRIBUTE_GENERIC_COMPRESSION_SUPPORTED, d);
+    if (r != CUDA_SUCCESS) return fail(SNK_ERR_CUDA, "cuDeviceGetAttribute: CUresult %d", (int)r);
+    *yes = vmm && comp;
+    return SNK_OK;
+}
+// one live snk_device_alloc allocation; vmm = false: a cudaMalloc block
+struct DevAlloc {
+    CUmemGenericAllocationHandle handle;
+    size_t size;                 // mapped (= reserved) bytes
+    int device;
+    bool vmm;
+};
+static std::mutex g_dev_allocs_mu;
+static std::unordered_map<void *, DevAlloc> g_dev_allocs;
+
+// *p stays NULL when the driver hands out memory that is not compressible: the caller then falls back to cudaMalloc
+static int vmm_alloc_compressible(const Vmm &v, int device, size_t bytes, void **p, DevAlloc *a) {
+    CUmemAllocationProp prop = {};
+    prop.type = CU_MEM_ALLOCATION_TYPE_PINNED;
+    prop.location.type = CU_MEM_LOCATION_TYPE_DEVICE;
+    prop.location.id = device;
+    prop.allocFlags.compressionType = CU_MEM_ALLOCATION_COMP_GENERIC;
+    size_t g = 0;
+    CUresult r = v.granularity(&g, &prop, CU_MEM_ALLOC_GRANULARITY_MINIMUM);
+    if (r != CUDA_SUCCESS) return fail(SNK_ERR_CUDA, "cuMemGetAllocationGranularity: CUresult %d", (int)r);
+    const size_t size = (bytes + g - 1) / g * g;
+    CUmemGenericAllocationHandle h;
+    r = v.create(&h, size, &prop, 0);
+    if (r != CUDA_SUCCESS) return fail(SNK_ERR_CUDA, "cuMemCreate(%zu bytes, compressible): CUresult %d", size, (int)r);
+    CUmemAllocationProp got = {};
+    r = v.properties(&got, h);
+    if (r != CUDA_SUCCESS || got.allocFlags.compressionType != CU_MEM_ALLOCATION_COMP_GENERIC) {   // the hint was not honoured
+        v.release(h);
+        return r == CUDA_SUCCESS ? SNK_OK : fail(SNK_ERR_CUDA, "cuMemGetAllocationPropertiesFromHandle: CUresult %d", (int)r);
+    }
+    CUdeviceptr d = 0;
+    r = v.address_reserve(&d, size, 0, 0, 0);
+    if (r != CUDA_SUCCESS) {
+        v.release(h);
+        return fail(SNK_ERR_CUDA, "cuMemAddressReserve: CUresult %d", (int)r);
+    }
+    r = v.map(d, size, 0, h, 0);
+    CUmemAccessDesc acc = {};
+    acc.location = prop.location;
+    acc.flags = CU_MEM_ACCESS_FLAGS_PROT_READWRITE;
+    if (r == CUDA_SUCCESS) {
+        r = v.set_access(d, size, &acc, 1);
+        if (r != CUDA_SUCCESS) v.unmap(d, size);
+    }
+    if (r != CUDA_SUCCESS) {
+        v.address_free(d, size);
+        v.release(h);
+        return fail(SNK_ERR_CUDA, "cuMemMap / cuMemSetAccess: CUresult %d", (int)r);
+    }
+    *p = (void *)d;
+    *a = {h, size, device, true};
+    return SNK_OK;
+}
+
 extern "C" {
 
 // profiling aid: device buffer of 8 int64 receiving cycle counts of CTA 0 of the small-batch rollout kernel
@@ -1455,6 +1576,78 @@ int snk_host_alloc(void **p, size_t bytes) {
 }
 int snk_host_free(void *p) {
     if (p) SNK_CUDA(cudaFreeHost(p));
+    return SNK_OK;
+}
+
+int snk_compression_supported(int device, int *yes) {
+    SNK_REQUIRE(yes != nullptr, "null out");
+    *yes = 0;
+    int ndev = 0;
+    SNK_CUDA(cudaGetDeviceCount(&ndev));
+    SNK_REQUIRE(device >= 0 && device < ndev, "device index out of range");
+    DeviceGuard guard(device);
+    const Vmm *v = nullptr;
+    if (vmm_api(&v) != SNK_OK) return SNK_OK;             // a driver without the virtual-memory entry points: no compression
+    return vmm_compression_supported(*v, device, yes);
+}
+
+int snk_device_alloc(void **p, size_t bytes, int device, uint32_t flags, int *compressible) {
+    SNK_REQUIRE(p != nullptr && bytes > 0, "bad argument");
+    SNK_REQUIRE((flags & ~SNK_ALLOC_COMPRESSIBLE) == 0u, "unknown flag");
+    *p = nullptr;
+    if (compressible != nullptr) *compressible = 0;
+    int ndev = 0;
+    SNK_CUDA(cudaGetDeviceCount(&ndev));
+    SNK_REQUIRE(device >= 0 && device < ndev, "device index out of range");
+    DeviceGuard guard(device);
+    DevAlloc a = {0, bytes, device, false};
+    if (flags & SNK_ALLOC_COMPRESSIBLE) {
+        int yes = 0;
+        int rc = snk_compression_supported(device, &yes);
+        if (rc != SNK_OK) return rc;
+        if (yes) {
+            const Vmm *v = nullptr;
+            rc = vmm_api(&v);
+            if (rc == SNK_OK) rc = vmm_alloc_compressible(*v, device, bytes, p, &a);
+            if (rc != SNK_OK) return rc;
+        }
+    }
+    if (*p == nullptr) SNK_CUDA(cudaMalloc(p, bytes));     // not requested, not supported, or the driver gave plain memory
+    {
+        std::lock_guard<std::mutex> lk(g_dev_allocs_mu);
+        g_dev_allocs[*p] = a;
+    }
+    if (compressible != nullptr) *compressible = a.vmm ? 1 : 0;
+    return SNK_OK;
+}
+
+int snk_device_free(void *p) {
+    if (p == nullptr) return SNK_OK;
+    DevAlloc a;
+    {
+        std::lock_guard<std::mutex> lk(g_dev_allocs_mu);
+        auto it = g_dev_allocs.find(p);
+        SNK_REQUIRE(it != g_dev_allocs.end(), "pointer was not returned by snk_device_alloc (or was freed already)");
+        a = it->second;
+    }
+    // the entry is dropped only once the memory is given back: after a failed call (a device synchronise refused during a
+    // stream capture, a sticky error) the pointer stays registered and the call can be repeated
+    DeviceGuard guard(a.device);
+    if (!a.vmm) {
+        SNK_CUDA(cudaFree(p));
+    } else {
+        SNK_CUDA(cudaDeviceSynchronize());                // unmapping does not wait for kernels that may still write the range
+        const Vmm *v = nullptr;
+        int rc = vmm_api(&v);
+        if (rc != SNK_OK) return rc;
+        const CUdeviceptr d = (CUdeviceptr)p;
+        CUresult r = v->unmap(d, a.size);
+        if (r == CUDA_SUCCESS) r = v->address_free(d, a.size);
+        if (r == CUDA_SUCCESS) r = v->release(a.handle);
+        if (r != CUDA_SUCCESS) return fail(SNK_ERR_CUDA, "snk_device_free: CUresult %d", (int)r);
+    }
+    std::lock_guard<std::mutex> lk(g_dev_allocs_mu);
+    g_dev_allocs.erase(p);
     return SNK_OK;
 }
 

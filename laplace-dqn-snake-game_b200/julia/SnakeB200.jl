@@ -17,7 +17,7 @@ export BatchedSnakeGame, available_actions, step!, step_fused!, virtual_step, as
        GramShard, export_handle, connect!, run!, planes,
        step_device!, step_abs_device!, step_fused_device!, rollout_device!, state_device!, losing_mask_device!,
        lost_device!, steps_device!, error_flags_device!, count_errors, seed!, set_stream!, num_envs, library_version,
-       default_food_list
+       default_food_list, device_alloc, device_free, compression_supported
 
 const lib = get(ENV, "SNAKE_B200_LIB", joinpath(@__DIR__, "..", "libsnake_b200.so"))
 
@@ -451,6 +451,22 @@ function planes(g::GramShard)
     hi = Ref{Ptr{Cvoid}}(C_NULL); lo = Ref{Ptr{Cvoid}}(C_NULL); pitch = Ref{Int64}(0)
     check(ccall((:snk_gram_shard_planes, lib), Cint, (Ptr{Cvoid}, Ref{Ptr{Cvoid}}, Ref{Ptr{Cvoid}}, Ref{Int64}), g.handle, hi, lo, pitch))
     return hi[], lo[], Int(pitch[])
+end
+
+"""`bytes` of device memory on `device` for the outputs of the fused step; with `compressible`, memory with generic L2
+compression where the device supports it (lossless; the Float32 step writes fewer DRAM bytes).  Returns (pointer, compressible)."""
+function device_alloc(bytes::Integer, device::Integer = 0; compressible::Bool = true)
+    p = Ref{Ptr{Cvoid}}(C_NULL); got = Ref{Cint}(0)
+    check(ccall((:snk_device_alloc, lib), Cint, (Ref{Ptr{Cvoid}}, Csize_t, Cint, UInt32, Ref{Cint}),
+                p, bytes, device, compressible ? UInt32(1) : UInt32(0), got))
+    return p[], got[] != 0
+end
+"""frees memory from `device_alloc` (synchronises the device first)"""
+device_free(p::Ptr{Cvoid}) = check(ccall((:snk_device_free, lib), Cint, (Ptr{Cvoid},), p))
+function compression_supported(device::Integer = 0)
+    yes = Ref{Cint}(0)
+    check(ccall((:snk_compression_supported, lib), Cint, (Cint, Ref{Cint}), device, yes))
+    return yes[] != 0
 end
 
 end # module
