@@ -29,6 +29,33 @@ _OBS = {
 }
 
 
+def _obs_shape(fmt, lead):
+    """shape of the observations in format fmt for the leading dims `lead`: (*lead, 2, 10, 10) when one element is one cell"""
+    per = _OBS[fmt][2]
+    return (*lead, 2, 10, 10) if per == 200 else (*lead, per)
+
+
+def _fmt_code(out):
+    """obs_fmt code of an output dict: OBS_NONE when it holds no 'obs'"""
+    return _OBS[out["obs_fmt"]][0] if out.get("obs") is not None else OBS_NONE
+
+
+def _outputs(new, lead, obs, mask, ep_stats, act=False):
+    """the output dict of a step (lead = (N,)) or a rollout (lead = (T, N)); new(shape, dtype) allocates"""
+    out = {"reward": new(lead, torch.float32), "done": new(lead, torch.uint8)}
+    if obs:
+        out["obs"] = new(_obs_shape(obs, lead), _OBS[obs][1])
+        out["obs_fmt"] = obs
+    if mask:
+        out["mask"] = new((*lead, 3), torch.uint8)
+    if ep_stats:
+        out["ep_return"] = new(lead, torch.float32)
+        out["ep_score"] = new(lead, torch.int32)
+    if act:
+        out["act_idx"] = new(lead, torch.uint8)
+    return out
+
+
 def unpack_bits(rec):
     """Decodes SNK_OBS_BITS records (include/snake_b200.h): rec (N, 24) uint8, CPU or CUDA ->
     dict(state (N,2,10,10) int8 [= Julia (10,10,2,N): state[n, f, c, r]], reward (N,) f32, done (N,) u8, mask (N,3) u8 =
@@ -324,19 +351,7 @@ class SnakeGame:
         Allocate them outside CUDA graph captures: allocating and freeing such memory synchronises the device.  (A buffer
         that is garbage-collected during a capture on the current stream is freed after it.)"""
         new = (lambda shape, dt: compressible_empty(shape, dt, self.device)) if compressible else self._new
-        out = {"reward": new((self.n,), torch.float32), "done": new((self.n,), torch.uint8)}
-        if obs:
-            _, dt, per = _OBS[obs]
-            out["obs"] = new((self.n, 2, 10, 10) if per == 200 else (self.n, per), dt)
-            out["obs_fmt"] = obs
-        if mask:
-            out["mask"] = new((self.n, 3), torch.uint8)
-        if ep_stats:
-            out["ep_return"] = new((self.n,), torch.float32)
-            out["ep_score"] = new((self.n,), torch.int32)
-        if act:
-            out["act_idx"] = new((self.n,), torch.uint8)
-        return out
+        return _outputs(new, (self.n,), obs, mask, ep_stats, act)
 
     def step_fused(self, act_idx=None, q=None, eps=0.0, u=None, ridx=None, out=None, obs="f32", replay=None):
         """One kernel: [epsilon_greedy] + step! + virtual_step + next_state (+ Float32 cast).
@@ -347,7 +362,6 @@ class SnakeGame:
         """
         if out is None:            # buffers for one call: torch's caching allocator hands them out without a driver call
             out = self.alloc_outputs(obs=obs, act=q is not None, compressible=False)
-        fmt = _OBS[out["obs_fmt"]][0] if out.get("obs") is not None else OBS_NONE
         dev = self.device
         if q is not None:
             act_p = _ptr(out.get("act_idx"), torch.uint8, self.n, dev)
@@ -357,7 +371,7 @@ class SnakeGame:
             act_p = _ptr(act_idx, torch.uint8, self.n, dev)
         args = (_ptr(q, torch.float32, 3 * self.n, dev) if q is not None else None, float(eps),
                 _ptr(u, torch.float32, self.n, dev), _ptr(ridx, torch.uint8, self.n, dev), act_p,
-                _ptr(out.get("reward")), _ptr(out.get("done")), _ptr(out.get("obs")), fmt, _ptr(out.get("mask")),
+                _ptr(out.get("reward")), _ptr(out.get("done")), _ptr(out.get("obs")), _fmt_code(out), _ptr(out.get("mask")),
                 _ptr(out.get("ep_return")), _ptr(out.get("ep_score")))
         if replay is None:
             _check(lib().snk_step_fused(self._h, *args))
@@ -371,19 +385,9 @@ class SnakeGame:
         T = actions.shape[0]
         dev = self.device
         if out is None:
-            out = {"reward": self._new((T, self.n), torch.float32), "done": self._new((T, self.n), torch.uint8)}
-            if obs:
-                _, dt, per = _OBS[obs]
-                out["obs"] = self._new((T, self.n, 2, 10, 10) if per == 200 else (T, self.n, per), dt)
-                out["obs_fmt"] = obs
-            if mask:
-                out["mask"] = self._new((T, self.n, 3), torch.uint8)
-            if ep_stats:
-                out["ep_return"] = self._new((T, self.n), torch.float32)
-                out["ep_score"] = self._new((T, self.n), torch.int32)
-        fmt = _OBS[out["obs_fmt"]][0] if out.get("obs") is not None else OBS_NONE
+            out = _outputs(self._new, (T, self.n), obs, mask, ep_stats)
         _check(lib().snk_rollout_fused(self._h, _ptr(actions, torch.uint8, T * self.n, dev), T, int(is_abs),
-                                       _ptr(out.get("reward")), _ptr(out.get("done")), _ptr(out.get("obs")), fmt,
+                                       _ptr(out.get("reward")), _ptr(out.get("done")), _ptr(out.get("obs")), _fmt_code(out),
                                        _ptr(out.get("mask")), _ptr(out.get("ep_return")), _ptr(out.get("ep_score"))))
         return out
 
@@ -391,10 +395,9 @@ class SnakeGame:
         """Same through HOST (pinned) tensors: `host` is a dict of CPU tensors with the keys of
         alloc_outputs() plus the inputs ('act_idx', or 'q' [+ 'u', 'ridx']).  ASYNCHRONOUS: call sync() before
         reading an output or overwriting an input.  replay: also store! every transition into the device ring."""
-        fmt = _OBS[host["obs_fmt"]][0] if host.get("obs") is not None else OBS_NONE
         g = lambda k: _ptr(host.get(k))
         args = (g("q") if q else None, float(eps), g("u") if q else None, g("ridx") if q else None,
-                g("act_idx"), g("reward"), g("done"), g("obs"), fmt, g("mask"), g("ep_return"), g("ep_score"))
+                g("act_idx"), g("reward"), g("done"), g("obs"), _fmt_code(host), g("mask"), g("ep_return"), g("ep_score"))
         if replay is None:
             _check(lib().snk_step_fused_host(self._h, *args))
         else:
@@ -406,7 +409,7 @@ class SnakeGame:
         """(board_{t-1}, board_t) of every env: (N,2,10,10) [= Julia (10,10,2,N)]"""
         code, dt, per = _OBS[fmt]
         if out is None:
-            out = self._new((self.n, 2, 10, 10) if per == 200 else (self.n, per), dt)
+            out = self._new(_obs_shape(fmt, (self.n,)), dt)
         _check(lib().snk_state(self._h, _ptr(out, dt, self.n * per, self.device), code))
         return out
 
@@ -425,8 +428,8 @@ class SnakeGame:
         return out
 
     def assemble_state_host(self, fmt="f32"):
-        code, dt, per = _OBS[fmt]
-        return self._host(lib().snk_state_host, (self.n, 2, 10, 10) if per == 200 else (self.n, per), dt, code)
+        code, dt, _ = _OBS[fmt]
+        return self._host(lib().snk_state_host, _obs_shape(fmt, (self.n,)), dt, code)
 
     def virtual_step_host(self):
         return self._host(lib().snk_losing_mask_host, (self.n, 3), torch.uint8)

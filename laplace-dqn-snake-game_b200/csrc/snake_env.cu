@@ -26,6 +26,7 @@
 
 #include <new>
 #include <mutex>
+#include <type_traits>
 #include <unordered_map>
 
 #include <cuda.h>
@@ -104,11 +105,34 @@ constexpr u64 INIT_MISC = (7ull << M_HR) | (1ull << M_HC) | (8ull << M_TR) | (1u
 struct FoodTable {
     uint8_t bit[MAX_FOOD];   // interior bit index of list entry i
     int n;
+    __host__ __device__ u64 mask() const { return n >= 64 ? ~0ull : ((1ull << n) - 1ull); }   // the entries of the list
 };
 
 struct EnvState {
     u64 *occ, *pocc, *clo, *chi, *cons, *misc;
     float *ret;
+};
+
+// bytes of one env's observation; 0 for SNK_OBS_NONE and unknown formats
+__host__ __device__ constexpr int obs_bytes(int fmt) {
+    switch (fmt) {
+        case SNK_OBS_F32: return 800;
+        case SNK_OBS_I8: return 200;
+        case SNK_OBS_I64: return 1600;
+        case SNK_OBS_PACKED2: return 50;
+        case SNK_OBS_BITS: return 24;
+        default: return 0;
+    }
+}
+
+// the per-step outputs of the step and rollout kernels, any of them NULL
+struct StepOutputs {
+    float *reward;
+    uint8_t *done;
+    void *obs;
+    uint8_t *mask;
+    float *ep_return;
+    int32_t *ep_score;
 };
 
 struct StepArgs {
@@ -119,12 +143,7 @@ struct StepArgs {
     const uint8_t *ridx;     // (N) or NULL
     float eps;
     uint8_t *act_out;
-    float *reward;
-    uint8_t *done;
-    void *obs;
-    uint8_t *mask;
-    float *ep_return;
-    int32_t *ep_score;
+    StepOutputs out;
     long long env_begin, env_end;
     u64 seed, step_counter;
     int auto_reset, is_abs;
@@ -209,8 +228,19 @@ __device__ __forceinline__ void set_k(int r, int c, u64 &lo, u64 &hi) {
     u64 b = 1ull << (k & 63);
     if (k < 64) lo |= b; else hi |= b;
 }
-// Two bit-planes of one board, code = 2*p1 + p0: 0 empty, 1 snake, 2 food, 3 wall.  The head is drawn last
-// as snake, which reproduces update_board! overwriting the wall cell on a wall death (utils.jl:48-50).
+// Two bit-planes of one board in full-board bit space (cells 0..63 in lo, 64..99 in hi), code = 2*p1 + p0: 0 empty, 1 snake,
+// 2 food, 3 wall.  The head is drawn last as snake, which reproduces update_board! overwriting the wall cell on a wall death
+// (utils.jl:48-50).
+__device__ __forceinline__ void board_bits(u64 occ, int fr, int fc, bool has_head, int hr, int hc, u64 &p0lo, u64 &p0hi,
+                                           u64 &p1lo, u64 &p1hi) {
+    u64 slo, shi;
+    to_full(occ, slo, shi);
+    if (has_head) set_k(hr, hc, slo, shi);
+    u64 flo = WALL_LO, fhi = WALL_HI;
+    if (fr != 0) set_k(fr, fc, flo, fhi);
+    p0lo = slo | WALL_LO; p0hi = shi | WALL_HI;
+    p1lo = flo & ~slo; p1hi = fhi & ~shi;
+}
 // nibble i of x -> byte i of the result (low nibble of each byte)
 __device__ __forceinline__ u64 spread_nibbles(uint32_t x) {
     u64 v = x;
@@ -239,27 +269,18 @@ __device__ __forceinline__ u64 unit_word(uint32_t p0, uint32_t p1) {
 // so phase B needs one byte load per 16-byte store.
 template <bool PERM = true>
 __device__ __forceinline__ void board_planes(u64 occ, int fr, int fc, bool has_head, int hr, int hc, uint32_t *dst) {
-    u64 slo, shi;
-    to_full(occ, slo, shi);
-    if (has_head) set_k(hr, hc, slo, shi);
-    u64 flo = WALL_LO, fhi = WALL_HI;
-    if (fr != 0) set_k(fr, fc, flo, fhi);
-    const u64 p0lo = slo | WALL_LO, p0hi = shi | WALL_HI;
-    const u64 p1lo = flo & ~slo, p1hi = fhi & ~shi;
+    u64 p0lo, p0hi, p1lo, p1hi;
+    board_bits(occ, fr, fc, has_head, hr, hc, p0lo, p0hi, p1lo, p1hi);
     u64 *d = reinterpret_cast<u64 *>(dst);
     d[0] = unit_word<PERM>((uint32_t)p0lo, (uint32_t)p1lo);
     d[1] = unit_word<PERM>((uint32_t)(p0lo >> 32), (uint32_t)(p1lo >> 32));
     d[2] = unit_word<PERM>((uint32_t)p0hi, (uint32_t)p1hi);
     d[3] = unit_word<PERM>((uint32_t)(p0hi >> 32), (uint32_t)(p1hi >> 32));
 }
+// the same board as two 16-byte plane vectors (the transition record)
 __device__ __forceinline__ void board_planes_reg(u64 occ, int fr, int fc, bool has_head, int hr, int hc, uint4 &a, uint4 &b) {
-    u64 slo, shi;
-    to_full(occ, slo, shi);
-    if (has_head) set_k(hr, hc, slo, shi);
-    u64 flo = WALL_LO, fhi = WALL_HI;
-    if (fr != 0) set_k(fr, fc, flo, fhi);
-    u64 p0lo = slo | WALL_LO, p0hi = shi | WALL_HI;
-    u64 p1lo = flo & ~slo, p1hi = fhi & ~shi;
+    u64 p0lo, p0hi, p1lo, p1hi;
+    board_bits(occ, fr, fc, has_head, hr, hc, p0lo, p0hi, p1lo, p1hi);
     a = make_uint4((uint32_t)p0lo, (uint32_t)(p0lo >> 32), (uint32_t)p0hi, (uint32_t)(p0hi >> 32));
     b = make_uint4((uint32_t)p1lo, (uint32_t)(p1lo >> 32), (uint32_t)p1hi, (uint32_t)(p1hi >> 32));
 }
@@ -422,6 +443,20 @@ __device__ __forceinline__ uint32_t losing_mask3(u64 occ, u64 cons, int hr, int 
     return m;
 }
 
+// next_is_suicidal bits m3 as 3 bytes
+__device__ __forceinline__ void store_mask3(uint8_t *m, uint32_t m3) {
+    m[0] = (uint8_t)(m3 & 1u); m[1] = (uint8_t)((m3 >> 1) & 1u); m[2] = (uint8_t)((m3 >> 2) & 1u);
+}
+// the scalar outputs of env i's step (row i of a step's outputs)
+__device__ __forceinline__ void store_step_outputs(const StepOutputs &o, long long i, float reward, int done, uint32_t m3, float ret,
+                                                   int score) {
+    if (o.reward != nullptr) o.reward[i] = reward;
+    if (o.done != nullptr) o.done[i] = (uint8_t)done;
+    if (o.mask != nullptr) store_mask3(o.mask + 3 * i, m3);
+    if (o.ep_return != nullptr) o.ep_return[i] = ret;
+    if (o.ep_score != nullptr) o.ep_score[i] = score;
+}
+
 // ---- one env in registers ---------------------------------------------------------------------------
 constexpr int CHI_FROM_LEN = 32;          // see env_load
 struct Env {
@@ -434,18 +469,21 @@ struct Env {
 // CHI_LAZY = true: the second word of the direction chain (entries 32..63) only carries live entries for a snake of 34 or more
 // segments, and an entry that is live when it crosses from clo into chi does so at length >= 33: the word is fetched (and,
 // see env_store, written back) only from length 32 on.  Below that its content in memory is never looked at by anybody.
-template <bool POCC_ALWAYS = true, bool CHI_LAZY = false>
-__device__ __forceinline__ void env_load(Env &e, const EnvState &s, long long i) {
-    e.occ = s.occ[i]; e.clo = s.clo[i]; e.cons = s.cons[i]; e.ret = s.ret[i];
-    const u64 misc = s.misc[i];
-    e.pocc = (POCC_ALWAYS || ((misc >> M_DONE) & 1ull)) ? s.pocc[i] : 0ull;
-    e.chi = (!CHI_LAZY || ((int)(misc >> M_LEN) & 127) >= CHI_FROM_LEN) ? s.chi[i] : 0ull;
+__device__ __forceinline__ void env_unpack(Env &e, u64 misc) {
     e.hr = (int)(misc >> M_HR) & 15; e.hc = (int)(misc >> M_HC) & 15;
     e.tr = (int)(misc >> M_TR) & 15; e.tc = (int)(misc >> M_TC) & 15;
     e.fr = (int)(misc >> M_FR) & 15; e.fc = (int)(misc >> M_FC) & 15;
     e.pfr = (int)(misc >> M_PFR) & 15; e.pfc = (int)(misc >> M_PFC) & 15;
     e.pd = (int)(misc >> M_PD) & 3; e.len = (int)(misc >> M_LEN) & 127; e.t = (int)(misc >> M_T) & 1023;
     e.dn = (int)(misc >> M_DONE) & 1; e.err = (int)(misc >> M_ERR) & 15;
+}
+template <bool POCC_ALWAYS = true, bool CHI_LAZY = false>
+__device__ __forceinline__ void env_load(Env &e, const EnvState &s, long long i) {
+    e.occ = s.occ[i]; e.clo = s.clo[i]; e.cons = s.cons[i]; e.ret = s.ret[i];
+    const u64 misc = s.misc[i];
+    e.pocc = (POCC_ALWAYS || ((misc >> M_DONE) & 1ull)) ? s.pocc[i] : 0ull;
+    e.chi = (!CHI_LAZY || ((int)(misc >> M_LEN) & 127) >= CHI_FROM_LEN) ? s.chi[i] : 0ull;
+    env_unpack(e, misc);
 }
 __device__ __forceinline__ void env_store(const Env &e, const EnvState &s, long long i, bool store_chi = true, bool store_cons = true) {
     const u64 misc = ((u64)e.hr << M_HR) | ((u64)e.hc << M_HC) | ((u64)e.tr << M_TR) | ((u64)e.tc << M_TC) |
@@ -558,7 +596,7 @@ __global__ void __launch_bounds__(TPB, (OBS == SNK_OBS_F32 || OBS == SNK_OBS_I64
         env_load<SINK, true>(e, a.s, env);                         // the transition record needs board_{t-2}
         const bool chi_live = e.len >= CHI_FROM_LEN;
         const u64 cons_loaded = e.cons;                             // changes only when an apple is eaten or the env resets
-        const u64 list_mask = a.food.n >= 64 ? ~0ull : ((1ull << a.food.n) - 1ull);
+        const u64 list_mask = a.food.mask();
         const u64 occ_tm2 = e.pocc;                                 // board_{t-2}, for the transition record
         const int fr_tm2 = e.pfr, fc_tm2 = e.pfc, pd_before = e.pd;
 
@@ -585,15 +623,12 @@ __global__ void __launch_bounds__(TPB, (OBS == SNK_OBS_F32 || OBS == SNK_OBS_I64
         uint32_t m3 = 7u;
         if (!e.dn) reward = env_advance(e, aidx, a.is_abs, list_mask, s_food_bit, m3);
 
-        if (a.reward != nullptr) a.reward[env] = reward;
-        if (a.done != nullptr) a.done[env] = (uint8_t)e.dn;
-        if (a.mask != nullptr) {
-            a.mask[3 * env + 0] = (uint8_t)(m3 & 1u);
-            a.mask[3 * env + 1] = (uint8_t)((m3 >> 1) & 1u);
-            a.mask[3 * env + 2] = (uint8_t)((m3 >> 2) & 1u);
-        }
-        if (a.ep_return != nullptr) a.ep_return[env] = e.ret;
-        if (a.ep_score != nullptr) a.ep_score[env] = e.len - 2;
+        // (not store_step_outputs: through it ptxas gives the SINK kernels of three formats one or two registers more or less)
+        if (a.out.reward != nullptr) a.out.reward[env] = reward;
+        if (a.out.done != nullptr) a.out.done[env] = (uint8_t)e.dn;
+        if (a.out.mask != nullptr) store_mask3(a.out.mask + 3 * env, m3);
+        if (a.out.ep_return != nullptr) a.out.ep_return[env] = e.ret;
+        if (a.out.ep_score != nullptr) a.out.ep_score[env] = e.len - 2;
 
         if (obs_expands(OBS)) {
             constexpr bool PERM = OBS != SNK_OBS_F32 && OBS != SNK_OBS_I64;
@@ -601,7 +636,7 @@ __global__ void __launch_bounds__(TPB, (OBS == SNK_OBS_F32 || OBS == SNK_OBS_I64
             board_planes<PERM>(e.occ, e.fr, e.fc, true, e.hr, e.hc, s_planes + tid * PLANE_WORDS + 8);
         }
         if (OBS == SNK_OBS_BITS)
-            store_bits_record(a.obs, env, e.pocc, e.pfr, e.pfc, e.occ, e.fr, e.fc, e.hr, e.hc, m3, e.dn, aidx, reward);
+            store_bits_record(a.out.obs, env, e.pocc, e.pfr, e.pfc, e.occ, e.fr, e.fc, e.hr, e.hc, m3, e.dn, aidx, reward);
 
         if (SINK) {
             // store!(rpb, exp) for envs in index order == ring slot (stored_so_far + env) mod capacity; when the
@@ -629,7 +664,7 @@ __global__ void __launch_bounds__(TPB, (OBS == SNK_OBS_F32 || OBS == SNK_OBS_I64
 
     if (obs_expands(OBS)) {
         __syncthreads();
-        expand_obs<OBS>(a.obs, env0, n_local, s_planes, s_tb, tid);
+        expand_obs<OBS>(a.out.obs, env0, n_local, s_planes, s_tb, tid);
     }
 }
 
@@ -639,12 +674,7 @@ __global__ void __launch_bounds__(TPB, (OBS == SNK_OBS_F32 || OBS == SNK_OBS_I64
 struct RolloutArgs {
     EnvState s;
     const uint8_t *act;
-    float *reward;
-    uint8_t *done;
-    void *obs;
-    uint8_t *mask;
-    float *ep_return;
-    int32_t *ep_score;
+    StepOutputs out;
     long long n;
     int steps, auto_reset, is_abs;
     long long *prof;         // debug (snk_debug_rollout_timing): cycle counts of CTA 0's logic warp / expander thread 0
@@ -672,10 +702,10 @@ __global__ void __launch_bounds__(RTPB) k_rollout(const __grid_constant__ Rollou
     if (tid < MAX_FOOD) s_food_bit[tid] = a.food.bit[tid];
     if (OBS != SNK_OBS_NONE) fill_tables<OBS>(s_tb, tid, RTPB);
     __syncthreads();
-    const u64 list_mask = a.food.n >= 64 ? ~0ull : ((1ull << a.food.n) - 1ull);
+    const u64 list_mask = a.food.mask();
     Env e;
     if (mine) env_load(e, a.s, env);
-    const size_t obs_step = (size_t)a.n * (OBS == SNK_OBS_F32 ? 800 : OBS == SNK_OBS_I8 ? 200 : OBS == SNK_OBS_I64 ? 1600 : 50);
+    const size_t obs_step = (size_t)a.n * obs_bytes(OBS);
     for (int t = 0; t < a.steps; t++) {
         if (mine) {
             const long long o = (long long)t * a.n + env;
@@ -683,14 +713,7 @@ __global__ void __launch_bounds__(RTPB) k_rollout(const __grid_constant__ Rollou
             float reward = 0.0f;
             uint32_t m3 = 7u;
             if (!e.dn) reward = env_advance(e, aidx, a.is_abs, list_mask, s_food_bit, m3);
-            if (a.reward != nullptr) a.reward[o] = reward;
-            if (a.done != nullptr) a.done[o] = (uint8_t)e.dn;
-            if (a.mask != nullptr) {
-                uint8_t *m = a.mask + 3 * o;
-                m[0] = (uint8_t)(m3 & 1u); m[1] = (uint8_t)((m3 >> 1) & 1u); m[2] = (uint8_t)((m3 >> 2) & 1u);
-            }
-            if (a.ep_return != nullptr) a.ep_return[o] = e.ret;
-            if (a.ep_score != nullptr) a.ep_score[o] = e.len - 2;
+            store_step_outputs(a.out, o, reward, e.dn, m3, e.ret, e.len - 2);
             if (OBS != SNK_OBS_NONE) {
                 board_planes(e.pocc, e.pfr, e.pfc, false, 0, 0, s_planes + tid * PLANE_WORDS);
                 board_planes(e.occ, e.fr, e.fc, true, e.hr, e.hc, s_planes + tid * PLANE_WORDS + 8);
@@ -699,7 +722,7 @@ __global__ void __launch_bounds__(RTPB) k_rollout(const __grid_constant__ Rollou
         }
         if (OBS != SNK_OBS_NONE) {
             __syncthreads();
-            expand_obs<OBS, RTPB, 5, true>((uint8_t *)a.obs + (size_t)t * obs_step, env0, n_local, s_planes, s_tb, tid);
+            expand_obs<OBS, RTPB, 5, true>((uint8_t *)a.out.obs + (size_t)t * obs_step, env0, n_local, s_planes, s_tb, tid);
             __syncthreads();
         }
     }
@@ -753,7 +776,6 @@ __global__ void __launch_bounds__(WS_THREADS) k_rollout_ws(const __grid_constant
     // 0.65, Float32 0.80 / 0.82 — with the large formats the expansion chain sets the pace and the extra warp only adds
     // contention, so the second mask warp stays idle there (it waits at the final barrier).
     constexpr bool TWO_MASK = OBS != SNK_OBS_F32 && OBS != SNK_OBS_I64;
-    constexpr int PER = OBS == SNK_OBS_F32 ? 800 : OBS == SNK_OBS_I8 ? 200 : OBS == SNK_OBS_I64 ? 1600 : OBS == SNK_OBS_PACKED2 ? 50 : 0;
     __shared__ Handoff s_hand[2][EPB];
     __shared__ __align__(16) uint32_t s_planes[EPB * PLANE_WORDS];
     __shared__ ObsTables s_tb;
@@ -771,7 +793,7 @@ __global__ void __launch_bounds__(WS_THREADS) k_rollout_ws(const __grid_constant
     // warp 0 waits two steps later), XB among the expansion warps.  Consumers that have nothing to do for this format
     // (expansion warps without an observation) still take part in FULL / EMPTY so that the counts stay WS_BAR.
     constexpr int FULL = 1, EMPTY = 3, XB = 5;
-    const u64 list_mask = a.food.n >= 64 ? ~0ull : ((1ull << a.food.n) - 1ull);
+    const u64 list_mask = a.food.mask();
     Env e;
     const bool mine = warp == 0 && lane < n_local;
     const long long env = env0 + (mine ? lane : 0);
@@ -839,15 +861,7 @@ __global__ void __launch_bounds__(WS_THREADS) k_rollout_ws(const __grid_constant
                                       (int)(h.pk2 >> 10) & 1023, list_mask, s_food_bit, err);
                     if (err) atomicOr(&s_err[lane], err);
                 }
-                const long long o = (long long)t * a.n + env0 + lane;
-                if (a.reward != nullptr) a.reward[o] = h.reward;
-                if (a.done != nullptr) a.done[o] = (uint8_t)dn;
-                if (a.mask != nullptr) {
-                    uint8_t *m = a.mask + 3 * o;
-                    m[0] = (uint8_t)(m3 & 1u); m[1] = (uint8_t)((m3 >> 1) & 1u); m[2] = (uint8_t)((m3 >> 2) & 1u);
-                }
-                if (a.ep_return != nullptr) a.ep_return[o] = h.ret;
-                if (a.ep_score != nullptr) a.ep_score[o] = h.score;
+                store_step_outputs(a.out, (long long)t * a.n + env0 + lane, h.reward, dn, m3, h.ret, h.score);
             }
             if (prof) p_role += clock64() - c0;
         }
@@ -858,7 +872,7 @@ __global__ void __launch_bounds__(WS_THREADS) k_rollout_ws(const __grid_constant
         const int et = tid - 64;                             // 0..NX-1
         const bool prof = a.prof != nullptr && blockIdx.x == 0 && et == 0;
         long long p_exp = 0, p_xfull = 0;
-        const size_t obs_step = (size_t)a.n * PER;
+        const size_t obs_step = (size_t)a.n * obs_bytes(OBS);
         for (int t = 0; t < a.steps; t++) {
             const int b = t & 1;
             long long c0 = prof ? clock64() : 0;
@@ -879,7 +893,7 @@ __global__ void __launch_bounds__(WS_THREADS) k_rollout_ws(const __grid_constant
                 // (Staging the CTA's contiguous region of the step in shared memory and sending it off as one bulk asynchronous
                 // copy was measured slower: 1.04 against 0.90 us per step with Float32 observations.)
                 nbar_sync(XB, NX);
-                expand_obs<OBS, NX, 5, WS_STREAM>((uint8_t *)a.obs + (size_t)t * obs_step, env0, n_local, s_planes, s_tb, et);
+                expand_obs<OBS, NX, 5, WS_STREAM>((uint8_t *)a.out.obs + (size_t)t * obs_step, env0, n_local, s_planes, s_tb, et);
                 nbar_sync(XB, NX);
                 if (prof) p_exp += clock64() - c0;
             }
@@ -894,6 +908,8 @@ __global__ void __launch_bounds__(WS_THREADS) k_rollout_ws(const __grid_constant
 }
 
 // ---- stand-alone views of the state ------------------------------------------------------------
+// k_state and k_losing_mask decode only the misc fields they use: decoding through env_unpack costs k_state<F32> and
+// k_state<I64> 8 instructions and one or two registers more.
 template <int OBS>
 __global__ void __launch_bounds__(TPB) k_state(EnvState s, long long n, void *obs) {
     __shared__ __align__(16) uint32_t s_planes[TPB * PLANE_WORDS];
@@ -997,14 +1013,13 @@ __global__ void k_losing_mask(EnvState s, long long n, uint8_t *out, FoodTable f
     uint32_t m3 = 7u;
     if (!((misc >> M_DONE) & 1ull)) {
         int err = (int)(misc >> M_ERR) & 15, err0 = err;
-        const u64 list_mask = food.n >= 64 ? ~0ull : ((1ull << food.n) - 1ull);
         m3 = losing_mask3(s.occ[i], s.cons[i], (int)(misc >> M_HR) & 15, (int)(misc >> M_HC) & 15,
                           (int)(misc >> M_TR) & 15, (int)(misc >> M_TC) & 15, (int)(misc >> M_FR) & 15,
-                          (int)(misc >> M_FC) & 15, (int)(misc >> M_PD) & 3, (int)(misc >> M_T) & 1023, list_mask,
+                          (int)(misc >> M_FC) & 15, (int)(misc >> M_PD) & 3, (int)(misc >> M_T) & 1023, food.mask(),
                           s_food_bit, err);
         if (err != err0) s.misc[i] = (misc & ~(15ull << M_ERR)) | ((u64)err << M_ERR);
     }
-    out[3 * i + 0] = m3 & 1u; out[3 * i + 1] = (m3 >> 1) & 1u; out[3 * i + 2] = (m3 >> 2) & 1u;
+    store_mask3(out + 3 * i, m3);
 }
 
 __global__ void k_select(long long n, const float *q, float eps, const float *u, const uint8_t *ridx, u64 seed,
@@ -1165,6 +1180,18 @@ struct snk_env {
     size_t d_obs_bytes;
 };
 
+// the replay ring (ReplayBuffer, structs.jl:104-116)
+struct snk_replay_s {
+    long long capacity;
+    int device;
+    uint4 *ring;             // capacity x 128-byte records
+    long long total;         // transitions ever stored since the last clear
+    u64 draws;               // sample calls so far (counter of the keyed permutation)
+    int *d_bad;
+    uint8_t *stage;          // device staging of snk_replay_gather_host
+    size_t stage_bytes;
+};
+
 static const uint8_t kDefaultFoodRC[100] = {  // Xoshiro(42) list, structs.jl:70 (pinned by tests/test_oracle_golden.py)
     7, 5, 5, 7, 7, 3, 6, 7, 5, 4, 7, 7, 4, 4, 6, 2, 4, 3, 5, 5, 2, 6, 3, 6, 5, 4, 5, 8, 4, 6, 4, 3, 7, 4,
     2, 2, 7, 5, 7, 3, 6, 5, 8, 3, 4, 9, 4, 7, 8, 6, 4, 4, 6, 6, 4, 2, 2, 8, 9, 3, 7, 4, 4, 8, 7, 7, 4, 2,
@@ -1184,6 +1211,16 @@ static int set_food(FoodTable &ft, const uint8_t *rc, int n) {
 
 static inline unsigned nblocks(long long n, int tpb) { return (unsigned)((n + tpb - 1) / tpb); }
 
+// Runs f(std::integral_constant<int, FMT>()) for the FMT among FMTS that equals fmt, then checks the launches f made: a
+// runtime observation format becomes a template argument.  Each caller lists the formats it has kernels for.
+template <int... FMTS, class F>
+static int launch_obs_fmt(int fmt, F &&f) {
+    if (!((fmt == FMTS && (f(std::integral_constant<int, FMTS>()), true)) || ...))
+        return fail(SNK_ERR_INVALID, "unknown obs_fmt %d", fmt);
+    SNK_CUDA(cudaGetLastError());
+    return SNK_OK;
+}
+
 #define SNK_CHECK_HANDLE(h)                                                  \
     do {                                                                     \
         if ((h) == nullptr) return fail(SNK_ERR_INVALID, "%s: null handle", __func__); \
@@ -1194,6 +1231,36 @@ template <typename T>
 static cudaError_t ensure(T **p, size_t bytes) {
     if (*p != nullptr) return cudaSuccess;
     return cudaMalloc((void **)p, bytes);
+}
+
+// The device staging buffers of the host-buffer entry points are read by copies on copy_stream[0] that the handle's own
+// stream does NOT wait for (so that later work on it — e.g. the minibatch gather — overlaps those copies): whoever is about
+// to overwrite the staging buffers first orders itself behind the last such copy.
+static int staging_guard(snk_handle h) {
+    SNK_CUDA(cudaStreamWaitEvent(h->stream, h->ev_done, 0));
+    return SNK_OK;
+}
+
+// device staging buffer of the host getters (grown on demand)
+static int ensure_obs_staging(snk_handle h, size_t bytes) {
+    if (h->d_obs_bytes >= bytes) return SNK_OK;
+    if (h->d_obs) { SNK_CUDA(cudaStreamSynchronize(h->stream)); SNK_CUDA(cudaFree(h->d_obs)); h->d_obs = nullptr; h->d_obs_bytes = 0; }
+    SNK_CUDA(cudaMalloc(&h->d_obs, bytes));
+    h->d_obs_bytes = bytes;
+    return SNK_OK;
+}
+
+// The host getters: run(dev), the device form, writes `bytes` into the staging buffer dev, which is then copied down
+// (synchronously).  staging_guard comes first: nothing may write the staging buffer before it.
+template <class Run>
+static int get_host(snk_handle h, void *out_host, size_t bytes, Run &&run) {
+    int rc = staging_guard(h);
+    if (rc == SNK_OK) rc = ensure_obs_staging(h, bytes);
+    if (rc == SNK_OK) rc = run(h->d_obs);
+    if (rc != SNK_OK) return rc;
+    SNK_CUDA(cudaMemcpyAsync(out_host, h->d_obs, bytes, cudaMemcpyDeviceToHost, h->stream));
+    SNK_CUDA(cudaStreamSynchronize(h->stream));
+    return SNK_OK;
 }
 
 #ifndef SNK_HOST_CHUNK_MB
@@ -1451,77 +1518,93 @@ int snk_available_actions(snk_handle h, uint8_t *dirs_3xN) {
 }
 
 // launches the fused kernel for envs [begin, end) on `st`
-static int launch_step(snk_handle h, StepArgs &a, int obs_fmt, bool select, long long begin, long long end, cudaStream_t st) {
+static int launch_step(StepArgs &a, int obs_fmt, bool select, long long begin, long long end, cudaStream_t st) {
     a.env_begin = begin; a.env_end = end;
     unsigned grid = nblocks(end - begin, TPB);
     if (grid == 0) return SNK_OK;
-#define SNK_LAUNCH(FMT)                                                        \
-    do {                                                                       \
-        if (a.sink != nullptr) {                                               \
-            if (select) k_step<FMT, true, true><<<grid, TPB, 0, st>>>(a);      \
-            else k_step<FMT, false, true><<<grid, TPB, 0, st>>>(a);            \
-        } else {                                                               \
-            if (select) k_step<FMT, true, false><<<grid, TPB, 0, st>>>(a);     \
-            else k_step<FMT, false, false><<<grid, TPB, 0, st>>>(a);           \
-        }                                                                      \
-    } while (0)
-    switch (obs_fmt) {
-        case SNK_OBS_NONE: SNK_LAUNCH(SNK_OBS_NONE); break;
-        case SNK_OBS_F32: SNK_LAUNCH(SNK_OBS_F32); break;
-        case SNK_OBS_I8: SNK_LAUNCH(SNK_OBS_I8); break;
-        case SNK_OBS_I64: SNK_LAUNCH(SNK_OBS_I64); break;
-        case SNK_OBS_PACKED2: SNK_LAUNCH(SNK_OBS_PACKED2); break;
-        case SNK_OBS_BITS: SNK_LAUNCH(SNK_OBS_BITS); break;
-        default: return fail(SNK_ERR_INVALID, "unknown obs_fmt %d", obs_fmt);
-    }
-#undef SNK_LAUNCH
-    SNK_CUDA(cudaGetLastError());
-    return SNK_OK;
+    return launch_obs_fmt<SNK_OBS_NONE, SNK_OBS_F32, SNK_OBS_I8, SNK_OBS_I64, SNK_OBS_PACKED2, SNK_OBS_BITS>(obs_fmt, [&](auto fmt) {
+        constexpr int FMT = decltype(fmt)::value;
+        if (a.sink != nullptr) {
+            if (select) k_step<FMT, true, true><<<grid, TPB, 0, st>>>(a);
+            else k_step<FMT, false, true><<<grid, TPB, 0, st>>>(a);
+        } else {
+            if (select) k_step<FMT, true, false><<<grid, TPB, 0, st>>>(a);
+            else k_step<FMT, false, false><<<grid, TPB, 0, st>>>(a);
+        }
+    });
 }
 
-static void base_args(snk_handle h, StepArgs &a) {
+// The arguments of a step of every env of h.  q != NULL: act_idx receives the selected actions, else it holds the input
+// actions.  r != NULL: the step also stores every env's transition into the replay ring r.
+static StepArgs step_args(snk_handle h, const float *q, float eps, const float *u, const uint8_t *ridx, uint8_t *act_idx,
+                          const StepOutputs &out, const snk_replay_s *r) {
+    StepArgs a;
     memset(&a, 0, sizeof(a));
     a.s = h->s; a.food = h->food; a.seed = h->seed; a.step_counter = h->step_counter;
     a.auto_reset = (h->flags & SNK_AUTO_RESET) ? 1 : 0;
+    a.q = q; a.eps = eps; a.u = u; a.ridx = ridx;
+    if (q != nullptr) a.act_out = act_idx; else a.act = act_idx;
+    a.out = out;
+    if (r != nullptr) { a.sink = r->ring; a.sink_base = r->total; a.sink_cap = r->capacity; a.sink_n = h->n; }
+    return a;
+}
+
+// snk_step / snk_step_abs: the step without an observation
+static int step_plain(snk_handle h, const uint8_t *act, int is_abs, float *reward, uint8_t *done) {
+    StepArgs a = step_args(h, nullptr, 0.0f, nullptr, nullptr, nullptr, {reward, done}, nullptr);
+    a.act = act; a.is_abs = is_abs;
+    int rc = launch_step(a, SNK_OBS_NONE, false, 0, h->n, h->stream);
+    h->step_counter++;
+    return rc;
 }
 
 int snk_step(snk_handle h, const uint8_t *act_idx, float *reward, uint8_t *done) {
     SNK_CHECK_HANDLE(h);
     SNK_REQUIRE(act_idx != nullptr, "null actions");
-    StepArgs a;
-    base_args(h, a);
-    a.act = act_idx; a.reward = reward; a.done = done;
-    int rc = launch_step(h, a, SNK_OBS_NONE, false, 0, h->n, h->stream);
-    h->step_counter++;
-    return rc;
+    return step_plain(h, act_idx, 0, reward, done);
 }
 
 int snk_step_abs(snk_handle h, const uint8_t *dir, float *reward, uint8_t *done) {
     SNK_CHECK_HANDLE(h);
     SNK_REQUIRE(dir != nullptr, "null directions");
-    StepArgs a;
-    base_args(h, a);
-    a.act = dir; a.reward = reward; a.done = done; a.is_abs = 1;
-    int rc = launch_step(h, a, SNK_OBS_NONE, false, 0, h->n, h->stream);
+    return step_plain(h, dir, 1, reward, done);
+}
+
+// The argument checks of the fused step entry points; fn names the entry point in the messages.
+static int check_step_inputs(const char *fn, const float *q, const uint8_t *act_idx, const void *obs, int obs_fmt) {
+    if (q == nullptr && act_idx == nullptr) return fail(SNK_ERR_INVALID, "%s: need q (select) or act_idx (input)", fn);
+    if (obs_fmt != SNK_OBS_NONE && obs == nullptr) return fail(SNK_ERR_INVALID, "%s: obs_fmt given without an obs buffer", fn);
+    return SNK_OK;
+}
+// `what` names the store in the SNK_ERR_UNSUPPORTED message
+static int check_replay(const char *fn, snk_handle h, const snk_replay_s *r, const char *what) {
+    if (r->device != h->device) return fail(SNK_ERR_INVALID, "%s: replay ring and env live on different devices", fn);
+    if (!(h->flags & SNK_AUTO_RESET))
+        return fail(SNK_ERR_UNSUPPORTED, "%s needs an env created with SNK_AUTO_RESET (every env must step)", what);
+    return SNK_OK;
+}
+
+// The fused step with DEVICE buffers; with a replay ring r the same kernel also store!s every transition into it.
+static int step_fused_impl(const char *fn, snk_handle h, snk_replay_s *r, const float *q, float eps, const float *u,
+                           const uint8_t *ridx, uint8_t *act_idx, float *reward, uint8_t *done, void *obs, int obs_fmt,
+                           uint8_t *mask, float *ep_return, int32_t *ep_score) {
+    if (h == nullptr) return fail(SNK_ERR_INVALID, "%s: null handle", fn);
+    DeviceGuard guard(h->device);
+    int rc = r != nullptr ? check_replay(fn, h, r, fn) : SNK_OK;
+    if (rc == SNK_OK) rc = check_step_inputs(fn, q, act_idx, obs, obs_fmt);
+    if (rc != SNK_OK) return rc;
+    if (obs_fmt != SNK_OBS_NONE && ((uintptr_t)obs & 15u) != 0) return fail(SNK_ERR_INVALID, "%s: obs must be 16-byte aligned", fn);
+    StepArgs a = step_args(h, q, eps, u, ridx, act_idx, {reward, done, obs, mask, ep_return, ep_score}, r);
+    rc = launch_step(a, obs ? obs_fmt : SNK_OBS_NONE, q != nullptr, 0, h->n, h->stream);
     h->step_counter++;
+    if (rc == SNK_OK && r != nullptr) r->total += h->n;
     return rc;
 }
 
 int snk_step_fused(snk_handle h, const float *q, float eps, const float *u, const uint8_t *ridx, uint8_t *act_idx,
                    float *reward, uint8_t *done, void *obs, int obs_fmt, uint8_t *mask, float *ep_return,
                    int32_t *ep_score) {
-    SNK_CHECK_HANDLE(h);
-    SNK_REQUIRE(q != nullptr || act_idx != nullptr, "need q (select) or act_idx (input)");
-    SNK_REQUIRE(obs_fmt == SNK_OBS_NONE || obs != nullptr, "obs_fmt given without an obs buffer");
-    SNK_REQUIRE(obs_fmt == SNK_OBS_NONE || ((uintptr_t)obs & 15u) == 0, "obs must be 16-byte aligned");
-    StepArgs a;
-    base_args(h, a);
-    a.q = q; a.eps = eps; a.u = u; a.ridx = ridx;
-    if (q != nullptr) a.act_out = act_idx; else a.act = act_idx;
-    a.reward = reward; a.done = done; a.obs = obs; a.mask = mask; a.ep_return = ep_return; a.ep_score = ep_score;
-    int rc = launch_step(h, a, obs ? obs_fmt : SNK_OBS_NONE, q != nullptr, 0, h->n, h->stream);
-    h->step_counter++;
-    return rc;
+    return step_fused_impl(__func__, h, nullptr, q, eps, u, ridx, act_idx, reward, done, obs, obs_fmt, mask, ep_return, ep_score);
 }
 
 int snk_rollout_fused(snk_handle h, const uint8_t *act_TxN, int64_t T, int is_abs, float *reward, uint8_t *done, void *obs,
@@ -1532,41 +1615,20 @@ int snk_rollout_fused(snk_handle h, const uint8_t *act_TxN, int64_t T, int is_ab
     SNK_REQUIRE(obs == nullptr || ((uintptr_t)obs & 15u) == 0, "obs must be 16-byte aligned");
     RolloutArgs a;
     memset(&a, 0, sizeof(a));
-    a.s = h->s; a.food = h->food; a.act = act_TxN; a.reward = reward; a.done = done; a.obs = obs; a.mask = mask;
-    a.ep_return = ep_return; a.ep_score = ep_score; a.n = h->n; a.steps = (int)T; a.is_abs = is_abs;
+    a.s = h->s; a.food = h->food; a.act = act_TxN; a.out = {reward, done, obs, mask, ep_return, ep_score};
+    a.n = h->n; a.steps = (int)T; a.is_abs = is_abs;
     a.prof = g_rollout_prof;
     a.auto_reset = (h->flags & SNK_AUTO_RESET) ? 1 : 0;
-    const int fmt = obs ? obs_fmt : SNK_OBS_NONE;
     // small batches: the warp-specialised kernel, WS_EPB envs per CTA (4,096 envs -> 256 CTAs over the 148 SMs)
     const bool small = h->n <= 32 * 1024;
-#define SNK_RO(FMT)                                                                                       \
-    do {                                                                                                  \
-        if (small) k_rollout_ws<FMT, WS_EPB><<<nblocks(h->n, WS_EPB), WS_THREADS, 0, h->stream>>>(a);        \
-        else k_rollout<FMT, RTPB><<<nblocks(h->n, RTPB), RTPB, 0, h->stream>>>(a);                        \
-    } while (0)
-    switch (fmt) {
-        case SNK_OBS_NONE: SNK_RO(SNK_OBS_NONE); break;
-        case SNK_OBS_F32: SNK_RO(SNK_OBS_F32); break;
-        case SNK_OBS_I8: SNK_RO(SNK_OBS_I8); break;
-        case SNK_OBS_I64: SNK_RO(SNK_OBS_I64); break;
-        case SNK_OBS_PACKED2: SNK_RO(SNK_OBS_PACKED2); break;
-        default: return fail(SNK_ERR_INVALID, "unknown obs_fmt %d", obs_fmt);
-    }
-#undef SNK_RO
-    SNK_CUDA(cudaGetLastError());
-    h->step_counter += (u64)T;
-    return SNK_OK;
-}
-
-static size_t obs_bytes_per_env(int fmt) {
-    switch (fmt) {
-        case SNK_OBS_F32: return 800;
-        case SNK_OBS_I8: return 200;
-        case SNK_OBS_I64: return 1600;
-        case SNK_OBS_PACKED2: return 50;
-        case SNK_OBS_BITS: return 24;
-        default: return 0;
-    }
+    const int rc = launch_obs_fmt<SNK_OBS_NONE, SNK_OBS_F32, SNK_OBS_I8, SNK_OBS_I64, SNK_OBS_PACKED2>(
+        obs ? obs_fmt : SNK_OBS_NONE, [&](auto fmt) {
+            constexpr int FMT = decltype(fmt)::value;
+            if (small) k_rollout_ws<FMT, WS_EPB><<<nblocks(h->n, WS_EPB), WS_THREADS, 0, h->stream>>>(a);
+            else k_rollout<FMT, RTPB><<<nblocks(h->n, RTPB), RTPB, 0, h->stream>>>(a);
+        });
+    if (rc == SNK_OK) h->step_counter += (u64)T;
+    return rc;
 }
 
 int snk_host_alloc(void **p, size_t bytes) {
@@ -1651,49 +1713,13 @@ int snk_device_free(void *p) {
     return SNK_OK;
 }
 
-struct snk_replay_s;
-static int step_fused_host_impl(snk_handle h, snk_replay_s *r, const float *q, float eps, const float *u, const uint8_t *ridx,
-                                uint8_t *act_idx, float *reward, uint8_t *done, void *obs, int obs_fmt, uint8_t *mask,
-                                float *ep_return, int32_t *ep_score);
-
-int snk_step_fused_host(snk_handle h, const float *q, float eps, const float *u, const uint8_t *ridx, uint8_t *act_idx,
-                        float *reward, uint8_t *done, void *obs, int obs_fmt, uint8_t *mask, float *ep_return,
-                        int32_t *ep_score) {
-    return step_fused_host_impl(h, nullptr, q, eps, u, ridx, act_idx, reward, done, obs, obs_fmt, mask, ep_return, ep_score);
-}
-
-// The device staging buffers of the host-buffer entry points are read by copies on copy_stream[0] that the handle's own
-// stream does NOT wait for (so that later work on it — e.g. the minibatch gather — overlaps those copies): whoever is about
-// to overwrite the staging buffers first orders itself behind the last such copy.
-static int staging_guard(snk_handle h) {
-    SNK_CUDA(cudaStreamWaitEvent(h->stream, h->ev_done, 0));
-    return SNK_OK;
-}
-
-// device staging buffer of the host getters (grown on demand)
-static int ensure_obs_staging(snk_handle h, size_t bytes) {
-    if (h->d_obs_bytes >= bytes) return SNK_OK;
-    if (h->d_obs) { SNK_CUDA(cudaStreamSynchronize(h->stream)); SNK_CUDA(cudaFree(h->d_obs)); h->d_obs = nullptr; h->d_obs_bytes = 0; }
-    SNK_CUDA(cudaMalloc(&h->d_obs, bytes));
-    h->d_obs_bytes = bytes;
-    return SNK_OK;
-}
-
 int snk_state(snk_handle h, void *obs, int obs_fmt) {
     SNK_CHECK_HANDLE(h);
     SNK_REQUIRE(obs != nullptr, "null out");
     SNK_REQUIRE(((uintptr_t)obs & 15u) == 0, "obs must be 16-byte aligned");
-    unsigned grid = nblocks(h->n, TPB);
-    switch (obs_fmt) {
-        case SNK_OBS_F32: k_state<SNK_OBS_F32><<<grid, TPB, 0, h->stream>>>(h->s, h->n, obs); break;
-        case SNK_OBS_I8: k_state<SNK_OBS_I8><<<grid, TPB, 0, h->stream>>>(h->s, h->n, obs); break;
-        case SNK_OBS_I64: k_state<SNK_OBS_I64><<<grid, TPB, 0, h->stream>>>(h->s, h->n, obs); break;
-        case SNK_OBS_PACKED2: k_state<SNK_OBS_PACKED2><<<grid, TPB, 0, h->stream>>>(h->s, h->n, obs); break;
-        case SNK_OBS_BITS: k_state<SNK_OBS_BITS><<<grid, TPB, 0, h->stream>>>(h->s, h->n, obs); break;
-        default: return fail(SNK_ERR_INVALID, "unknown obs_fmt %d", obs_fmt);
-    }
-    SNK_CUDA(cudaGetLastError());
-    return SNK_OK;
+    return launch_obs_fmt<SNK_OBS_F32, SNK_OBS_I8, SNK_OBS_I64, SNK_OBS_PACKED2, SNK_OBS_BITS>(obs_fmt, [&](auto fmt) {
+        k_state<decltype(fmt)::value><<<nblocks(h->n, TPB), TPB, 0, h->stream>>>(h->s, h->n, obs);
+    });
 }
 
 int snk_patch_reset_obs(snk_handle h, const uint8_t *done, void *obs, int obs_fmt) {
@@ -1701,17 +1727,9 @@ int snk_patch_reset_obs(snk_handle h, const uint8_t *done, void *obs, int obs_fm
     SNK_REQUIRE(done != nullptr && obs != nullptr, "null argument");
     SNK_REQUIRE(((uintptr_t)obs & 15u) == 0, "obs must be 16-byte aligned");
     if (!(h->flags & SNK_AUTO_RESET)) return SNK_OK;          // frozen envs keep their terminal state
-    unsigned grid = nblocks(h->n, TPB);
-    switch (obs_fmt) {
-        case SNK_OBS_F32: k_patch_reset<SNK_OBS_F32><<<grid, TPB, 0, h->stream>>>(h->n, done, obs); break;
-        case SNK_OBS_I8: k_patch_reset<SNK_OBS_I8><<<grid, TPB, 0, h->stream>>>(h->n, done, obs); break;
-        case SNK_OBS_I64: k_patch_reset<SNK_OBS_I64><<<grid, TPB, 0, h->stream>>>(h->n, done, obs); break;
-        case SNK_OBS_PACKED2: k_patch_reset<SNK_OBS_PACKED2><<<grid, TPB, 0, h->stream>>>(h->n, done, obs); break;
-        case SNK_OBS_BITS: k_patch_reset<SNK_OBS_BITS><<<grid, TPB, 0, h->stream>>>(h->n, done, obs); break;
-        default: return fail(SNK_ERR_INVALID, "unknown obs_fmt %d", obs_fmt);
-    }
-    SNK_CUDA(cudaGetLastError());
-    return SNK_OK;
+    return launch_obs_fmt<SNK_OBS_F32, SNK_OBS_I8, SNK_OBS_I64, SNK_OBS_PACKED2, SNK_OBS_BITS>(obs_fmt, [&](auto fmt) {
+        k_patch_reset<decltype(fmt)::value><<<nblocks(h->n, TPB), TPB, 0, h->stream>>>(h->n, done, obs);
+    });
 }
 
 int snk_losing_mask(snk_handle h, uint8_t *mask_3xN) {
@@ -1771,17 +1789,6 @@ int snk_count_errors_host(snk_handle h, int64_t *count) {
 
 
 // ---- replay ring (ReplayBuffer, structs.jl:104-116; store!/sample/stack_exp, utils.jl:265-383) ----------
-struct snk_replay_s {
-    long long capacity;
-    int device;
-    uint4 *ring;             // capacity x 128-byte records
-    long long total;         // transitions ever stored since the last clear
-    u64 draws;               // sample calls so far (counter of the keyed permutation)
-    int *d_bad;
-    uint8_t *stage;          // device staging of snk_replay_gather_host
-    size_t stage_bytes;
-};
-
 int snk_replay_create(snk_replay *out, int64_t capacity, int device) {
     SNK_REQUIRE(out != nullptr, "null out");
     SNK_REQUIRE(capacity >= 64, "batch_size (64) cannot be greater than the capacity of the buffer");   // structs.jl:113
@@ -1827,24 +1834,8 @@ int snk_replay_length(snk_replay r, int64_t *length, int64_t *position) {
 int snk_step_fused_store(snk_handle h, snk_replay r, const float *q, float eps, const float *u, const uint8_t *ridx,
                          uint8_t *act_idx, float *reward, uint8_t *done, void *obs, int obs_fmt, uint8_t *mask,
                          float *ep_return, int32_t *ep_score) {
-    SNK_CHECK_HANDLE(h);
     SNK_REQUIRE(r != nullptr, "null replay");
-    SNK_REQUIRE(r->device == h->device, "replay ring and env live on different devices");
-    if (!(h->flags & SNK_AUTO_RESET))
-        return fail(SNK_ERR_UNSUPPORTED, "snk_step_fused_store needs an env created with SNK_AUTO_RESET (every env must step)");
-    SNK_REQUIRE(q != nullptr || act_idx != nullptr, "need q (select) or act_idx (input)");
-    SNK_REQUIRE(obs_fmt == SNK_OBS_NONE || obs != nullptr, "obs_fmt given without an obs buffer");
-    SNK_REQUIRE(obs_fmt == SNK_OBS_NONE || ((uintptr_t)obs & 15u) == 0, "obs must be 16-byte aligned");
-    StepArgs a;
-    base_args(h, a);
-    a.q = q; a.eps = eps; a.u = u; a.ridx = ridx;
-    if (q != nullptr) a.act_out = act_idx; else a.act = act_idx;
-    a.reward = reward; a.done = done; a.obs = obs; a.mask = mask; a.ep_return = ep_return; a.ep_score = ep_score;
-    a.sink = r->ring; a.sink_base = r->total; a.sink_cap = r->capacity; a.sink_n = h->n;
-    int rc = launch_step(h, a, obs ? obs_fmt : SNK_OBS_NONE, q != nullptr, 0, h->n, h->stream);
-    h->step_counter++;
-    if (rc == SNK_OK) r->total += h->n;
-    return rc;
+    return step_fused_impl(__func__, h, r, q, eps, u, ridx, act_idx, reward, done, obs, obs_fmt, mask, ep_return, ep_score);
 }
 
 int snk_replay_gather(snk_replay r, const int64_t *idx, int64_t B, float *states, float *next_states, uint8_t *actions,
@@ -1888,15 +1879,11 @@ static int step_fused_host_impl(snk_handle h, snk_replay_s *r, const float *q, f
                                 uint8_t *act_idx, float *reward, uint8_t *done, void *obs, int obs_fmt, uint8_t *mask,
                                 float *ep_return, int32_t *ep_score) {
     SNK_CHECK_HANDLE(h);
-    SNK_REQUIRE(q != nullptr || act_idx != nullptr, "need q (select) or act_idx (input)");
-    SNK_REQUIRE(obs_fmt == SNK_OBS_NONE || obs != nullptr, "obs_fmt given without an obs buffer");
-    if (r != nullptr) {
-        SNK_REQUIRE(r->device == h->device, "replay ring and env live on different devices");
-        if (!(h->flags & SNK_AUTO_RESET))
-            return fail(SNK_ERR_UNSUPPORTED, "storing transitions needs an env created with SNK_AUTO_RESET (every env must step)");
-    }
+    int rc = check_step_inputs(__func__, q, act_idx, obs, obs_fmt);
+    if (rc == SNK_OK && r != nullptr) rc = check_replay(__func__, h, r, "storing transitions");
+    if (rc != SNK_OK) return rc;
     const size_t n = (size_t)h->n;
-    const size_t opb = obs ? obs_bytes_per_env(obs_fmt) : 0;
+    const size_t opb = obs ? obs_bytes(obs_fmt) : 0;
     if (obs && opb == 0) return fail(SNK_ERR_INVALID, "unknown obs_fmt %d", obs_fmt);
     // device staging
     SNK_CUDA(ensure(&h->d_act, n));
@@ -1908,17 +1895,13 @@ static int step_fused_host_impl(snk_handle h, snk_replay_s *r, const float *q, f
     if (mask) { SNK_CUDA(ensure(&h->d_mask, 3 * n)); }
     if (ep_return) { SNK_CUDA(ensure(&h->d_ep_return, 4 * n)); }
     if (ep_score) { SNK_CUDA(ensure(&h->d_ep_score, 4 * n)); }
-    if (opb) { int rc = ensure_obs_staging(h, opb * n); if (rc != SNK_OK) return rc; }
-    { int rc = staging_guard(h); if (rc != SNK_OK) return rc; }
+    if (opb && (rc = ensure_obs_staging(h, opb * n)) != SNK_OK) return rc;
+    if ((rc = staging_guard(h)) != SNK_OK) return rc;
     cudaStream_t st = h->stream, down = h->copy_stream[0], up = h->copy_stream[1];
-    StepArgs a;
-    base_args(h, a);
-    a.q = q ? h->d_q : nullptr; a.eps = eps; a.u = u ? h->d_u : nullptr; a.ridx = ridx ? h->d_ridx : nullptr;
-    if (q) a.act_out = act_idx ? h->d_act : nullptr; else a.act = h->d_act;
-    a.reward = reward ? h->d_reward : nullptr; a.done = done ? h->d_done : nullptr; a.obs = opb ? h->d_obs : nullptr;
-    a.mask = mask ? h->d_mask : nullptr; a.ep_return = ep_return ? h->d_ep_return : nullptr;
-    a.ep_score = ep_score ? h->d_ep_score : nullptr;
-    if (r != nullptr) { a.sink = r->ring; a.sink_base = r->total; a.sink_cap = r->capacity; a.sink_n = h->n; }
+    StepArgs a = step_args(h, q ? h->d_q : nullptr, eps, u ? h->d_u : nullptr, ridx ? h->d_ridx : nullptr, act_idx ? h->d_act : nullptr,
+                           {reward ? h->d_reward : nullptr, done ? h->d_done : nullptr, opb ? h->d_obs : nullptr,
+                            mask ? h->d_mask : nullptr, ep_return ? h->d_ep_return : nullptr, ep_score ? h->d_ep_score : nullptr},
+                           r);
     // Chunking trades copy/kernel overlap (and the time before the first output copy can start) against per-copy overhead
     // (~8 us per cudaMemcpyAsync): about SNK_HOST_CHUNK_MB of traffic per chunk, at most 16 chunks; only the observation is copied per chunk, the small per-env outputs go down once at the end.
     // (A first chunk of 1/8 size, so that the output copies start earlier, was A/B-measured on one box: 1.365 against 1.363 ms
@@ -1942,8 +1925,7 @@ static int step_fused_host_impl(snk_handle h, snk_replay_s *r, const float *q, f
         if (!q) SNK_CUDA(cudaMemcpyAsync(h->d_act + b, act_idx + b, nb, cudaMemcpyHostToDevice, up));
         SNK_CUDA(cudaEventRecord(h->ev_up[ci], up));
         SNK_CUDA(cudaStreamWaitEvent(st, h->ev_up[ci], 0));
-        int rc = launch_step(h, a, opb ? obs_fmt : SNK_OBS_NONE, q != nullptr, b, e, st);
-        if (rc != SNK_OK) return rc;
+        if ((rc = launch_step(a, opb ? obs_fmt : SNK_OBS_NONE, q != nullptr, b, e, st)) != SNK_OK) return rc;
         SNK_CUDA(cudaEventRecord(h->ev_chunk[ci], st));
         SNK_CUDA(cudaStreamWaitEvent(down, h->ev_chunk[ci], 0));
         if (opb) SNK_CUDA(cudaMemcpyAsync((char *)obs + opb * b, (char *)h->d_obs + opb * b, opb * nb, cudaMemcpyDeviceToHost, down));
@@ -1962,6 +1944,12 @@ static int step_fused_host_impl(snk_handle h, snk_replay_s *r, const float *q, f
     return SNK_OK;
 }
 
+int snk_step_fused_host(snk_handle h, const float *q, float eps, const float *u, const uint8_t *ridx, uint8_t *act_idx,
+                        float *reward, uint8_t *done, void *obs, int obs_fmt, uint8_t *mask, float *ep_return,
+                        int32_t *ep_score) {
+    return step_fused_host_impl(h, nullptr, q, eps, u, ridx, act_idx, reward, done, obs, obs_fmt, mask, ep_return, ep_score);
+}
+
 int snk_step_fused_store_host(snk_handle h, snk_replay r, const float *q, float eps, const float *u, const uint8_t *ridx,
                               uint8_t *act_idx, float *reward, uint8_t *done, void *obs, int obs_fmt, uint8_t *mask,
                               float *ep_return, int32_t *ep_score) {
@@ -1971,52 +1959,30 @@ int snk_step_fused_store_host(snk_handle h, snk_replay r, const float *q, float 
 
 // Per-call getters with HOST outputs (any host memory; pinned is faster).  Unlike the enqueue-and-return entry points these
 // return when the data has arrived: they are what a Julia host calls where the reference reads a field of `game`.
-static int to_host(snk_handle h, void *dst_host, const void *src_dev, size_t bytes) {
-    SNK_CUDA(cudaMemcpyAsync(dst_host, src_dev, bytes, cudaMemcpyDeviceToHost, h->stream));
-    SNK_CUDA(cudaStreamSynchronize(h->stream));
-    return SNK_OK;
-}
-
 int snk_state_host(snk_handle h, void *obs_host, int obs_fmt) {
     SNK_CHECK_HANDLE(h);
-    { int rc0 = staging_guard(h); if (rc0 != SNK_OK) return rc0; }
     SNK_REQUIRE(obs_host != nullptr, "null out");
-    const size_t opb = obs_bytes_per_env(obs_fmt);
+    const size_t opb = obs_bytes(obs_fmt);
     if (opb == 0) return fail(SNK_ERR_INVALID, "unknown obs_fmt %d", obs_fmt);
-    int rc = ensure_obs_staging(h, opb * (size_t)h->n);
-    if (rc != SNK_OK) return rc;
-    if ((rc = snk_state(h, h->d_obs, obs_fmt)) != SNK_OK) return rc;
-    return to_host(h, obs_host, h->d_obs, opb * (size_t)h->n);
+    return get_host(h, obs_host, opb * (size_t)h->n, [&](void *d) { return snk_state(h, d, obs_fmt); });
 }
 
 int snk_losing_mask_host(snk_handle h, uint8_t *mask_3xN_host) {
     SNK_CHECK_HANDLE(h);
-    { int rc0 = staging_guard(h); if (rc0 != SNK_OK) return rc0; }
     SNK_REQUIRE(mask_3xN_host != nullptr, "null out");
-    SNK_CUDA(ensure(&h->d_mask, 3 * (size_t)h->n));
-    int rc = snk_losing_mask(h, h->d_mask);
-    if (rc != SNK_OK) return rc;
-    return to_host(h, mask_3xN_host, h->d_mask, 3 * (size_t)h->n);
+    return get_host(h, mask_3xN_host, 3 * (size_t)h->n, [&](void *d) { return snk_losing_mask(h, (uint8_t *)d); });
 }
 
 int snk_available_actions_host(snk_handle h, uint8_t *dirs_3xN_host) {
     SNK_CHECK_HANDLE(h);
-    { int rc0 = staging_guard(h); if (rc0 != SNK_OK) return rc0; }
     SNK_REQUIRE(dirs_3xN_host != nullptr, "null out");
-    SNK_CUDA(ensure(&h->d_mask, 3 * (size_t)h->n));
-    int rc = snk_available_actions(h, h->d_mask);
-    if (rc != SNK_OK) return rc;
-    return to_host(h, dirs_3xN_host, h->d_mask, 3 * (size_t)h->n);
+    return get_host(h, dirs_3xN_host, 3 * (size_t)h->n, [&](void *d) { return snk_available_actions(h, (uint8_t *)d); });
 }
 
 static int scalars_host(snk_handle h, int which, void *out_host, size_t elem) {
     SNK_CHECK_HANDLE(h);
-    { int rc0 = staging_guard(h); if (rc0 != SNK_OK) return rc0; }
     SNK_REQUIRE(out_host != nullptr, "null out");
-    SNK_CUDA(ensure(&h->d_ep_score, 4 * (size_t)h->n));          // 4 bytes per env covers the u8 and the i32 scalars
-    int rc = scalars(h, which, h->d_ep_score);
-    if (rc != SNK_OK) return rc;
-    return to_host(h, out_host, h->d_ep_score, elem * (size_t)h->n);
+    return get_host(h, out_host, elem * (size_t)h->n, [&](void *d) { return scalars(h, which, d); });
 }
 int snk_get_score_host(snk_handle h, int32_t *score_host) { return scalars_host(h, 0, score_host, 4); }
 int snk_get_done_host(snk_handle h, uint8_t *done_host) { return scalars_host(h, 1, done_host, 1); }
