@@ -1,0 +1,44 @@
+#!/usr/bin/env python3
+"""train! (utils.jl:420-494) on the device: fill the replay ring, then play, sample 64, target, RMSProp update, target sync
+every 1,000 updates, epsilon decay — train.Trainer over the library.  Prints the loss and the moving average of the
+episode returns every --report updates.  Needs a B200.
+
+One play advances every one of --envs games by one step (the reference plays one whole episode of one game per update);
+--updates-per-step sets how many updates follow each play.
+"""
+import argparse
+import os
+import sys
+
+import torch
+
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
+import __graft_entry__ as graft  # noqa: E402
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--envs", type=int, default=4096)
+    ap.add_argument("--batches", type=int, default=20000, help="updates in all (the reference's n_batches)")
+    ap.add_argument("--updates-per-step", type=int, default=1)
+    ap.add_argument("--precision", default="f32", choices=["f32", "bf16"])
+    ap.add_argument("--report", type=int, default=1000)
+    ap.add_argument("--window", type=int, default=1000, help="episodes in the moving average of the returns")
+    args = ap.parse_args()
+    S = graft.load_package()
+    tr = S.train.Trainer(n_envs=args.envs, precision=args.precision, updates_per_step=args.updates_per_step)
+    tr.fill_buffer()
+    print("filled: %d transitions stored, replay %d/%d" % (tr.stored, len(tr.replay), tr.replay.capacity))
+    while tr.n_updates < args.batches:
+        tr.iteration()
+        if tr.n_updates % args.report < args.updates_per_step:
+            rets = tr.episode_returns()
+            avg = float(rets[-args.window:].mean()) if rets.numel() else float("nan")
+            loss = float(torch.stack(tr.losses[-args.report:]).mean())
+            print("batch %7d  loss %.5f  episodes %8d  avg return (last %d) %.3f  epsilon %.4f"
+                  % (tr.n_updates, loss, rets.numel(), args.window, avg, tr.epsilon))
+    print("env errors %d" % tr.env.count_errors())
+
+
+if __name__ == "__main__":
+    main()

@@ -282,6 +282,26 @@ SNK_API int snk_qnet_overflow_host(snk_qnet q, int *flag);
 SNK_API int snk_qnet_sample_grads(snk_qnet q, const float *states, const uint8_t *actions, const double *targets, int64_t B,
                                   void *hi, void *lo, int64_t pitch_elems, float *J_f32, int64_t ldJ, float *loss,
                                   void *cuda_stream);
+/* ---- the learner  utils.jl:452-472 ------------------------------------------------------------------------------------
+ * snk_qnet_train_step: Flux.gradient of mean(huber(q_net(s)[a], y)) + Flux.Optimise.update!(RMSProp(eta, rho, epsilon), θ, g)
+ * on the device (utils.jl:452-466).  g = Float32(Σ_i J_i / B) with J_i the rows of snk_qnet_sample_grads, summed in Float64
+ * in sample order; then acc = Float32(rho acc + (1 - rho) g g), θ -= Float32(g eta / (sqrt(acc) + epsilon)) in Float64 with
+ * a Float32 sqrt (Flux.Optimise's promotions).  Inputs as for snk_qnet_sample_grads, B >= 1.  acc = the optimiser's state for
+ * θ (181,395 f32, caller-owned, zero-initialised = a fresh RMSProp).  Every device layout of the handle (both forward
+ * precisions, the gradient kernel's copy) follows the new θ.  grad_out (181,395 f32, g) and loss_out (1 f32, the batch mean of
+ * the per-sample losses) are optional.  SNK_QNET_F32: a θ outside the fp16 range sets the snk_qnet_overflow_host flag.
+ * snk_qnet_set_params: θ = theta_dev (181,395 f32 on the handle's device, e.g. another handle's snk_qnet_params), every
+ * layout re-derived: update_target_net! (utils.jl:469-472).  snk_qnet_params: the handle's own θ, Flux.destructure order,
+ * read-only; it changes with every train step.
+ * Both updates enqueue on cuda_stream and return.  The caller orders a train step or set_params and any other call on the
+ * same handle (forward, sample_grads, a set_params reading its θ): the same stream, or an event.  The next snk_qnet_forward
+ * waits on the host for the update's copy of conv1's 304 weights (they are kernel parameters), so it fails with
+ * SNK_ERR_INVALID inside a stream capture: run one forward after an update outside the capture. */
+SNK_API int snk_qnet_train_step(snk_qnet q, const float *states, const uint8_t *actions, const double *targets, int64_t B,
+                                float *acc, double eta, double rho, double epsilon, float *grad_out, float *loss_out,
+                                void *cuda_stream);
+SNK_API int snk_qnet_set_params(snk_qnet q, const float *theta_dev, void *cuda_stream);   /* update_target_net!, utils.jl:469-472 */
+SNK_API int snk_qnet_params(snk_qnet q, const float **theta_dev);
 /* profiling aid (SNK_QNET_BF16): device buffer of 512 int64 that receives clock64 stamps of the conv phases of CTA 0 on every
  * later forward (64 slots for each of its first 8 iterations, tools/qnet_phases17.py); NULL switches it off */
 SNK_API int snk_qnet_debug_timing(snk_qnet q, long long *device_buf);

@@ -148,6 +148,8 @@ def lib():
         "snk_qnet_forward": [vp, vp, i64, vp, vp], "snk_qnet_precision": [vp, C.POINTER(i32)],
         "snk_qnet_overflow_host": [vp, C.POINTER(i32)], "snk_qnet_debug_timing": [vp, vp],
         "snk_qnet_sample_grads": [vp, vp, vp, vp, i64, vp, vp, i64, vp, i64, vp, vp],
+        "snk_qnet_train_step": [vp, vp, vp, vp, i64, vp, f64, f64, f64, vp, vp, vp],
+        "snk_qnet_set_params": [vp, vp, vp], "snk_qnet_params": [vp, C.POINTER(vp)],
         "snk_gram_workspace_bytes": [i64, i64, i32, C.POINTER(C.c_size_t)],
         "snk_gram_pack": [vp, i32, i64, i64, vp, vp],
         "snk_gram": [vp, i64, i64, i32, i32, i32, vp, vp],
@@ -673,4 +675,4 @@ class ReplayBuffer:
 
 
 from . import shard  # noqa: E402,F401
-from . import bson_io, laplace, qnet, rollout  # noqa: E402,F401
+from . import bson_io, laplace, qnet, rollout, train  # noqa: E402,F401

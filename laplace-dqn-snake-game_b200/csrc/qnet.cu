@@ -41,6 +41,7 @@
 #include <vector>
 
 #include "common.h"
+#include "qnet_theta.h"
 
 namespace snk {
 namespace qgrad {       // qnet_grads.cu
@@ -1150,8 +1151,8 @@ __global__ void __launch_bounds__(HB_THREADS, 1) k_qnet_head(const __grid_consta
     }
 }
 
-// ---- host: parameter packing ------------------------------------------------------------------------------
-static uint16_t f2bf(float f) {            // round-to-nearest-even
+// ---- parameter packing (host: pack_params at create; device: k_qnet_train_apply after every update) ----------------
+__host__ __device__ static inline uint16_t f2bf(float f) {            // round-to-nearest-even
     uint32_t u;
     memcpy(&u, &f, 4);
     if ((u & 0x7F800000u) == 0x7F800000u) return (uint16_t)(u >> 16);
@@ -1159,7 +1160,7 @@ static uint16_t f2bf(float f) {            // round-to-nearest-even
     return (uint16_t)(u >> 16);
 }
 // w = hi + lo in fp16 (lo unscaled): part 0 = lo, part 1 = hi
-static uint16_t f2h_part(float w, int part) {
+__host__ __device__ static inline uint16_t f2h_part(float w, int part) {
     const __half h = __float2half_rn(w);
     if (part) return __half_as_ushort(h);
     return __half_as_ushort(__float2half_rn(w - __half2float(h)));
@@ -1228,6 +1229,109 @@ static void pack_params(const float *th, std::vector<uint8_t> &blob) {
     memcpy(blob.data() + P_B5, b5, 12);
 }
 
+// pack_params + build_theta_ext for ONE parameter, as a scatter from its Flux index p: writes every byte the host packers derive
+// from theta[p], with the same rounding, so a blob updated on the device equals the blob snk_qnet_create would build from the
+// new theta byte for byte.  `theta` is the handle's extended copy (the two re-ordered W3 copies behind it).
+__device__ __forceinline__ void scatter_param(float w, int p, float *theta, uint8_t *params) {
+    using namespace qgrad;
+    auto h = [&](size_t off) { return reinterpret_cast<uint16_t *>(params + off); };
+    auto f = [&](size_t off) { return reinterpret_cast<float *>(params + off); };
+    theta[p] = w;
+    if (p < O_B1) {                                     // W1 (3,3,2,16) -> [tap = k2*3 + k1][c][o], flipped: k = 2 - a
+        const int a1 = p % 3, a2 = (p / 3) % 3, c = (p / 9) % 2, o = p / 18;
+        f(P_W1)[(((2 - a2) * 3 + (2 - a1)) * 2 + c) * 16 + o] = w;
+    } else if (p < O_W2) {
+        f(P_BIAS)[p - O_B1] = w;
+    } else if (p < O_B2) {                              // W2 (3,3,16,32) -> [k2][k1][chunk][o][8]; split: [k2][k1][chunk][hi|lo o][8]
+        const int i = p - O_W2, a1 = i % 3, a2 = (i / 3) % 3, c = (i / 9) % 16, o = i / 144;
+        const int kc = ((2 - a2) * 3 + (2 - a1)) * 2 + c / 8;
+        h(P_W2)[(kc * 32 + o) * 8 + c % 8] = f2bf(w);
+        h(P_S_W2)[(kc * 64 + o) * 8 + c % 8] = f2h_part(w, 1);
+        h(P_S_W2)[(kc * 64 + 32 + o) * 8 + c % 8] = f2h_part(w, 0);
+    } else if (p < O_W3) {
+        f(P_BIAS)[16 + p - O_B2] = w;
+    } else if (p < O_B3) {                              // W3 (6,6,32,64): the gradient kernel's two copies and both tensor-core layouts
+        const int i = p - O_W3, t = i % 36, c = (i / 36) % 32, o = i / 1152;
+        theta[O_W3OF + (c * 36 + t) * 64 + o] = w;
+        theta[O_W3CF + (o * 36 + t) * 32 + c] = w;
+        const int k1 = 5 - t % 6, k2 = 5 - t / 6, m = c / 16, kk = c % 16;
+        auto core = [&](int R) { return (((kk / 8) * 16 + R / 8) * 8 + R % 8) * 8 + kk % 8; };
+        h(P_W3B)[(size_t)(((k2 / 2) * 6 + k1) * 2 + m) * 2048 + core(64 * (k2 % 2) + o)] = f2bf(w);
+        const size_t blk = (size_t)((k2 * 6 + k1) * 2 + m) * 2048;
+        h(P_S_W3)[blk + core(o)] = f2h_part(w, 1);
+        h(P_S_W3)[blk + core(64 + o)] = f2h_part(w, 0);
+    } else if (p < O_W4) {
+        f(P_BIAS)[48 + p - O_B3] = w;
+    } else if (p < O_B4) {                              // W4 (64,1600), kF = x + 5 y + 25 c -> [n][(y*5 + x)*64 + c]
+        const int i = p - O_W4, n = i % 64, kF = i / 64;
+        const size_t k = (size_t)((kF / 5) % 5 * 5 + kF % 5) * 64 + kF / 25;
+        h(P_W4)[(size_t)n * 1600 + k] = f2bf(w);
+        h(P_S_W4)[(size_t)n * 1600 + k] = f2h_part(w, 1);
+        h(P_S_W4)[(size_t)(64 + n) * 1600 + k] = f2h_part(w, 0);
+    } else if (p < O_W5) {
+        f(P_B4)[p - O_B4] = w;
+    } else if (p < O_B5) {
+        f(P_W5)[p - O_W5] = w;
+    } else {
+        f(P_B5)[p - O_B5] = w;
+    }
+}
+
+struct ApplyArgs {
+    const float *rows;           // [nrows][NP] per-sample gradient rows of one chunk of the minibatch (k_sample_grads), or NULL:
+    const float *losses;         //   no update, theta_src is the new theta (snk_qnet_set_params);  [nrows] per-sample losses
+    int nrows;
+    int first, last;             // the chunk is the first / the last of the minibatch
+    double *gsum;                // [NP + 1] Float64 running sums carried between chunks; [NP] = the loss
+    long long B;
+    const float *theta_src;
+    float *acc;                  // RMSProp state of theta
+    double eta, rho, one_m_rho, eps;
+    float *grad_out, *loss_out;  // optional
+    float *theta;                // the handle's extended theta
+    uint8_t *params;             // the handle's packed blob
+    int *overflow;               // SNK_QNET_F32: a parameter left the fp16 range of the split operands; NULL in bf16 mode
+};
+
+// One thread per parameter (thread NP: the loss).  g = Float32(sum_i J_i / B), the sum a Float64 running sum in sample order,
+// rounded once: the order depends on B only.  Then Flux.Optimise's RMSProp (apply! + update!, utils.jl:466) with Julia's
+// promotions: Float64 hyper-parameters, Float32 arrays, every operation rounded on its own (no FMA contraction).
+constexpr int APPLY_THREADS = 256;
+__global__ void __launch_bounds__(APPLY_THREADS) k_qnet_train_apply(const ApplyArgs a) {
+    using qgrad::NP;
+    const int p = blockIdx.x * APPLY_THREADS + threadIdx.x;
+    if (p > NP) return;
+    float w;
+    if (a.rows != nullptr) {
+        const float *src = p < NP ? a.rows + p : a.losses;
+        const long long ld = p < NP ? NP : 1;
+        double s = a.first ? 0.0 : a.gsum[p];
+#pragma unroll 8
+        for (int r = 0; r < a.nrows; r++) s = __dadd_rn(s, (double)src[r * ld]);
+        if (!a.last) {
+            a.gsum[p] = s;
+            return;
+        }
+        const float g = (float)__ddiv_rn(s, (double)a.B);
+        if (p == NP) {
+            if (a.loss_out != nullptr) *a.loss_out = g;
+            return;
+        }
+        if (a.grad_out != nullptr) a.grad_out[p] = g;
+        const double gd = (double)g;
+        // acc = rho acc + (1 - rho) g g;  delta = g (eta / (sqrt(acc) + eps)), sqrt in Float32;  theta -= delta
+        const float acc = (float)__dadd_rn(__dmul_rn(a.rho, (double)a.acc[p]), __dmul_rn(__dmul_rn(a.one_m_rho, gd), gd));
+        a.acc[p] = acc;
+        const float delta = (float)__dmul_rn(gd, __ddiv_rn(a.eta, __dadd_rn((double)__fsqrt_rn(acc), a.eps)));
+        w = __fsub_rn(a.theta[p], delta);
+    } else {
+        if (p == NP) return;
+        w = a.theta_src[p];
+    }
+    if (a.overflow != nullptr && !(fabsf(w) <= 65504.0f)) *a.overflow = 1;
+    scatter_param(w, p, a.theta, a.params);
+}
+
 typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
                                   const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
                                   CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
@@ -1275,7 +1379,42 @@ struct snk_qnet_s {
     long long out3_cap;          // in samples
     int *d_overflow;             // SNK_QNET_F32: an activation left the fp16 range
     int sms;
+    // learner (snk_qnet_train_step): per-sample gradient rows of one chunk of the minibatch, grown on demand up to 2 * sms samples
+    float *rows;
+    float *row_loss;
+    double *gsum;                // NP + 1 running sums carried between chunks
+    long long rows_cap;          // in samples
+    // conv1's weights are kernel parameters read from w1h / b1h / w1f / b1f (DESIGN §5b): a device-side update copies them into
+    // conv1_host and records conv1_ready; the next forward waits for that event and rebuilds the host fields before its launch
+    float *conv1_host;           // pinned: P_W1 (288) then b1 (16)
+    cudaEvent_t conv1_ready;
+    int conv1_pending;
 };
+
+static void set_conv1(snk_qnet_s *q, const float *w1f, const float *b1f) {
+    for (int i = 0; i < 144; i++) q->w1h[i] = __floats2half2_rn(w1f[2 * i], w1f[2 * i + 1]);
+    for (int i = 0; i < 8; i++) q->b1h[i] = __floats2half2_rn(b1f[2 * i], b1f[2 * i + 1]);
+    memcpy(q->w1f, w1f, sizeof(q->w1f));
+    memcpy(q->b1f, b1f, sizeof(q->b1f));
+}
+
+// after k_qnet_train_apply: bring conv1's new weights to the host (the forward launches read them from there)
+static int enqueue_conv1_refresh(snk_qnet_s *q, cudaStream_t st) {
+    SNK_CUDA(cudaMemcpyAsync(q->conv1_host, q->params + P_W1, 288 * 4, cudaMemcpyDeviceToHost, st));
+    SNK_CUDA(cudaMemcpyAsync(q->conv1_host + 288, q->params + P_BIAS, 16 * 4, cudaMemcpyDeviceToHost, st));
+    SNK_CUDA(cudaEventRecord(q->conv1_ready, st));
+    q->conv1_pending = 1;
+    return SNK_OK;
+}
+
+static int launch_apply(snk_qnet_s *q, ApplyArgs &a, cudaStream_t st) {
+    a.theta = q->theta;
+    a.params = q->params;
+    a.overflow = q->precision == SNK_QNET_F32 ? q->d_overflow : nullptr;
+    k_qnet_train_apply<<<(qgrad::NP + APPLY_THREADS) / APPLY_THREADS, APPLY_THREADS, 0, st>>>(a);
+    SNK_CUDA(cudaGetLastError());
+    return SNK_OK;
+}
 
 extern "C" {
 
@@ -1297,14 +1436,7 @@ int snk_qnet_create(snk_qnet *out, const float *theta_host, int64_t n_params, in
     if (q == nullptr) return fail(SNK_ERR_INVALID, "out of host memory");
     q->device = device;
     q->precision = precision;
-    {
-        const float *w1f = reinterpret_cast<const float *>(blob.data() + P_W1);
-        const float *b1f = reinterpret_cast<const float *>(blob.data() + P_BIAS);
-        for (int i = 0; i < 144; i++) q->w1h[i] = __floats2half2_rn(w1f[2 * i], w1f[2 * i + 1]);
-        for (int i = 0; i < 8; i++) q->b1h[i] = __floats2half2_rn(b1f[2 * i], b1f[2 * i + 1]);
-        memcpy(q->w1f, w1f, sizeof(q->w1f));
-        memcpy(q->b1f, b1f, sizeof(q->b1f));
-    }
+    set_conv1(q, reinterpret_cast<const float *>(blob.data() + P_W1), reinterpret_cast<const float *>(blob.data() + P_BIAS));
     cudaDeviceGetAttribute(&q->sms, cudaDevAttrMultiProcessorCount, device);
     cudaError_t e = cudaMalloc((void **)&q->params, blob.size());
     if (e == cudaSuccess) e = cudaMemcpy(q->params, blob.data(), blob.size(), cudaMemcpyHostToDevice);
@@ -1314,10 +1446,13 @@ int snk_qnet_create(snk_qnet *out, const float *theta_host, int64_t n_params, in
     if (e == cudaSuccess) e = cudaMemcpy(q->theta, ext.data(), ext.size() * 4, cudaMemcpyHostToDevice);
     if (e == cudaSuccess) e = cudaMalloc((void **)&q->d_overflow, sizeof(int));
     if (e == cudaSuccess) e = cudaMemset(q->d_overflow, 0, sizeof(int));
+    if (e == cudaSuccess) e = cudaMallocHost((void **)&q->conv1_host, 304 * 4);
+    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&q->conv1_ready, cudaEventDisableTiming);
     if (e != cudaSuccess) {
         if (q->params) cudaFree(q->params);
         if (q->theta) cudaFree(q->theta);
         if (q->d_overflow) cudaFree(q->d_overflow);
+        if (q->conv1_host) cudaFreeHost(q->conv1_host);
         delete q;
         return fail(SNK_ERR_CUDA, "snk_qnet_create: %s", cudaGetErrorString(e));
     }
@@ -1332,7 +1467,67 @@ int snk_qnet_destroy(snk_qnet q) {
     if (q->theta) cudaFree(q->theta);
     if (q->out3) cudaFree(q->out3);
     if (q->d_overflow) cudaFree(q->d_overflow);
+    if (q->rows) cudaFree(q->rows);
+    if (q->row_loss) cudaFree(q->row_loss);
+    if (q->gsum) cudaFree(q->gsum);
+    if (q->conv1_ready) cudaEventDestroy(q->conv1_ready);
+    if (q->conv1_host) cudaFreeHost(q->conv1_host);
     delete q;
+    return SNK_OK;
+}
+
+// Flux.gradient of mean(huber(q_net(s)[a], y)) + update!(RMSProp(eta, rho, epsilon), theta, g) (utils.jl:452-466): the
+// per-sample rows of k_sample_grads, chunk by chunk, reduced and applied by k_qnet_train_apply, which also re-derives every
+// device layout of the weights
+int snk_qnet_train_step(snk_qnet q, const float *states, const uint8_t *actions, const double *targets, int64_t B, float *acc,
+                        double eta, double rho, double epsilon, float *grad_out, float *loss_out, void *cuda_stream) {
+    SNK_REQUIRE(B >= 1, "B must be >= 1");
+    SNK_REQUIRE(eta > 0.0 && rho >= 0.0 && rho < 1.0 && epsilon >= 0.0, "RMSProp needs eta > 0, 0 <= rho < 1 and epsilon >= 0");
+    SNK_REQUIRE(q != nullptr && states != nullptr && actions != nullptr && targets != nullptr && acc != nullptr, "null argument");
+    DeviceGuard guard(q->device);
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    const long long chunk = 2ll * q->sms;          // one CTA of k_sample_grads per sample and slot; bounds the scratch (215 MB)
+    const long long need = B < chunk ? B : chunk;
+    if (q->rows_cap < need) {
+        SNK_CUDA(cudaStreamSynchronize(st));
+        if (q->rows) { SNK_CUDA(cudaFree(q->rows)); q->rows = nullptr; }
+        if (q->row_loss) { SNK_CUDA(cudaFree(q->row_loss)); q->row_loss = nullptr; }
+        q->rows_cap = 0;
+        SNK_CUDA(cudaMalloc((void **)&q->rows, (size_t)need * qgrad::NP * 4));
+        SNK_CUDA(cudaMalloc((void **)&q->row_loss, (size_t)need * 4));
+        if (q->gsum == nullptr) SNK_CUDA(cudaMalloc((void **)&q->gsum, (qgrad::NP + 1) * sizeof(double)));
+        q->rows_cap = need;
+    }
+    ApplyArgs a = {};
+    a.rows = q->rows; a.losses = q->row_loss; a.gsum = q->gsum; a.B = B;
+    a.acc = acc; a.eta = eta; a.rho = rho; a.one_m_rho = 1.0 - rho; a.eps = epsilon;
+    a.grad_out = grad_out; a.loss_out = loss_out;
+    for (long long s0 = 0; s0 < B; s0 += chunk) {
+        const long long n = B - s0 < chunk ? B - s0 : chunk;
+        int rc = qgrad::launch_sample_grads(q->theta, states + s0 * 200, actions + s0, targets + s0, n, nullptr, nullptr, 0, q->rows,
+                                            qgrad::NP, q->row_loss, q->sms, st);
+        if (rc != SNK_OK) return rc;
+        a.nrows = (int)n; a.first = s0 == 0; a.last = s0 + n == B;
+        if ((rc = launch_apply(q, a, st)) != SNK_OK) return rc;
+    }
+    return enqueue_conv1_refresh(q, st);
+}
+
+// theta <- theta_dev (update_target_net!, utils.jl:469-472): the same kernel without a gradient re-derives every layout
+int snk_qnet_set_params(snk_qnet q, const float *theta_dev, void *cuda_stream) {
+    SNK_REQUIRE(q != nullptr && theta_dev != nullptr, "null argument");
+    DeviceGuard guard(q->device);
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    ApplyArgs a = {};
+    a.theta_src = theta_dev;
+    int rc = launch_apply(q, a, st);
+    if (rc != SNK_OK) return rc;
+    return enqueue_conv1_refresh(q, st);
+}
+
+int snk_qnet_params(snk_qnet q, const float **theta_dev) {
+    SNK_REQUIRE(q != nullptr && theta_dev != nullptr, "null argument");
+    *theta_dev = q->theta;
     return SNK_OK;
 }
 
@@ -1379,6 +1574,17 @@ int snk_qnet_forward(snk_qnet q, const float *obs_f32, int64_t N, float *q_out_3
     DeviceGuard guard(q->device);
     cudaStream_t st = (cudaStream_t)cuda_stream;
     const bool f32 = q->precision == SNK_QNET_F32;
+    if (q->conv1_pending) {
+        cudaStreamCaptureStatus cs = cudaStreamCaptureStatusNone;
+        SNK_CUDA(cudaStreamIsCapturing(st, &cs));
+        if (cs != cudaStreamCaptureStatusNone)
+            return fail(SNK_ERR_INVALID, "snk_qnet_forward: the weights of this handle changed on the device (snk_qnet_train_step / "
+                                         "snk_qnet_set_params) and conv1's kernel parameters must be fetched by the host first: "
+                                         "run one forward outside the stream capture");
+        SNK_CUDA(cudaEventSynchronize(q->conv1_ready));
+        set_conv1(q, q->conv1_host, q->conv1_host + 288);
+        q->conv1_pending = 0;
+    }
     const size_t row_bytes = f32 ? 2 * 1600 * 2 : 1600 * 2;             // per sample
     if (q->out3_cap < N) {
         if (q->out3) { SNK_CUDA(cudaStreamSynchronize(st)); SNK_CUDA(cudaFree(q->out3)); q->out3 = nullptr; q->out3_cap = 0; }

@@ -13,7 +13,7 @@ module SnakeB200
 export BatchedSnakeGame, available_actions, step!, step_fused!, virtual_step, assemble_state!,
        epsilon_greedy, masked_target, center_columns!, reset!, set_food_list!, score, lost,
        DeviceReplayBuffer, store_step!, store_step_host!, store_step_host_bits!, stack_exp, sample_indices, DeviceQNet, forward!, overflowed,
-       sample_grads!, store_snapshot!, gram!, sample_model_weights!, empty_buffer!, patch_reset_obs!,
+       sample_grads!, RMSPropState, train_step!, update_target_net!, params_device, store_snapshot!, gram!, sample_model_weights!, empty_buffer!, patch_reset_obs!,
        GramShard, export_handle, connect!, run!, planes,
        step_device!, step_abs_device!, step_fused_device!, rollout_device!, state_device!, losing_mask_device!,
        lost_device!, steps_device!, error_flags_device!, count_errors, seed!, set_stream!, num_envs, library_version,
@@ -328,6 +328,45 @@ sample_grads!(q::DeviceQNet, d_states::Ptr{Float32}, d_actions::Ptr{UInt8}, d_ta
                 (Ptr{Cvoid}, Ptr{Float32}, Ptr{UInt8}, Ptr{Float64}, Int64, Ptr{Cvoid}, Ptr{Cvoid}, Int64, Ptr{Float32}, Int64,
                  Ptr{Float32}, Ptr{Cvoid}),
                 q.handle, d_states, d_actions, d_targets, B, d_hi, d_lo, pitch, d_J, ldJ, d_loss, C_NULL))
+
+# ---- the learner (utils.jl:452-472) --------------------------------------------------------------------------------
+"""Flux.Optimise.RMSProp(eta, rho, epsilon) (structs.jl:137: RMSProp(5e-4) = (0.0005, 0.9, 1e-8)) and its state for θ:
+181,395 Float32 on `device`, zero-initialised here (a fresh optimiser), freed with the object."""
+mutable struct RMSPropState
+    d_acc::Ptr{Float32}
+    eta::Float64
+    rho::Float64
+    epsilon::Float64
+    function RMSPropState(; eta::Real = 5e-4, rho::Real = 0.9, epsilon::Real = 1e-8, device::Integer = 0)
+        p, _ = device_alloc(181395 * 4, device; compressible = false)
+        zero = zeros(Float32, 181395)
+        check(ccall((:snk_copy_async, lib), Cint, (Ptr{Cvoid}, Ptr{Float32}, Csize_t, Ptr{Cvoid}), p, zero, sizeof(zero), C_NULL))
+        o = new(Ptr{Float32}(p), eta, rho, epsilon)
+        finalizer(x -> device_free(Ptr{Cvoid}(x.d_acc)), o)
+        return o
+    end
+end
+
+"""One minibatch update of `q` on the device (utils.jl:452-466): Flux.gradient of mean(huber(q_net(s)[a], y)) and
+update!(opt, θ, g).  Device pointers as for `sample_grads!`; d_grad (181,395 Float32) and d_loss (1 Float32, the batch mean)
+optional.  Enqueued on the default stream; order it with any forward of `q` (the same stream does)."""
+train_step!(q::DeviceQNet, opt::RMSPropState, d_states::Ptr{Float32}, d_actions::Ptr{UInt8}, d_targets::Ptr{Float64}, B::Integer;
+            d_grad::Ptr{Float32} = Ptr{Float32}(C_NULL), d_loss::Ptr{Float32} = Ptr{Float32}(C_NULL)) =
+    check(ccall((:snk_qnet_train_step, lib), Cint,
+                (Ptr{Cvoid}, Ptr{Float32}, Ptr{UInt8}, Ptr{Float64}, Int64, Ptr{Float32}, Cdouble, Cdouble, Cdouble, Ptr{Float32},
+                 Ptr{Float32}, Ptr{Cvoid}),
+                q.handle, d_states, d_actions, d_targets, B, opt.d_acc, opt.eta, opt.rho, opt.epsilon, d_grad, d_loss, C_NULL))
+
+"""θ of `q` on the device (Flux.destructure order, 181,395 Float32): read-only, changes with every update"""
+function params_device(q::DeviceQNet)
+    p = Ref{Ptr{Float32}}(C_NULL)
+    check(ccall((:snk_qnet_params, lib), Cint, (Ptr{Cvoid}, Ref{Ptr{Float32}}), q.handle, p))
+    return p[]
+end
+
+"""update_target_net! (utils.jl:469-472): t's parameters become a copy of q's, on the device"""
+update_target_net!(t::DeviceQNet, q::DeviceQNet) =
+    check(ccall((:snk_qnet_set_params, lib), Cint, (Ptr{Cvoid}, Ptr{Float32}, Ptr{Cvoid}), t.handle, params_device(q), C_NULL))
 
 # ---- Laplace deviation matrix (compute_D.jl, plot_traj.jl, la_utils.jl) ----------------------------------------
 """deviation_matrix[:, position] = Float64.(theta) (compute_D.jl:67-71); position is 1-based like Julia's."""

@@ -5,7 +5,8 @@
 
 `QNet` hands Flux.destructure(q_net) to snk_qnet_create and runs snk_qnet_forward (tcgen05 implicit-GEMM convolutions,
 csrc/qnet.cu).  precision="f32" (default) is the Float32-faithful mode the reference's Float32 network needs for
-identical greedy actions; precision="bf16" is the fast, lower-precision mode.  There is no library (cuDNN) path in the
+identical greedy actions; precision="bf16" is the fast, lower-precision mode.  QNet.train_step with an RMSProp is the learner of train!
+(utils.jl:452-466) on the device; load_params_from is update_target_net!.  There is no library (cuDNN) path in the
 product: the torch restatement used as a timing baseline and cross-check lives in tools/torch_qnet.py.
 """
 import ctypes as C
@@ -61,13 +62,14 @@ class QNet:
         if self.device.type != "cuda":
             raise ValueError("QNet runs on a CUDA device only (no CPU fallback)")
         self.precision = precision
-        self.theta = np.ascontiguousarray(bson_io.destructure(layers), dtype=np.float32)
-        if self.theta.size != N_PARAMS:
+        self._theta = np.ascontiguousarray(bson_io.destructure(layers), dtype=np.float32)
+        if self._theta.size != N_PARAMS:
             raise ValueError("the native Q-net is the two-frame network of structs.jl:127-139 (%d parameters), got %d"
-                             % (N_PARAMS, self.theta.size))
-        self.n_params = int(self.theta.size)
+                             % (N_PARAMS, self._theta.size))
+        self.n_params = int(self._theta.size)
+        self._updated = False          # theta changed on the device since create (train_step / load_params_from)
         self._q = C.c_void_p()
-        _check(lib().snk_qnet_create(C.byref(self._q), self.theta.ctypes.data_as(C.c_void_p), self.theta.size,
+        _check(lib().snk_qnet_create(C.byref(self._q), self._theta.ctypes.data_as(C.c_void_p), self._theta.size,
                                      self.device.index or 0, PRECISIONS[precision]))
 
     def close(self):
@@ -120,9 +122,80 @@ class QNet:
                                            _ptr(out.get("loss")), st))
         return out
 
+    @property
+    def theta(self):
+        """Flux.destructure(q_net): (181,395) float32 numpy array of the current parameters (downloaded after an update)."""
+        if self._updated:
+            return self.theta_device.cpu().numpy()
+        return self._theta
+
+    @property
+    def theta_device(self):
+        """The net's own parameters on the device, (181,395) float32 in Flux.destructure order: a view, read-only, that changes
+        with every train_step / load_params_from."""
+        from . import _check, lib
+        p = C.c_void_p()
+        _check(lib().snk_qnet_params(self._q, C.byref(p)))
+        return torch.as_tensor(_ParamsView(self, p.value), device=self.device)
+
+    def train_step(self, states, actions, targets, opt, want_grad=False):
+        """One minibatch update (utils.jl:452-466): Flux.gradient of mean(huber(q_net(s)[a], y)) and update!(opt, theta, g),
+        on the device; every layout of this net (both forward precisions, sample_grads) follows the new theta.
+        states (B,2,10,10) f32, actions (B) u8 (0-based), targets (B) f64 as for sample_grads; opt an RMSProp.
+        Returns (loss, g): loss a 0-d f32 tensor (the batch mean), g (181,395) f32 if want_grad else None.  Enqueued on the
+        current stream."""
+        from . import _check, _ptr, lib
+        B = states.shape[0]
+        dev = self.device
+        acc = opt.state(dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        g = torch.empty(N_PARAMS, dtype=torch.float32, device=dev) if want_grad else None
+        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _check(lib().snk_qnet_train_step(self._q, _ptr(states, torch.float32, B * 200, dev), _ptr(actions, torch.uint8, B, dev),
+                                         _ptr(targets, torch.float64, B, dev), B, _ptr(acc, torch.float32, N_PARAMS, dev),
+                                         opt.eta, opt.rho, opt.epsilon, _ptr(g), _ptr(loss), st))
+        self._updated = True
+        return loss, g
+
+    def load_params_from(self, other):
+        """update_target_net! (utils.jl:469-472): this net's parameters become a copy of `other`'s (a QNet on the same device,
+        either precision), on the device, enqueued on the current stream."""
+        from . import _check, lib
+        if other.device != self.device:
+            raise ValueError("load_params_from: nets on %s and %s" % (other.device, self.device))
+        p = C.c_void_p()
+        _check(lib().snk_qnet_params(other._q, C.byref(p)))
+        st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        _check(lib().snk_qnet_set_params(self._q, p, st))
+        self._updated = True
+
     def overflow(self):
         """f32 mode: True if an activation left the fp16 range of the split operands since the last call (synchronises)."""
         from . import _check, lib
         f = C.c_int(0)
         _check(lib().snk_qnet_overflow_host(self._q, C.byref(f)))
         return bool(f.value)
+
+
+class _ParamsView:
+    """__cuda_array_interface__ of a QNet's device theta; keeps the net alive as long as a tensor views it."""
+
+    def __init__(self, net, ptr):
+        self.net = net
+        self.__cuda_array_interface__ = {"shape": (N_PARAMS,), "typestr": "<f4", "data": (ptr, False), "version": 3,
+                                         "strides": None, "stream": None}
+
+
+class RMSProp:
+    """Flux.Optimise.RMSProp(eta, rho, epsilon) of the reference's trainer (structs.jl:137: RMSProp(5e-4), stored as
+    (0.0005, 0.9, 1e-8)).  `acc` is its state for theta: (181,395) f32 on the net's device, zero on the first update (a fresh
+    optimiser); an ordinary tensor, so it can be saved and restored with the parameters."""
+
+    def __init__(self, eta=5e-4, rho=0.9, epsilon=1e-8, acc=None):
+        self.eta, self.rho, self.epsilon = float(eta), float(rho), float(epsilon)
+        self.acc = acc
+
+    def state(self, device):
+        if self.acc is None:
+            self.acc = torch.zeros(N_PARAMS, dtype=torch.float32, device=device)
+        return self.acc
