@@ -24,11 +24,11 @@
 // Two TMEM accumulator stages (2 x 256 columns): the tensor core fills one while the other is drained.
 // Work item = (128 x 256 output tile, split of the contraction); partial tiles are reduced (deterministically)
 // by k_gram_finish, which also mirrors the upper triangle of a symmetric problem.
-#include <cuda.h>
 #include <cuda_bf16.h>
 #include <string.h>
 
 #include "common.h"
+#include "sm100.h"
 
 namespace snk {
 namespace gram {
@@ -56,103 +56,9 @@ struct Cfg {
     static constexpr int STAGES = (200 * 1024) / STAGE_BYTES > 8 ? 8 : (200 * 1024) / STAGE_BYTES;
     static constexpr int CH = chunk_k<TERMS>() / BK;                            // k-blocks per TMEM accumulation chunk
     static constexpr int SMEM_BYTES = STAGES * STAGE_BYTES + 1024 /*align*/ + 256 /*barriers*/;
-    static constexpr uint64_t LAYOUT = (BK == 64) ? 2ull /*SWIZZLE_128B*/ : 4ull /*SWIZZLE_64B*/;
-    static constexpr uint64_t SBO = (8 * ROW_BYTES) >> 4;                      // 8-row swizzle atom pitch
+    static constexpr uint64_t LAYOUT = (BK == 64) ? LAYOUT_SW128 : LAYOUT_SW64;
+    static constexpr uint32_t SBO_BYTES = 8 * ROW_BYTES;                       // 8-row swizzle atom pitch
 };
-
-// ---- PTX wrappers --------------------------------------------------------------------------------
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile(
-        "{\n\t.reg .pred P1;\n\t"
-        "mbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\t"
-        "selp.b32 %0, 1, 0, P1;\n\t}"
-        : "=r"(ok)
-        : "r"(smem_u32(bar)), "r"(parity)
-        : "memory");
-    return ok != 0;
-}
-// Bounded wait: a protocol bug must fault (trap), never hang the GPU.
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {
-    if (mbar_try_wait(bar, parity)) return;
-    const long long t0 = clock64();
-    while (!mbar_try_wait(bar, parity)) {
-        if (clock64() - t0 > 4000000000ll) {   // ~2 s
-            printf("snk gram: mbarrier wait timed out (block %d thread %d)\n", blockIdx.x, threadIdx.x);
-            __trap();
-        }
-    }
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-
-__device__ __forceinline__ void tma_load_2d(const CUtensorMap *map, uint64_t *bar, void *dst, int c_inner, int c_row) {
-    asm volatile(
-        "cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-        ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c_inner), "r"(c_row)
-        : "memory");
-}
-__device__ __forceinline__ void tma_prefetch_desc(const CUtensorMap *map) {
-    asm volatile("prefetch.tensormap [%0];" ::"l"((uint64_t)map) : "memory");
-}
-
-__device__ __forceinline__ void tmem_alloc(uint32_t *dst_smem, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-
-// D[tmem] (+)= A[smem] * B[smem]^T ; both operands K-major
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile(
-        "{\n\t.reg .pred p;\n\t"
-        "setp.ne.b32 p, %4, 0;\n\t"
-        "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-        ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate)
-        : "memory");
-}
-// arrives on the mbarrier once all previously issued MMAs of this thread have completed
-__device__ __forceinline__ void umma_commit(uint64_t *bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&v)[32]) {
-    asm volatile(
-        "tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-        "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, "
-        "%16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-        : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-          "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]),
-          "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]), "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]),
-          "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]), "=r"(v[31])
-        : "r"(taddr)
-        : "memory");
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-
-// K-major shared-memory operand descriptor (cute::UMMA::SmemDescriptor bit layout):
-//   [0,14) start address >> 4 | [16,30) leading byte offset >> 4 (1: unused for swizzled K-major)
-//   [32,46) stride byte offset >> 4 (pitch between 8-row swizzle atoms) | [46,48) version = 1 | [61,64) swizzle mode
-template <int BK, int TERMS>
-__device__ __forceinline__ uint64_t make_desc(uint32_t smem_addr) {
-    return (uint64_t)((smem_addr >> 4) & 0x3FFFu) | (1ull << 16) | (Cfg<BK, TERMS>::SBO << 32) | (1ull << 46) |
-           (Cfg<BK, TERMS>::LAYOUT << 61);
-}
-// instruction descriptor (cute::UMMA::InstrDescriptor): f32 accumulate, bf16 x bf16, both K-major, M=128, N=256
-constexpr uint32_t IDESC = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM >> 4) << 24);
 
 // Tile order: column panels PANEL tiles wide, swept down the rows.  The CTAs (or CTA pairs) that run concurrently then
 // cover a roughly square block of the output, so per k-step they pull ~2*sqrt(n) distinct operand tiles through L2
@@ -261,6 +167,7 @@ k_gram(const __grid_constant__ CUtensorMap map_a_hi,   // A side hi, box BM rows
         // ================= MMA issuer (one thread) =================
         if (lane == 0) {
             constexpr int CH = C::CH;                                 // k-blocks per TMEM accumulation chunk
+            constexpr uint32_t IDESC = idesc_bf16(BM, BN);
             int stage = 0, acc = 0;
             uint32_t phase = 0, acc_phase = 0;
             for (int w = blockIdx.x; w < n_work; w += gridDim.x) {
@@ -277,10 +184,10 @@ k_gram(const __grid_constant__ CUtensorMap map_a_hi,   // A side hi, box BM rows
                     mbar_wait(&full[stage], phase);                   // TMA bytes have landed
                     tc_fence_after();
                     const uint32_t a_addr = smem_u32(smem + stage * C::STAGE_BYTES);
-                    const uint64_t ah_desc = make_desc<BK, TERMS>(a_addr);
-                    const uint64_t al_desc = make_desc<BK, TERMS>(a_addr + C::A_BYTES);
-                    const uint64_t bh_desc = make_desc<BK, TERMS>(a_addr + C::PLANES * C::A_BYTES);
-                    const uint64_t bl_desc = make_desc<BK, TERMS>(a_addr + 2 * C::A_BYTES + C::B_BYTES);
+                    const uint64_t ah_desc = desc_sw<C::SBO_BYTES, C::LAYOUT>(a_addr);
+                    const uint64_t al_desc = desc_sw<C::SBO_BYTES, C::LAYOUT>(a_addr + C::A_BYTES);
+                    const uint64_t bh_desc = desc_sw<C::SBO_BYTES, C::LAYOUT>(a_addr + C::PLANES * C::A_BYTES);
+                    const uint64_t bl_desc = desc_sw<C::SBO_BYTES, C::LAYOUT>(a_addr + 2 * C::A_BYTES + C::B_BYTES);
 #pragma unroll
                     for (int k = 0; k < BK / UMMA_K; k++) {
                         const uint64_t adv = (uint64_t)((k * UMMA_K * 2) >> 4);   // +32 B along K inside the swizzled row
@@ -360,36 +267,6 @@ k_gram(const __grid_constant__ CUtensorMap map_a_hi,   // A side hi, box BM rows
 //   arrivals to both CTAs; the peer's accumulate warps release the accumulator on the leader's barrier (mapa).
 // =================================================================================================================
 constexpr int BM2 = 256;
-__device__ __forceinline__ uint32_t cluster_ctarank() { uint32_t r; asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r)); return r; }
-__device__ __forceinline__ void cluster_sync_all() {
-    asm volatile("barrier.cluster.arrive.release.aligned;" ::: "memory");
-    asm volatile("barrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_alloc2(uint32_t *dst_smem, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc2(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma2_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma2_commit_mc(uint64_t *bar) {      // arrives on this barrier in BOTH CTAs of the pair
-    asm volatile("tcgen05.commit.cta_group::2.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-                 ::"r"(smem_u32(bar)), "h"((uint16_t)3) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d_pair(const CUtensorMap *map, uint64_t *leader_bar, void *dst, int c_inner, int c_row) {
-    // the transaction bytes are credited to the LEADER CTA's barrier (peer bit of the shared::cluster address cleared)
-    asm volatile("cp.async.bulk.tensor.2d.cta_group::2.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(leader_bar) & 0xFEFFFFFFu), "r"(c_inner), "r"(c_row) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_on_rank(uint64_t *bar, uint32_t rank) {
-    asm volatile("{\n\t.reg .b32 ra;\n\tmapa.shared::cluster.u32 ra, %0, %1;\n\tmbarrier.arrive.release.cluster.shared::cluster.b64 _, [ra];\n\t}"
-                 ::"r"(smem_u32(bar)), "r"(rank) : "memory");
-}
-constexpr uint32_t IDESC2 = (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(BN >> 3) << 17) | ((uint32_t)(BM2 >> 4) << 24);
 
 template <int BK, int TERMS>
 struct Cfg2 {
@@ -467,6 +344,8 @@ k_gram2(const __grid_constant__ CUtensorMap map_a_hi,   // hi of the A side, box
         // ================= MMA issuer: one thread of the leader CTA =================
         if (lane == 0 && rank == 0) {
             constexpr int CH = C::CH;
+            constexpr uint32_t IDESC = idesc_bf16(BM2, BN);
+            using D = Cfg<BK, TERMS>;                                 // a CTA's operand rows have the single-CTA kernel's layout
             int stage = 0, acc = 0;
             uint32_t phase = 0, acc_phase = 0;
             for (int w = cluster_id; w < n_work; w += n_clusters) {
@@ -483,17 +362,17 @@ k_gram2(const __grid_constant__ CUtensorMap map_a_hi,   // hi of the A side, box
                     mbar_wait(&full[stage], phase);
                     tc_fence_after();
                     const uint32_t a_addr = smem_u32(smem + stage * C::STAGE_BYTES);
-                    const uint64_t ah_desc = make_desc<BK, TERMS>(a_addr);
-                    const uint64_t al_desc = make_desc<BK, TERMS>(a_addr + C::A_BYTES);
-                    const uint64_t bh_desc = make_desc<BK, TERMS>(a_addr + C::PLANES * C::A_BYTES);
-                    const uint64_t bl_desc = make_desc<BK, TERMS>(a_addr + 2 * C::A_BYTES + C::B_BYTES);
+                    const uint64_t ah_desc = desc_sw<D::SBO_BYTES, D::LAYOUT>(a_addr);
+                    const uint64_t al_desc = desc_sw<D::SBO_BYTES, D::LAYOUT>(a_addr + C::A_BYTES);
+                    const uint64_t bh_desc = desc_sw<D::SBO_BYTES, D::LAYOUT>(a_addr + C::PLANES * C::A_BYTES);
+                    const uint64_t bl_desc = desc_sw<D::SBO_BYTES, D::LAYOUT>(a_addr + 2 * C::A_BYTES + C::B_BYTES);
 #pragma unroll
                     for (int k = 0; k < BK / UMMA_K; k++) {
                         const uint64_t adv = (uint64_t)((k * UMMA_K * 2) >> 4);
-                        umma2_bf16(d_tmem, ah_desc + adv, bh_desc + adv, IDESC2, (in_chunk > 0 || k > 0) ? 1u : 0u);
+                        umma2_bf16(d_tmem, ah_desc + adv, bh_desc + adv, IDESC, (in_chunk > 0 || k > 0) ? 1u : 0u);
                         if (TERMS > 1) {
-                            umma2_bf16(d_tmem, ah_desc + adv, bl_desc + adv, IDESC2, 1u);
-                            umma2_bf16(d_tmem, al_desc + adv, bh_desc + adv, IDESC2, 1u);
+                            umma2_bf16(d_tmem, ah_desc + adv, bl_desc + adv, IDESC, 1u);
+                            umma2_bf16(d_tmem, al_desc + adv, bh_desc + adv, IDESC, 1u);
                         }
                     }
                     umma2_commit_mc(&empty[stage]);                   // frees the stage in both CTAs
@@ -594,40 +473,6 @@ __global__ void k_gram_pack(const T *__restrict__ A, long long P, long long K, l
 }
 
 // ---- host side -------------------------------------------------------------------------------------
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-
-static int get_encode(EncodeTiledFn *fn) {
-    static EncodeTiledFn cached = nullptr;
-    if (cached == nullptr) {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        SNK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres));
-        if (qres != cudaDriverEntryPointSuccess || p == nullptr)
-            return fail(SNK_ERR_CUDA, "cuTensorMapEncodeTiled not available from the driver");
-        cached = (EncodeTiledFn)p;
-    }
-    *fn = cached;
-    return SNK_OK;
-}
-
-static int make_map(CUtensorMap *m, const void *base, long long rows, long long cols, long long pitch_elems, int box_rows,
-                    int bk) {
-    EncodeTiledFn enc = nullptr;
-    int rc = get_encode(&enc);
-    if (rc != SNK_OK) return rc;
-    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};          // innermost first
-    cuuint64_t strides[1] = {(cuuint64_t)pitch_elems * 2};
-    cuuint32_t box[2] = {(cuuint32_t)bk, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), dims, strides, box, estr,
-                     CU_TENSOR_MAP_INTERLEAVE_NONE, bk == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B,
-                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(SNK_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-    return SNK_OK;
-}
-
 struct Plan {
     long long rows_a, rows_b, P, Ppad, Mt, Nt;
     int tiles_m, tiles_n, n_tiles, sym, splits, kblocks, kb_per_split, bk, pair;
@@ -686,12 +531,16 @@ static int launch(const Plan &pl, const void *a_hi, const void *a_lo, const void
     using C = Cfg<BK, TERMS>;
     if (TERMS == 1) { a_lo = a_hi; b_lo = b_hi; }               // the lo maps are never dereferenced then
     const int box_b = pl.pair ? BN / 2 : BN;                     // the pair stages half a B tile per CTA
+    auto make_map = [&](CUtensorMap *m, const void *base, long long rows, int box_rows) {      // swizzle matches C::LAYOUT
+        return make_map_2d_16bit(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, base, rows, pl.P, pl.Ppad, box_rows, BK,
+                                 BK == 64 ? CU_TENSOR_MAP_SWIZZLE_128B : CU_TENSOR_MAP_SWIZZLE_64B);
+    };
     CUtensorMap mah, mal, mbh, mbl;
     int rc;
-    if ((rc = make_map(&mah, a_hi, pl.rows_a, pl.P, pl.Ppad, BM, BK)) != SNK_OK) return rc;
-    if ((rc = make_map(&mal, a_lo, pl.rows_a, pl.P, pl.Ppad, BM, BK)) != SNK_OK) return rc;
-    if ((rc = make_map(&mbh, b_hi, pl.rows_b, pl.P, pl.Ppad, box_b, BK)) != SNK_OK) return rc;
-    if ((rc = make_map(&mbl, b_lo, pl.rows_b, pl.P, pl.Ppad, box_b, BK)) != SNK_OK) return rc;
+    if ((rc = make_map(&mah, a_hi, pl.rows_a, BM)) != SNK_OK) return rc;
+    if ((rc = make_map(&mal, a_lo, pl.rows_a, BM)) != SNK_OK) return rc;
+    if ((rc = make_map(&mbh, b_hi, pl.rows_b, box_b)) != SNK_OK) return rc;
+    if ((rc = make_map(&mbl, b_lo, pl.rows_b, box_b)) != SNK_OK) return rc;
     GramArgs g;
     g.partials = scratch;
     g.tiles_m = pl.tiles_m; g.tiles_n = pl.tiles_n; g.n_tiles = pl.n_tiles; g.sym = pl.sym; g.splits = pl.splits;

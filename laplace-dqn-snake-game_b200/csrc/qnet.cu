@@ -30,7 +30,6 @@
 //          halves of a WEIGHT are two MMAs into the same accumulator (lo first, so that the tensor core's truncating
 //          FP32 accumulation hits the small terms while the accumulator is small).  8 real samples per iteration, 4x the
 //          MMAs of the bf16 mode per sample; conv1 and Dense(64,3) are plain FP32 FMAs.  Tolerance: tests/test_qnet_gpu.py.
-#include <cuda.h>
 #include <cuda_bf16.h>
 #include <cuda_fp16.h>
 #include <math.h>
@@ -42,6 +41,7 @@
 
 #include "common.h"
 #include "qnet_theta.h"
+#include "sm100.h"
 
 namespace snk {
 namespace qgrad {       // qnet_grads.cu
@@ -70,99 +70,9 @@ constexpr size_t P_S_W3 = P_S_W2 + 2 * 9 * 1024;             // 72 blocks (k2, k
 constexpr size_t P_S_W4 = P_S_W3 + 72 * 4096;                // [128][1600] fp16: rows [0,64) = hi, [64,128) = lo (one N = 128 operand)
 constexpr size_t P_END = P_S_W4 + 128 * 1600 * 2;
 
-__device__ __forceinline__ uint32_t smem_u32(const void *p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(uint64_t *bar, uint32_t count) {
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count));
-}
-__device__ __forceinline__ void mbar_expect_tx(uint64_t *bar, uint32_t bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(uint64_t *bar) {
-    asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(uint64_t *bar, uint32_t parity) {
-    uint32_t ok;
-    asm volatile("{\n\t.reg .pred P1;\n\tmbarrier.try_wait.parity.shared::cta.b64 P1, [%1], %2;\n\tselp.b32 %0, 1, 0, P1;\n\t}"
-                 : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void mbar_wait(uint64_t *bar, uint32_t parity) {     // bounded: a protocol bug traps, never hangs
-    if (mbar_try_wait(bar, parity)) return;
-    const long long t0 = clock64();
-    while (!mbar_try_wait(bar, parity)) {
-        if (clock64() - t0 > 4000000000ll) {
-            printf("snk qnet: mbarrier wait timed out (block %d thread %d)\n", blockIdx.x, threadIdx.x);
-            __trap();
-        }
-    }
-}
-// the same for a wait that is known to be long (an epilogue warp waiting for a whole MMA phase): back off between polls so
-// that a dozen polling warps do not compete with the tensor core's operand fetch for the shared-memory pipeline
-__device__ __forceinline__ void mbar_wait_relaxed(uint64_t *bar, uint32_t parity) {
-    if (mbar_try_wait(bar, parity)) return;
-    const long long t0 = clock64();
-    while (!mbar_try_wait(bar, parity)) {
-        __nanosleep(128);
-        if (clock64() - t0 > 4000000000ll) {
-            printf("snk qnet: mbarrier wait timed out (block %d thread %d)\n", blockIdx.x, threadIdx.x);
-            __trap();
-        }
-    }
-}
-__device__ __forceinline__ void fence_barrier_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
-__device__ __forceinline__ void fence_proxy_async() { asm volatile("fence.proxy.async.shared::cta;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
-__device__ __forceinline__ void tmem_alloc(uint32_t *dst_smem, uint32_t cols) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(smem_u32(dst_smem)), "r"(cols) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-__device__ __forceinline__ void tmem_dealloc(uint32_t taddr, uint32_t cols) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(taddr), "r"(cols) : "memory");
-}
-__device__ __forceinline__ void umma_bf16(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
-__device__ __forceinline__ void umma_commit(uint64_t *bar) {
-    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ bool elect_one() {
-    uint32_t p;
-    asm volatile("{\n\t.reg .pred P1;\n\telect.sync _|P1, 0xffffffff;\n\tselp.b32 %0, 1, 0, P1;\n\t}" : "=r"(p));
-    return p != 0;
-}
-__device__ __forceinline__ void tmem_ld_wait() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-__device__ __forceinline__ void tmem_ld16(uint32_t taddr, uint32_t (&v)[16]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0,%1,%2,%3,%4,%5,%6,%7,%8,%9,%10,%11,%12,%13,%14,%15}, [%16];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-                   "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-                 : "r"(taddr) : "memory");
-}
-__device__ __forceinline__ void bulk_load(void *dst_smem, const void *src_gmem, uint32_t bytes, uint64_t *bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"(smem_u32(dst_smem)), "l"((uint64_t)src_gmem), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void tma_load_2d(const CUtensorMap *map, uint64_t *bar, void *dst, int c_inner, int c_row) {
-    asm volatile("cp.async.bulk.tensor.2d.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1, {%3, %4}], [%2];"
-                 ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c_inner), "r"(c_row) : "memory");
-}
-
-// no-swizzle K-major operand descriptor: core matrix = 8 rows x 16 B; LBO = byte distance between the two 8-element
-// K chunks of one K=16 MMA, SBO = byte distance between 8-row groups (cute::UMMA::SmemDescriptor, layout_type 0)
-__device__ __forceinline__ uint64_t desc_nosw(uint32_t addr, uint32_t lbo_bytes, uint32_t sbo_bytes) {
-    return (uint64_t)((addr >> 4) & 0x3FFFu) | ((uint64_t)((lbo_bytes >> 4) & 0x3FFFu) << 16) |
-           ((uint64_t)((sbo_bytes >> 4) & 0x3FFFu) << 32) | (1ull << 46);
-}
-__host__ __device__ constexpr uint32_t idesc_bf16(int M, int N) {
-    return (1u << 4) | (1u << 7) | (1u << 10) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
-}
 __device__ __forceinline__ uint32_t pack_relu_bf16(float a, float b) {
     __nv_bfloat162 h = __floats2bfloat162_rn(fmaxf(a, 0.f), fmaxf(b, 0.f));
     return *reinterpret_cast<uint32_t *>(&h);
-}
-__host__ __device__ constexpr uint32_t idesc_f16(int M, int N) {      // a_format = b_format = 0 (F16), FP32 accumulator
-    return (1u << 4) | ((uint32_t)(N >> 3) << 17) | ((uint32_t)(M >> 4) << 24);
 }
 
 struct ConvArgs {
@@ -637,7 +547,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_qnet_convs_split(const __grid_co
                             scratch[(y * 40 + h * 8 + i) * 64 + oc] = fmaf(__uint_as_float(v[i + 8]), LO_UNSCALE, __uint_as_float(v[i]));
                     }
                 }
-                asm volatile("bar.sync 1, 384;" ::: "memory");
+                nbar_sync(1, 384);
                 const float bo = bias[48 + oc];
                 const int live = (int)(a.n - s0 < SR ? a.n - s0 : SR);
                 for (int y = grp; y < 5; y += NGRP) {
@@ -733,10 +643,6 @@ static_assert(SMEM <= 232448, "engine 17 shared memory over the 227 KB limit");
 
 // debug stamps of CTA 0 (snk_qnet_debug_timing): 64 slots per iteration, first 8 iterations; the buffer holds 512 int64
 #define E17_STAMP(slot) do { if (a.timing != nullptr && blockIdx.x == 0 && lane == 0 && it_local >= 0 && it_local < 8) a.timing[it_local * 64 + (slot)] = clock64(); } while (0)
-__device__ __forceinline__ void umma_bf16_ts(uint32_t d_tmem, uint32_t a_tmem, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
-    asm volatile("{\n\t.reg .pred p;\n\tsetp.ne.b32 p, %4, 0;\n\ttcgen05.mma.cta_group::1.kind::f16 [%0], [%1], %2, %3, p;\n\t}"
-                 ::"r"(d_tmem), "r"(a_tmem), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
-}
 #ifndef E17_NOSTORE
 #define E17_NOSTORE 0   /* timing experiment: conv3 epilogue without its global stores */
 #endif
@@ -757,11 +663,6 @@ __device__ __forceinline__ uint32_t cvt_relu_bf16x2(float hi, float lo) {      /
     asm("cvt.rn.relu.bf16x2.f32 %0, %1, %2;" : "=r"(d) : "f"(hi), "f"(lo));
     return d;
 }
-__device__ __forceinline__ void tmem_st8(uint32_t taddr, const uint4 &lo, const uint4 &hi) {
-    asm volatile("tcgen05.st.sync.aligned.32x32b.x8.b32 [%0], {%1,%2,%3,%4,%5,%6,%7,%8};"
-                 ::"r"(taddr), "r"(lo.x), "r"(lo.y), "r"(lo.z), "r"(lo.w), "r"(hi.x), "r"(hi.y), "r"(hi.z), "r"(hi.w) : "memory");
-}
-
 __global__ void __launch_bounds__(NTHREADS, 1) k_qnet_convs17(const __grid_constant__ ConvArgs a) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t *smem = (uint8_t *)(((uintptr_t)smem_raw + 127) & ~(uintptr_t)127);
@@ -800,7 +701,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_qnet_convs17(const __grid_const
             const uint4 lo = *reinterpret_cast<const uint4 *>(src), hi = *reinterpret_cast<const uint4 *>(src + 2048);
             tmem_st8(tmem + ((uint32_t)(q * 32) << 16) + TM_W3 + be * 8, lo, hi);
         }
-        asm volatile("tcgen05.wait::st.sync.aligned;" ::: "memory");
+        tmem_st_wait();
     }
     const long long n_iter = (a.n + S - 1) / S;
     tc_fence_before();
@@ -947,7 +848,7 @@ __global__ void __launch_bounds__(NTHREADS, 1) k_qnet_convs17(const __grid_const
                     mbar_wait(&c3_full[b], (u >> 1) & 1);
                     tc_fence_after();
                     if (warp == 6) E17_STAMP(24 + t);
-                    asm volatile("bar.sync %0, 128;" ::"r"(1 + grp) : "memory");
+                    nbar_sync(1 + grp, 128);
                     const uint32_t my = tmem + ((uint32_t)(q * 32) << 16) + TM_C3 + b * 80;
                     if (q < 2 && t < 5) {
                         const uint32_t park = scr + (uint32_t)((t & 1) * SCR);
@@ -1032,10 +933,6 @@ struct HeadArgs {
     long long n;
 };
 
-__device__ __forceinline__ uint64_t desc_sw128(uint32_t addr) {
-    return (uint64_t)((addr >> 4) & 0x3FFFu) | (1ull << 16) | (64ull << 32) | (1ull << 46) | (2ull << 61);
-}
-
 template <bool SPLIT>
 __global__ void __launch_bounds__(HB_THREADS, 1) k_qnet_head(const __grid_constant__ CUtensorMap map_x,   // out3, box 128 x 64
                                                              const __grid_constant__ CUtensorMap map_w,   // W4', box N x 64
@@ -1093,9 +990,9 @@ __global__ void __launch_bounds__(HB_THREADS, 1) k_qnet_head(const __grid_consta
                     tc_fence_after();
                     const uint32_t base = smem_u32(smem + stage * C::STAGE_BYTES);
 #pragma unroll
-                    for (int k = 0; k < HB_K / 16; k++)
-                        umma_bf16(tmem + acc * C::N, desc_sw128(base) + (uint64_t)(2 * k), desc_sw128(base + HB_M * 128) + (uint64_t)(2 * k),
-                                  IDESC, (kb | k) ? 1u : 0u);
+                    for (int k = 0; k < HB_K / 16; k++)          // 128-byte swizzled rows: 8-row atoms 1024 B apart
+                        umma_bf16(tmem + acc * C::N, desc_sw<1024, LAYOUT_SW128>(base) + (uint64_t)(2 * k),
+                                  desc_sw<1024, LAYOUT_SW128>(base + HB_M * 128) + (uint64_t)(2 * k), IDESC, (kb | k) ? 1u : 0u);
                     umma_commit(&empty[stage]);
                     if (++stage == HB_STAGES) { stage = 0; phase ^= 1; }
                 }
@@ -1332,35 +1229,6 @@ __global__ void __launch_bounds__(APPLY_THREADS) k_qnet_train_apply(const ApplyA
     scatter_param(w, p, a.theta, a.params);
 }
 
-typedef CUresult (*EncodeTiledFn)(CUtensorMap *, CUtensorMapDataType, cuuint32_t, void *, const cuuint64_t *,
-                                  const cuuint64_t *, const cuuint32_t *, const cuuint32_t *, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-static int tensor_map_encoder(EncodeTiledFn *out) {
-    static EncodeTiledFn enc = nullptr;
-    if (enc == nullptr) {
-        void *p = nullptr;
-        cudaDriverEntryPointQueryResult qres;
-        SNK_CUDA(cudaGetDriverEntryPoint("cuTensorMapEncodeTiled", &p, cudaEnableDefault, &qres));
-        if (qres != cudaDriverEntryPointSuccess || p == nullptr) return fail(SNK_ERR_CUDA, "cuTensorMapEncodeTiled unavailable");
-        enc = (EncodeTiledFn)p;
-    }
-    *out = enc;
-    return SNK_OK;
-}
-static int make_map_16bit(CUtensorMap *m, bool fp16, const void *base, long long rows, long long cols, int box_rows, int box_cols) {
-    EncodeTiledFn enc = nullptr;
-    int rc = tensor_map_encoder(&enc);
-    if (rc != SNK_OK) return rc;
-    cuuint64_t dims[2] = {(cuuint64_t)cols, (cuuint64_t)rows};
-    cuuint64_t strides[1] = {(cuuint64_t)cols * 2};
-    cuuint32_t box[2] = {(cuuint32_t)box_cols, (cuuint32_t)box_rows};
-    cuuint32_t estr[2] = {1, 1};
-    CUresult r = enc(m, fp16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<void *>(base), dims,
-                     strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B,
-                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    if (r != CUDA_SUCCESS) return fail(SNK_ERR_CUDA, "cuTensorMapEncodeTiled failed with CUresult %d", (int)r);
-    return SNK_OK;
-}
 }  // namespace qnet
 }  // namespace snk
 
@@ -1595,6 +1463,10 @@ int snk_qnet_forward(snk_qnet q, const float *obs_f32, int64_t N, float *q_out_3
     }
     int grid, rc;
     CUtensorMap mx, mw;
+    auto make_map = [&](CUtensorMap *m, const void *base, long long rows, int box_rows) {     // rows of 1600 fp16 / bf16
+        return make_map_2d_16bit(m, f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, base, rows, 1600, 1600,
+                                 box_rows, HB_K, CU_TENSOR_MAP_SWIZZLE_128B);
+    };
     if (f32) {
         SplitArgs sa;
         sa.obs = obs_f32; sa.n = N; sa.params = q->params; sa.out3 = (__half *)q->out3; sa.overflow = q->d_overflow;
@@ -1606,8 +1478,8 @@ int snk_qnet_forward(snk_qnet q, const float *obs_f32, int64_t N, float *q_out_3
         SNK_CUDA(cudaFuncSetAttribute(split::k_qnet_convs_split, cudaFuncAttributeMaxDynamicSharedMemorySize, split::SMEM));
         split::k_qnet_convs_split<<<grid, THREADS, split::SMEM, st>>>(sa);
         SNK_CUDA(cudaGetLastError());
-        if ((rc = make_map_16bit(&mx, true, q->out3, 2 * q->out3_cap, 1600, HB_M, HB_K)) != SNK_OK) return rc;
-        if ((rc = make_map_16bit(&mw, true, q->params + P_S_W4, 128, 1600, 128, HB_K)) != SNK_OK) return rc;
+        if ((rc = make_map(&mx, q->out3, 2 * q->out3_cap, HB_M)) != SNK_OK) return rc;
+        if ((rc = make_map(&mw, q->params + P_S_W4, 128, 128)) != SNK_OK) return rc;
     } else {
         ConvArgs ca;
         ca.obs = obs_f32; ca.n = N; ca.params = q->params; ca.out3 = (__nv_bfloat16 *)q->out3; ca.timing = q->timing;
@@ -1618,8 +1490,8 @@ int snk_qnet_forward(snk_qnet q, const float *obs_f32, int64_t N, float *q_out_3
         SNK_CUDA(cudaFuncSetAttribute(e17::k_qnet_convs17, cudaFuncAttributeMaxDynamicSharedMemorySize, e17::SMEM));
         e17::k_qnet_convs17<<<grid, e17::NTHREADS, e17::SMEM, st>>>(ca);
         SNK_CUDA(cudaGetLastError());
-        if ((rc = make_map_16bit(&mx, false, q->out3, q->out3_cap, 1600, HB_M, HB_K)) != SNK_OK) return rc;
-        if ((rc = make_map_16bit(&mw, false, q->params + P_W4, 64, 1600, 64, HB_K)) != SNK_OK) return rc;
+        if ((rc = make_map(&mx, q->out3, q->out3_cap, HB_M)) != SNK_OK) return rc;
+        if ((rc = make_map(&mw, q->params + P_W4, 64, 64)) != SNK_OK) return rc;
     }
     HeadArgs ha;
     ha.params = q->params; ha.q_out = q_out_3xN; ha.n = N;

@@ -32,6 +32,7 @@
 #include <cuda.h>
 
 #include "common.h"
+#include "sm100.h"
 
 // how phase B stores the observation: 0 = st.global.cs (streaming), 1 = plain st.global (default), 2 = st.global.wt.
 // Measured at 2^20 envs on B200: 166.5 us with .cs, 162.8 us with plain or .wt stores (87.4 % of the HBM copy peak); into
@@ -755,8 +756,6 @@ struct __align__(16) Handoff {
     float reward, ret;
     int score, pad;
 };
-__device__ __forceinline__ void nbar_sync(int id, int n) { asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(n) : "memory"); }
-__device__ __forceinline__ void nbar_arrive(int id, int n) { asm volatile("bar.arrive %0, %1;" ::"r"(id), "r"(n) : "memory"); }
 #ifndef SNK_WS_XW
 #define SNK_WS_XW 5              // expansion warps per CTA; measured at 4,096 envs, Float32 observations: 2 -> 1.13 us per step, 3 -> 1.02, 4 -> 0.90, 5 -> 0.87, 6 -> 0.97, 8 -> 0.98
 #endif
