@@ -37,7 +37,6 @@
 #include <string.h>
 
 #include <new>
-#include <vector>
 
 #include "common.h"
 #include "qnet_theta.h"
@@ -45,8 +44,6 @@
 
 namespace snk {
 namespace qgrad {       // qnet_grads.cu
-long long theta_ext_floats();
-void build_theta_ext(const float *theta_host, float *ext);     // theta + the two re-ordered copies of W3 the gradient kernel reads
 int launch_sample_grads(const float *theta_dev, const float *states, const uint8_t *actions, const double *targets, long long B,
                         void *hi, void *lo, long long pitch, float *J, long long ldJ, float *loss, int sms, cudaStream_t st);
 }
@@ -1048,8 +1045,8 @@ __global__ void __launch_bounds__(HB_THREADS, 1) k_qnet_head(const __grid_consta
     }
 }
 
-// ---- parameter packing (host: pack_params at create; device: k_qnet_train_apply after every update) ----------------
-__host__ __device__ static inline uint16_t f2bf(float f) {            // round-to-nearest-even
+// ---- parameter packing: k_qnet_train_apply at create, after every update and in set_params --------------------------
+__device__ static inline uint16_t f2bf(float f) {            // round-to-nearest-even
     uint32_t u;
     memcpy(&u, &f, 4);
     if ((u & 0x7F800000u) == 0x7F800000u) return (uint16_t)(u >> 16);
@@ -1057,78 +1054,15 @@ __host__ __device__ static inline uint16_t f2bf(float f) {            // round-t
     return (uint16_t)(u >> 16);
 }
 // w = hi + lo in fp16 (lo unscaled): part 0 = lo, part 1 = hi
-__host__ __device__ static inline uint16_t f2h_part(float w, int part) {
+__device__ static inline uint16_t f2h_part(float w, int part) {
     const __half h = __float2half_rn(w);
     if (part) return __half_as_ushort(h);
     return __half_as_ushort(__float2half_rn(w - __half2float(h)));
 }
 
-// theta = Flux.destructure(q_net): W1(3,3,2,16) b1 W2(3,3,16,32) b2 W3(6,6,32,64) b3 W4(64,1600) b4 W5(3,64) b5, column-major
-static void pack_params(const float *th, std::vector<uint8_t> &blob) {
-    blob.assign(P_END, 0);
-    const float *W1 = th, *b1 = W1 + 288, *W2 = b1 + 16, *b2 = W2 + 4608, *W3 = b2 + 32, *b3 = W3 + 73728;
-    const float *W4 = b3 + 64, *b4 = W4 + 102400, *W5 = b4 + 64, *b5 = W5 + 192;
-    auto bf = [&](size_t off) { return reinterpret_cast<uint16_t *>(blob.data() + off); };
-    // flipped kernels: Wf[k1,k2,c,o] = W[K-1-k1, K-1-k2, c, o]; Flux layout index = a1 + K*(a2 + K*(c + C*o))
-    auto w1 = [&](int k1, int k2, int c, int o) { return W1[(2 - k1) + 3 * ((2 - k2) + 3 * (c + 2 * o))]; };
-    auto w2 = [&](int k1, int k2, int c, int o) { return W2[(2 - k1) + 3 * ((2 - k2) + 3 * (c + 16 * o))]; };
-    auto w3 = [&](int k1, int k2, int c, int o) { return W3[(5 - k1) + 6 * ((5 - k2) + 6 * (c + 32 * o))]; };
-    // W1 (fp32, CUDA-core conv1): [tap = k2*3 + k1][c][o]
-    float *w1f = reinterpret_cast<float *>(blob.data() + P_W1);
-    for (int k2 = 0; k2 < 3; k2++)
-        for (int k1 = 0; k1 < 3; k1++)
-            for (int c = 0; c < 2; c++)
-                for (int o = 0; o < 16; o++) w1f[((k2 * 3 + k1) * 2 + c) * 16 + o] = w1(k1, k2, c, o);
-    // W2: [k2][k1][chunk (2)][o (32)][8]; the fp16 pair: [part][...]
-    for (int k2 = 0; k2 < 3; k2++)
-        for (int k1 = 0; k1 < 3; k1++)
-            for (int c = 0; c < 16; c++)
-                for (int o = 0; o < 32; o++) {
-                    const size_t i = (((k2 * 3 + k1) * 2 + c / 8) * 32 + o) * 8 + c % 8;
-                    bf(P_W2)[i] = f2bf(w2(k1, k2, c, o));
-                    // split mode: [k2][k1][chunk (2)][n = 32 half + o (64)][8], half 0 = hi, 1 = lo
-                    for (int half = 0; half < 2; half++)
-                        bf(P_S_W2)[(((k2 * 3 + k1) * 2 + c / 8) * 64 + half * 32 + o) * 8 + c % 8] = f2h_part(w2(k1, k2, c, o), 1 - half);
-                }
-    // W3: 36 blocks (j, k1, m) of 128 stacked rows x 16 channels, canonical K-major core matrices:
-    // row R = 64 h + o carries kernel row k2 = 2 j + h; [K chunk (2)][row group (16)][row (8)][8 channels]
-    for (int j = 0; j < 3; j++)
-        for (int k1 = 0; k1 < 6; k1++)
-            for (int m = 0; m < 2; m++)
-                for (int R = 0; R < 128; R++)
-                    for (int kk = 0; kk < 16; kk++) {
-                        const size_t i = (size_t)((j * 6 + k1) * 2 + m) * 2048 + (((kk / 8) * 16 + R / 8) * 8 + R % 8) * 8 + kk % 8;
-                        const float w = w3(k1, 2 * j + R / 64, 16 * m + kk, R % 64);
-                        bf(P_W3B)[i] = f2bf(w);
-                    }
-    // split mode: 72 blocks (k2, k1, m) of 128 rows x 16 channels: row R = 64 half + o, half 0 = hi, 1 = lo; same core-matrix order
-    for (int k2 = 0; k2 < 6; k2++)
-        for (int k1 = 0; k1 < 6; k1++)
-            for (int m = 0; m < 2; m++)
-                for (int R = 0; R < 128; R++)
-                    for (int kk = 0; kk < 16; kk++)
-                        bf(P_S_W3)[(size_t)((k2 * 6 + k1) * 2 + m) * 2048 + (((kk / 8) * 16 + R / 8) * 8 + R % 8) * 8 + kk % 8] =
-                            f2h_part(w3(k1, k2, 16 * m + kk, R % 64), 1 - R / 64);
-    float *bias = reinterpret_cast<float *>(blob.data() + P_BIAS);
-    memcpy(bias, b1, 64); memcpy(bias + 16, b2, 128); memcpy(bias + 48, b3, 256);
-    // W4 (64,1600) column-major, Flux flatten index kF = x + 5 y + 25 c  ->  [n][k' = (y*5 + x)*64 + c]
-    for (int n = 0; n < 64; n++)
-        for (int c = 0; c < 64; c++)
-            for (int y = 0; y < 5; y++)
-                for (int x = 0; x < 5; x++) {
-                    const float w = W4[n + 64 * (x + 5 * y + 25 * c)];
-                    const size_t k = (size_t)(y * 5 + x) * 64 + c;
-                    bf(P_W4)[(size_t)n * 1600 + k] = f2bf(w);
-                    for (int half = 0; half < 2; half++) bf(P_S_W4)[(size_t)(half * 64 + n) * 1600 + k] = f2h_part(w, 1 - half);
-                }
-    memcpy(blob.data() + P_B4, b4, 256);
-    memcpy(blob.data() + P_W5, W5, 768);          // (3,64) column-major: W5[a + 3 c]
-    memcpy(blob.data() + P_B5, b5, 12);
-}
-
-// pack_params + build_theta_ext for ONE parameter, as a scatter from its Flux index p: writes every byte the host packers derive
-// from theta[p], with the same rounding, so a blob updated on the device equals the blob snk_qnet_create would build from the
-// new theta byte for byte.  `theta` is the handle's extended copy (the two re-ordered W3 copies behind it).
+// The one definition of every device layout of the weights, as a scatter from a parameter's Flux index p (theta =
+// Flux.destructure(q_net): W1(3,3,2,16) b1 W2(3,3,16,32) b2 W3(6,6,32,64) b3 W4(64,1600) b4 W5(3,64) b5, column-major): writes
+// every byte derived from theta[p].  `theta` is the handle's extended copy (the two re-ordered W3 copies behind it).
 __device__ __forceinline__ void scatter_param(float w, int p, float *theta, uint8_t *params) {
     using namespace qgrad;
     auto h = [&](size_t off) { return reinterpret_cast<uint16_t *>(params + off); };
@@ -1252,8 +1186,9 @@ struct snk_qnet_s {
     float *row_loss;
     double *gsum;                // NP + 1 running sums carried between chunks
     long long rows_cap;          // in samples
-    // conv1's weights are kernel parameters read from w1h / b1h / w1f / b1f (DESIGN §5b): a device-side update copies them into
-    // conv1_host and records conv1_ready; the next forward waits for that event and rebuilds the host fields before its launch
+    // conv1's weights are kernel parameters read from w1h / b1h / w1f / b1f (DESIGN §5b): every write of the weights on the device
+    // copies them into conv1_host and records conv1_ready; create, and after an update the next forward, waits for that event and
+    // rebuilds the host fields (fetch_conv1)
     float *conv1_host;           // pinned: P_W1 (288) then b1 (16)
     cudaEvent_t conv1_ready;
     int conv1_pending;
@@ -1272,6 +1207,13 @@ static int enqueue_conv1_refresh(snk_qnet_s *q, cudaStream_t st) {
     SNK_CUDA(cudaMemcpyAsync(q->conv1_host + 288, q->params + P_BIAS, 16 * 4, cudaMemcpyDeviceToHost, st));
     SNK_CUDA(cudaEventRecord(q->conv1_ready, st));
     q->conv1_pending = 1;
+    return SNK_OK;
+}
+
+static int fetch_conv1(snk_qnet_s *q) {
+    SNK_CUDA(cudaEventSynchronize(q->conv1_ready));
+    set_conv1(q, q->conv1_host, q->conv1_host + 288);
+    q->conv1_pending = 0;
     return SNK_OK;
 }
 
@@ -1298,31 +1240,34 @@ int snk_qnet_create(snk_qnet *out, const float *theta_host, int64_t n_params, in
                             (long long)i, (double)theta_host[i]);
     DeviceGuard guard(device);
     SNK_CUDA(cudaGetLastError());
-    std::vector<uint8_t> blob;
-    pack_params(theta_host, blob);
-    snk_qnet_s *q = new (std::nothrow) snk_qnet_s();      // value-initialised: every member zero
+    snk_qnet_s *q = new (std::nothrow) snk_qnet_s();      // value-initialised: every member zero, so destroy frees what exists
     if (q == nullptr) return fail(SNK_ERR_INVALID, "out of host memory");
     q->device = device;
     q->precision = precision;
-    set_conv1(q, reinterpret_cast<const float *>(blob.data() + P_W1), reinterpret_cast<const float *>(blob.data() + P_BIAS));
     cudaDeviceGetAttribute(&q->sms, cudaDevAttrMultiProcessorCount, device);
-    cudaError_t e = cudaMalloc((void **)&q->params, blob.size());
-    if (e == cudaSuccess) e = cudaMemcpy(q->params, blob.data(), blob.size(), cudaMemcpyHostToDevice);
-    std::vector<float> ext((size_t)qgrad::theta_ext_floats());
-    qgrad::build_theta_ext(theta_host, ext.data());
-    if (e == cudaSuccess) e = cudaMalloc((void **)&q->theta, ext.size() * 4);
-    if (e == cudaSuccess) e = cudaMemcpy(q->theta, ext.data(), ext.size() * 4, cudaMemcpyHostToDevice);
-    if (e == cudaSuccess) e = cudaMalloc((void **)&q->d_overflow, sizeof(int));
-    if (e == cudaSuccess) e = cudaMemset(q->d_overflow, 0, sizeof(int));
-    if (e == cudaSuccess) e = cudaMallocHost((void **)&q->conv1_host, 304 * 4);
-    if (e == cudaSuccess) e = cudaEventCreateWithFlags(&q->conv1_ready, cudaEventDisableTiming);
-    if (e != cudaSuccess) {
-        if (q->params) cudaFree(q->params);
-        if (q->theta) cudaFree(q->theta);
-        if (q->d_overflow) cudaFree(q->d_overflow);
-        if (q->conv1_host) cudaFreeHost(q->conv1_host);
-        delete q;
-        return fail(SNK_ERR_CUDA, "snk_qnet_create: %s", cudaGetErrorString(e));
+    auto build = [&]() -> int {
+        SNK_CUDA(cudaMalloc((void **)&q->params, P_END));
+        SNK_CUDA(cudaMemset(q->params, 0, P_END));                       // the padding no layout writes
+        SNK_CUDA(cudaMalloc((void **)&q->theta, qgrad::THETA_EXT * 4));
+        SNK_CUDA(cudaMemset(q->theta, 0, qgrad::THETA_EXT * 4));         // the gap [NP, O_W3OF)
+        SNK_CUDA(cudaMalloc((void **)&q->d_overflow, sizeof(int)));
+        SNK_CUDA(cudaMemset(q->d_overflow, 0, sizeof(int)));
+        SNK_CUDA(cudaMallocHost((void **)&q->conv1_host, 304 * 4));
+        SNK_CUDA(cudaEventCreateWithFlags(&q->conv1_ready, cudaEventDisableTiming));
+        SNK_CUDA(cudaMemcpy(q->theta, theta_host, qgrad::NP * 4, cudaMemcpyHostToDevice));
+        // in place on the legacy stream behind the copies: thread p reads theta_src[p] before it writes theta[p], and its
+        // other writes lie at >= O_W3OF, which no thread reads
+        ApplyArgs a = {};
+        a.theta_src = q->theta;
+        int rc;
+        if ((rc = launch_apply(q, a, 0)) != SNK_OK) return rc;
+        if ((rc = enqueue_conv1_refresh(q, 0)) != SNK_OK) return rc;
+        return fetch_conv1(q);
+    };
+    const int rc = build();
+    if (rc != SNK_OK) {
+        snk_qnet_destroy(q);
+        return rc;
     }
     *out = q;
     return SNK_OK;
@@ -1449,9 +1394,8 @@ int snk_qnet_forward(snk_qnet q, const float *obs_f32, int64_t N, float *q_out_3
             return fail(SNK_ERR_INVALID, "snk_qnet_forward: the weights of this handle changed on the device (snk_qnet_train_step / "
                                          "snk_qnet_set_params) and conv1's kernel parameters must be fetched by the host first: "
                                          "run one forward outside the stream capture");
-        SNK_CUDA(cudaEventSynchronize(q->conv1_ready));
-        set_conv1(q, q->conv1_host, q->conv1_host + 288);
-        q->conv1_pending = 0;
+        const int rc = fetch_conv1(q);
+        if (rc != SNK_OK) return rc;
     }
     const size_t row_bytes = f32 ? 2 * 1600 * 2 : 1600 * 2;             // per sample
     if (q->out3_cap < N) {

@@ -598,20 +598,6 @@ __global__ void __launch_bounds__(NT, 2) k_sample_grads(const GradArgs a) {
     }
 }
 
-// theta as the kernel wants it on the device: Flux.destructure order, then W3 twice more (see O_W3OF / O_W3CF)
-long long theta_ext_floats() { return THETA_EXT; }
-void build_theta_ext(const float *theta_host, float *ext) {
-    for (int i = 0; i < NP; i++) ext[i] = theta_host[i];
-    for (int i = NP; i < O_W3OF; i++) ext[i] = 0.f;
-    for (int o = 0; o < 64; o++)
-        for (int c = 0; c < 32; c++)
-            for (int t = 0; t < 36; t++) {                        // t = a1 + 6 a2
-                const float w = theta_host[O_W3 + t + 36 * (c + 32 * o)];
-                ext[O_W3OF + (c * 36 + t) * 64 + o] = w;
-                ext[O_W3CF + (o * 36 + t) * 32 + c] = w;
-            }
-}
-
 int launch_sample_grads(const float *theta_dev, const float *states, const uint8_t *actions, const double *targets, long long B,
                         void *hi, void *lo, long long pitch, float *J, long long ldJ, float *loss, int sms, cudaStream_t st) {
     GradArgs a;
