@@ -4,7 +4,8 @@ every 1,000 updates, epsilon decay — train.Trainer over the library.  Prints t
 episode returns every --report updates.  Needs a B200.
 
 One play advances every one of --envs games by one step (the reference plays one whole episode of one game per update);
---updates-per-step sets how many updates follow each play.
+--updates-per-step sets how many updates follow each play.  --save PATH writes a checkpoint at the end (save_trainer,
+utils.jl:408-412); --resume PATH continues a saved run bit for bit (load_trainer, utils.jl:413-418) up to --batches updates in all.
 """
 import argparse
 import os
@@ -24,9 +25,15 @@ def main():
     ap.add_argument("--precision", default="f32", choices=["f32", "bf16"])
     ap.add_argument("--report", type=int, default=1000)
     ap.add_argument("--window", type=int, default=1000, help="episodes in the moving average of the returns")
+    ap.add_argument("--save", metavar="PATH", help="write a checkpoint of the run here at the end")
+    ap.add_argument("--resume", metavar="PATH", help="continue the run saved here (its --envs and --precision are the checkpoint's)")
     args = ap.parse_args()
     S = graft.load_package()
-    tr = S.train.Trainer(n_envs=args.envs, precision=args.precision, updates_per_step=args.updates_per_step)
+    if args.resume:
+        tr = S.train.Trainer.load(args.resume)
+        print("resumed %s: %d updates, %d transitions stored" % (args.resume, tr.n_updates, tr.stored))
+    else:
+        tr = S.train.Trainer(n_envs=args.envs, precision=args.precision, updates_per_step=args.updates_per_step)
     tr.fill_buffer()
     print("filled: %d transitions stored, replay %d/%d" % (tr.stored, len(tr.replay), tr.replay.capacity))
     while tr.n_updates < args.batches:
@@ -38,6 +45,9 @@ def main():
             print("batch %7d  loss %.5f  episodes %8d  avg return (last %d) %.3f  epsilon %.4f"
                   % (tr.n_updates, loss, rets.numel(), args.window, avg, tr.epsilon))
     print("env errors %d" % tr.env.count_errors())
+    if args.save:
+        tr.save(args.save)
+        print("saved %s" % args.save)
 
 
 if __name__ == "__main__":

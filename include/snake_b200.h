@@ -218,6 +218,20 @@ SNK_API int snk_get_steps_host(snk_handle h, int32_t *steps_host);
 /* number of envs with any error bit set (synchronises) */
 SNK_API int snk_count_errors_host(snk_handle h, int64_t *count);
 
+/* ---- checkpoints of a handle: save_trainer / load_trainer (utils.jl:408-418) -------------------------------------------
+ * A blob (host memory, opaque, little endian) holds everything a later call on the handle depends on: a header (magic, format
+ * version, N, the snk_create flags, seed, the call counter of the internal generator, the food list) and the raw state arrays
+ * of the N envs — a handle loaded from it continues bit for bit like the one it was saved from.  snk_env_checkpoint_bytes gives
+ * the size (176 + 52 N bytes); snk_env_save_host waits for the work enqueued on the handle's stream, copies and returns.
+ * snk_env_load_host checks the header, then the blob's every env on the device (DESIGN §5e: coordinates, length, step count,
+ * the direction chain against occupancy and tail, consumed food entries within the blob's list); only a blob that passes
+ * replaces the handle's state, seed, counter and food list.  A refused blob (SNK_ERR_INVALID: wrong magic or version, a size
+ * that is not the blob's, another N or auto-reset flag, an env that fails a rule — *first_bad_env (may be NULL) = the lowest
+ * such env, else -1) leaves the handle as it was.  A blob saved on one device loads on another.  Both synchronise. */
+SNK_API int snk_env_checkpoint_bytes(snk_handle h, size_t *bytes);
+SNK_API int snk_env_save_host(snk_handle h, void *blob_host, size_t bytes);
+SNK_API int snk_env_load_host(snk_handle h, const void *blob_host, size_t bytes, int64_t *first_bad_env);
+
 /* ---- replay buffer  ReplayBuffer (structs.jl:104-116), store! / sample / stack_exp (utils.jl:265-383) -------
  * The ring lives on the device as one 128-byte record per transition (three 2-bit-plane boards + scalars);
  * snk_step_fused_store is snk_step_fused that additionally store!s every env's Experience in env order — the
@@ -248,6 +262,14 @@ SNK_API int snk_replay_gather_host(snk_replay r, const int64_t *idx_host, int64_
                                    uint8_t *actions, float *rewards, uint8_t *dones, uint8_t *mask, void *cuda_stream);
 SNK_API int snk_replay_sample_indices(snk_replay r, uint64_t seed, int64_t B, int64_t *idx_out, void *cuda_stream);
 SNK_API int snk_replay_bad_index_host(snk_replay r, int *flag);
+/* checkpoints of the ring: save_buffer / load_buffer (utils.jl:316-340).  The blob: a header (magic, format version, capacity,
+ * transitions stored, sample calls so far) and the min(stored, capacity) filled records (40 + 128 per record bytes).  Save and
+ * load synchronise the ring's device first (the ring has no stream of its own).  Load checks every record's scalars on the
+ * device (action index <= 2, done <= 1, mask bits <= 7, previous direction <= 3) and refuses as snk_env_load_host does:
+ * *first_bad_slot = the lowest failing record (else -1), the ring left as it was. */
+SNK_API int snk_replay_checkpoint_bytes(snk_replay r, size_t *bytes);
+SNK_API int snk_replay_save_host(snk_replay r, void *blob_host, size_t bytes);
+SNK_API int snk_replay_load_host(snk_replay r, const void *blob_host, size_t bytes, int64_t *first_bad_slot);
 
 /* ---- Q-network forward  structs.jl:127-139; call sites utils.jl:165 (acting), 448 (t_net targets) -------------
  * Conv(3x3,2=>16,relu,pad 1) -> Conv(3x3,16=>32,relu,pad 1) -> Conv(6x6,32=>64,relu) -> flatten -> Dense(1600,64,relu)

@@ -135,6 +135,10 @@ def lib():
         "snk_masked_target": [vp, vp, vp, vp, f64, f32, vp, vp, i64, vp],
         "snk_get_score": [vp, vp], "snk_get_done": [vp, vp], "snk_get_error_flags": [vp, vp],
         "snk_get_steps": [vp, vp], "snk_count_errors_host": [vp, C.POINTER(i64)],
+        "snk_env_checkpoint_bytes": [vp, C.POINTER(C.c_size_t)], "snk_env_save_host": [vp, vp, C.c_size_t],
+        "snk_env_load_host": [vp, vp, C.c_size_t, C.POINTER(i64)],
+        "snk_replay_checkpoint_bytes": [vp, C.POINTER(C.c_size_t)], "snk_replay_save_host": [vp, vp, C.c_size_t],
+        "snk_replay_load_host": [vp, vp, C.c_size_t, C.POINTER(i64)],
         "snk_center_columns": [vp, i64, i64, vp, vp, vp],
         "snk_d_store_snapshot": [vp, i64, i64, i64, vp, vp],
         "snk_laplace_sample_weights": [vp, vp, vp, i64, i64, vp, vp, vp, vp],
@@ -188,6 +192,30 @@ def lib():
 def _check(rc):
     if rc != 0:
         raise SnakeB200Error("libsnake_b200 error %d: %s" % (rc, lib().snk_last_error().decode()))
+
+
+def _save_blob(size_fn, save_fn, handle):
+    """a checkpoint blob of the library (snk_*_save_host) as a uint8 CPU tensor"""
+    n = C.c_size_t(0)
+    _check(size_fn(handle, C.byref(n)))
+    blob = torch.empty(n.value, dtype=torch.uint8)
+    _check(save_fn(handle, C.c_void_p(blob.data_ptr()), n.value))
+    return blob
+
+
+def _load_blob(load_fn, handle, d):
+    """snk_*_load_host of d['blob']; a refusal raises SnakeB200Error with the library's message and `first_bad`, the index of
+    the lowest record that failed validation (-1 when the blob was refused for another reason)"""
+    blob = d.get("blob") if isinstance(d, dict) else None
+    if not isinstance(blob, torch.Tensor) or blob.dtype != torch.uint8 or blob.dim() != 1:
+        raise ValueError("a state_dict with 'blob': a 1-d uint8 tensor (from state_dict()) is required")
+    blob = blob.cpu().contiguous()
+    bad = C.c_int64(-1)
+    rc = load_fn(handle, C.c_void_p(blob.data_ptr()), blob.numel(), C.byref(bad))
+    if rc != 0:
+        err = SnakeB200Error("libsnake_b200 error %d: %s" % (rc, lib().snk_last_error().decode()))
+        err.first_bad = bad.value
+        raise err
 
 
 def _ptr(t, dtype=None, numel=None, device=None):
@@ -488,6 +516,17 @@ class SnakeGame:
         _check(lib().snk_count_errors_host(self._h, C.byref(c)))
         return c.value
 
+    # -- checkpoints (save_trainer / load_trainer, utils.jl:408-418) ---------------------------------------------------
+    def state_dict(self):
+        """{'blob': uint8 CPU tensor}: the N games, the generator's seed and call count and the food list (snk_env_save_host),
+        after the work enqueued so far"""
+        return {"blob": _save_blob(lib().snk_env_checkpoint_bytes, lib().snk_env_save_host, self._h)}
+
+    def load_state_dict(self, d):
+        """The games continue bit for bit from where state_dict() left them.  Needs the same N and auto_reset; a blob the
+        library refuses raises SnakeB200Error and leaves the games as they were."""
+        _load_blob(lib().snk_env_load_host, self._h, d)
+
 
 def masked_target(q_next, mask, rewards, dones, gamma=0.97, fill=-100.0, out_dtype=torch.float64):
     """utils.jl:448-451: q_next[mask] .= -100; y = r + 0.97 * max_a q_next * (1 - done).
@@ -672,6 +711,22 @@ class ReplayBuffer:
         f = C.c_int(0)
         _check(lib().snk_replay_bad_index_host(self._r, C.byref(f)))
         return bool(f.value)
+
+    # -- checkpoints (save_buffer / load_buffer, utils.jl:316-340) -----------------------------------------------------
+    def state_dict(self):
+        """{'blob': uint8 CPU tensor (the filled records, the stored count, the sampler's call count), 'seed', 'batch_size'}"""
+        return {"blob": _save_blob(lib().snk_replay_checkpoint_bytes, lib().snk_replay_save_host, self._r),
+                "seed": self.seed, "batch_size": self.batch_size}
+
+    def load_state_dict(self, d):
+        """The ring continues bit for bit (the same samples, the same slots filled next).  Needs the same capacity; a blob the
+        library refuses raises SnakeB200Error and leaves the ring as it was."""
+        if not isinstance(d, dict) or not isinstance(d.get("seed"), int) or not isinstance(d.get("batch_size"), int):
+            raise ValueError("a ReplayBuffer state_dict holds 'blob', 'seed' and 'batch_size'")
+        if not 0 < d["batch_size"] <= self.capacity:
+            raise ValueError("batch_size cannot be greater than the capacity of the buffer.")
+        _load_blob(lib().snk_replay_load_host, self._r, d)
+        self.seed, self.batch_size = d["seed"], d["batch_size"]
 
 
 from . import shard  # noqa: E402,F401

@@ -1153,6 +1153,84 @@ __global__ void k_replay_sample(long long n, long long B, u64 key, long long *ou
     out[i] = (long long)x;
 }
 
+// ---- checkpoint validation (snk_env_load_host, snk_replay_load_host; DESIGN §5e) ----------------------------------------
+// A checkpoint comes from a file: input from outside the program.  The kernels decode coordinates, lengths and chain entries
+// from the state and trust them, so a load accepts only states the step kernel can have stored.  Rule codes index
+// kEnvRuleText / kReplayRuleText.
+enum EnvRule { ER_OK, ER_BITS, ER_HEAD, ER_TAIL, ER_FOOD, ER_PFOOD, ER_LEN, ER_STEPS, ER_CONS, ER_PD, ER_CHAIN, ER_CHAIN_TAIL, ER_OCC };
+enum ReplayRule { RR_OK, RR_ACTION, RR_DONE, RR_MASK, RR_PD };
+
+__device__ __forceinline__ bool interior(int r, int c) { return r >= 1 && r <= 8 && c >= 1 && c <= 8; }
+__device__ __forceinline__ u64 interior_bit(int r, int c) { return 1ull << ((r - 1) + 8 * (c - 1)); }
+
+// the first rule env i's state breaks, ER_OK if none
+__device__ __forceinline__ int env_rule(u64 occ, u64 clo, u64 chi, u64 cons, u64 misc, u64 list_mask) {
+    Env e;
+    env_unpack(e, misc);
+    if (misc >> (M_ERR + 2)) return ER_BITS;                       // error bits beyond FOOD | ACTION, bits 56..63
+    // a wall death draws the head on the wall ring (next to an interior cell: never a corner)
+    const bool on_wall = ((e.hr == 0 || e.hr == 9) && e.hc >= 1 && e.hc <= 8) || ((e.hc == 0 || e.hc == 9) && e.hr >= 1 && e.hr <= 8);
+    const bool head_in = interior(e.hr, e.hc);
+    if (!head_in && !(e.dn && on_wall)) return ER_HEAD;
+    if (!interior(e.tr, e.tc)) return ER_TAIL;
+    if (!interior(e.fr, e.fc) && (e.fr | e.fc) != 0) return ER_FOOD;   // (0, 0) = no food on the board
+    if (!interior(e.pfr, e.pfc) && (e.pfr | e.pfc) != 0) return ER_PFOOD;
+    if (e.len < 2 || e.len > 64) return ER_LEN;
+    if (e.t > (e.dn ? 500 : 499)) return ER_STEPS;                 // the 500th step loses (utils.jl:88)
+    if (cons & ~list_mask) return ER_CONS;
+    if (chain_get(clo, chi, 0) != e.pd) return ER_PD;              // prev_dir is the last move
+    // the body from the head: segment j+1 = segment j - delta(entry j); distinct interior cells, the last one the tail
+    int r = e.hr, c = e.hc;
+    u64 body = 0;
+    for (int j = 0; j < e.len - 1; j++) {
+        int dr, dc;
+        dir_delta(chain_get(clo, chi, j), dr, dc);
+        r -= dr;
+        c -= dc;
+        if (!interior(r, c) || (body & interior_bit(r, c))) return ER_CHAIN;
+        body |= interior_bit(r, c);
+    }
+    if (r != e.tr || c != e.tc) return ER_CHAIN_TAIL;
+    // occ = body + head cell; only a lost head may share a cell with the body (it ran into it)
+    if (head_in) {
+        if (!e.dn && (body & interior_bit(e.hr, e.hc))) return ER_CHAIN;
+        body |= interior_bit(e.hr, e.hc);
+    }
+    return occ == body ? ER_OK : ER_OCC;
+}
+
+// the lowest failing index of the launch and its rule, packed as index << 8 | rule: a block-wide OR skips clean CTAs, the
+// others reduce in shared memory and issue one global atomicMin
+__device__ __forceinline__ void report_first_bad(int rule, long long i, unsigned long long *first) {
+    __shared__ unsigned long long s_min;
+    if (!__syncthreads_or(rule != 0)) return;
+    if (threadIdx.x == 0) s_min = ~0ull;
+    __syncthreads();
+    if (rule != 0) atomicMin(&s_min, ((unsigned long long)i << 8) | (unsigned)rule);
+    __syncthreads();
+    if (threadIdx.x == 0) atomicMin(first, s_min);
+}
+
+__global__ void __launch_bounds__(256) k_env_validate(EnvState s, long long n, u64 list_mask, unsigned long long *first) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    const int rule = i < n ? env_rule(s.occ[i], s.clo[i], s.chi[i], s.cons[i], s.misc[i], list_mask) : ER_OK;
+    report_first_bad(rule, i, first);
+}
+
+// the scalar bytes of a 128-byte record (see REC_U4): word 1 of rec[6] = action | done << 8 | mask bits << 16 | prev_dir << 24
+__global__ void __launch_bounds__(256) k_replay_validate(const uint4 *ring, long long n, unsigned long long *first) {
+    const long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    int rule = RR_OK;
+    if (i < n) {
+        const uint32_t w = ring[i * REC_U4 + 6].y;
+        if ((w & 0xFF) > 2) rule = RR_ACTION;                      // k_sample_grads indexes the three Q-values with it
+        else if (((w >> 8) & 0xFF) > 1) rule = RR_DONE;
+        else if (((w >> 16) & 0xFF) > 7) rule = RR_MASK;
+        else if ((w >> 24) > 3) rule = RR_PD;
+    }
+    report_first_bad(rule, i, first);
+}
+
 }  // namespace snk
 
 // ================================================================================================
@@ -1374,6 +1452,67 @@ static int vmm_alloc_compressible(const Vmm &v, int device, size_t bytes, void *
     }
     *p = (void *)d;
     *a = {h, size, device, true};
+    return SNK_OK;
+}
+
+// ---- checkpoints (snk_env_* / snk_replay_* _checkpoint_bytes, _save_host, _load_host; DESIGN §5e) -----------------------
+// Blob = header + raw device arrays.  The env arrays go in the order of EnvState, copied as they are in memory (also the lazily
+// maintained chi of short snakes, which nobody reads), so a continued run's checkpoints equal an uninterrupted run's byte for byte.
+constexpr uint32_t CKPT_VERSION = 1;
+static const char kEnvMagic[8] = {'s', 'n', 'k', '-', 'e', 'n', 'v', 0};
+static const char kReplayMagic[8] = {'s', 'n', 'k', '-', 'r', 'p', 'l', 0};
+struct EnvCkptHeader {
+    char magic[8];
+    uint32_t version, flags;            // CKPT_VERSION; the snk_create flags
+    int64_t n;
+    uint64_t seed, step_counter;        // the internal generator's key and call count
+    int32_t food_n, reserved;
+    uint8_t food_rc[2 * MAX_FOOD];      // the food list, 1-based (row, col) pairs as snk_set_food_list_host takes it
+};
+struct ReplayCkptHeader {
+    char magic[8];
+    uint32_t version, record_bytes;
+    int64_t capacity, total;            // transitions stored since the last clear
+    uint64_t draws;                     // snk_replay_sample_indices calls so far
+};
+static_assert(sizeof(EnvCkptHeader) == 176 && sizeof(ReplayCkptHeader) == 40, "blob headers are part of the format");
+constexpr size_t ENV_STATE_BYTES = 52;  // per env: occ pocc clo chi cons misc (u64) + ret (f32)
+static const char *const kEnvRuleText[] = {
+    "", "unused bits of misc set (error bits beyond 3, bits 56..63)", "head outside the board (the wall only for a lost env)",
+    "tail not an interior cell", "food neither an interior cell nor the no-food code", "previous food neither an interior cell nor the no-food code",
+    "length outside 2..64", "step count above 500 (499 for a live env)", "consumed food entries outside the food list",
+    "previous direction is not the chain's last move", "direction chain leaves the board or crosses itself",
+    "direction chain does not end on the tail", "occupancy disagrees with the direction chain"};
+static const char *const kReplayRuleText[] = {"", "action index above 2", "done above 1", "mask bits above 7", "previous direction above 3"};
+
+// the env arrays in blob order: device pointer and bytes per env
+static void env_arrays(const EnvState &s, void *p[7], size_t b[7]) {
+    void *q[7] = {s.occ, s.pocc, s.clo, s.chi, s.cons, s.misc, s.ret};
+    for (int k = 0; k < 7; k++) { p[k] = q[k]; b[k] = k < 6 ? 8 : 4; }
+}
+
+// device scratch of a load: the validation result (8 bytes, set to ~0 = no failure) and, 256 bytes in, the blob's arrays;
+// freed by the destructor on every path
+struct LoadScratch {
+    uint8_t *p = nullptr;
+    ~LoadScratch() { if (p) cudaFree(p); }
+    unsigned long long *first() const { return reinterpret_cast<unsigned long long *>(p); }
+    uint8_t *data() const { return p + 256; }
+};
+static int load_scratch(LoadScratch &sc, const void *src_host, size_t bytes, cudaStream_t st) {
+    SNK_CUDA(cudaMalloc((void **)&sc.p, 256 + bytes));
+    SNK_CUDA(cudaMemsetAsync(sc.p, 0xFF, 8, st));
+    if (bytes) SNK_CUDA(cudaMemcpyAsync(sc.data(), src_host, bytes, cudaMemcpyHostToDevice, st));
+    return SNK_OK;
+}
+// the validation result: index of the lowest failing record (-1 if none) and its rule
+static int load_verdict(const LoadScratch &sc, cudaStream_t st, long long *idx, int *rule) {
+    SNK_CUDA(cudaGetLastError());
+    unsigned long long f = 0;
+    SNK_CUDA(cudaMemcpyAsync(&f, sc.first(), 8, cudaMemcpyDeviceToHost, st));
+    SNK_CUDA(cudaStreamSynchronize(st));
+    *idx = f == ~0ull ? -1 : (long long)(f >> 8);
+    *rule = (int)(f & 0xFF);
     return SNK_OK;
 }
 
@@ -2019,6 +2158,156 @@ int snk_replay_gather_host(snk_replay r, const int64_t *idx_host, int64_t B, flo
     if (dones) SNK_CUDA(cudaMemcpyAsync(dones, d_dn, (size_t)B, cudaMemcpyDeviceToHost, st));
     if (mask) SNK_CUDA(cudaMemcpyAsync(mask, d_mk, 3 * (size_t)B, cudaMemcpyDeviceToHost, st));
     SNK_CUDA(cudaStreamSynchronize(st));
+    return SNK_OK;
+}
+
+// ---- checkpoints: save_trainer / load_trainer (utils.jl:408-418), save_buffer / load_buffer (utils.jl:316-340) -----------
+int snk_env_checkpoint_bytes(snk_handle h, size_t *bytes) {
+    if (h == nullptr || bytes == nullptr) return fail(SNK_ERR_INVALID, "%s: null argument", __func__);
+    *bytes = sizeof(EnvCkptHeader) + ENV_STATE_BYTES * (size_t)h->n;
+    return SNK_OK;
+}
+
+int snk_env_save_host(snk_handle h, void *blob_host, size_t bytes) {
+    SNK_CHECK_HANDLE(h);
+    SNK_REQUIRE(blob_host != nullptr, "null blob");
+    size_t need = 0;
+    snk_env_checkpoint_bytes(h, &need);
+    if (bytes != need) return fail(SNK_ERR_INVALID, "%s: blob of %zu bytes, the checkpoint has %zu", __func__, bytes, need);
+    EnvCkptHeader hd;
+    memset(&hd, 0, sizeof(hd));
+    memcpy(hd.magic, kEnvMagic, 8);
+    hd.version = CKPT_VERSION; hd.flags = h->flags; hd.n = h->n; hd.seed = h->seed; hd.step_counter = h->step_counter;
+    hd.food_n = h->food.n;
+    for (int i = 0; i < h->food.n; i++) {
+        hd.food_rc[2 * i] = (uint8_t)((h->food.bit[i] & 7) + 2);
+        hd.food_rc[2 * i + 1] = (uint8_t)((h->food.bit[i] >> 3) + 2);
+    }
+    memcpy(blob_host, &hd, sizeof(hd));
+    void *p[7];
+    size_t b[7];
+    env_arrays(h->s, p, b);
+    uint8_t *dst = (uint8_t *)blob_host + sizeof(hd);
+    for (int k = 0; k < 7; k++) {
+        SNK_CUDA(cudaMemcpyAsync(dst, p[k], b[k] * (size_t)h->n, cudaMemcpyDeviceToHost, h->stream));
+        dst += b[k] * (size_t)h->n;
+    }
+    SNK_CUDA(cudaStreamSynchronize(h->stream));
+    return SNK_OK;
+}
+
+int snk_env_load_host(snk_handle h, const void *blob_host, size_t bytes, int64_t *first_bad_env) {
+    if (first_bad_env != nullptr) *first_bad_env = -1;
+    SNK_CHECK_HANDLE(h);
+    SNK_REQUIRE(blob_host != nullptr, "null blob");
+    EnvCkptHeader hd;
+    if (bytes < sizeof(hd))
+        return fail(SNK_ERR_INVALID, "%s: truncated blob: %zu bytes, the header alone has %zu", __func__, bytes, sizeof(hd));
+    memcpy(&hd, blob_host, sizeof(hd));
+    if (memcmp(hd.magic, kEnvMagic, 8) != 0) return fail(SNK_ERR_INVALID, "%s: not an env checkpoint (wrong magic)", __func__);
+    if (hd.version != CKPT_VERSION)
+        return fail(SNK_ERR_INVALID, "%s: checkpoint format version %u, this library reads %u", __func__, hd.version, CKPT_VERSION);
+    if (hd.n != h->n) return fail(SNK_ERR_INVALID, "%s: checkpoint of %lld envs, the handle has %lld", __func__, (long long)hd.n, h->n);
+    if ((hd.flags ^ h->flags) & SNK_AUTO_RESET)
+        return fail(SNK_ERR_INVALID, "%s: checkpoint %s SNK_AUTO_RESET, the handle %s", __func__, (hd.flags & SNK_AUTO_RESET) ? "has" : "lacks",
+                    (h->flags & SNK_AUTO_RESET) ? "has it" : "does not");
+    const size_t arrays = ENV_STATE_BYTES * (size_t)h->n;
+    if (bytes != sizeof(hd) + arrays)
+        return fail(SNK_ERR_INVALID, "%s: blob of %zu bytes, a checkpoint of %lld envs has %zu", __func__, bytes, h->n, sizeof(hd) + arrays);
+    FoodTable ft;
+    if (set_food(ft, hd.food_rc, hd.food_n) != SNK_OK) {
+        char why[512];
+        snprintf(why, sizeof(why), "%s", err_buf());
+        return fail(SNK_ERR_INVALID, "%s: the checkpoint's food list: %s", __func__, why);
+    }
+    // the blob's arrays into device scratch, validated there; the live state is touched only if every env passes
+    LoadScratch sc;
+    int rc = load_scratch(sc, (const uint8_t *)blob_host + sizeof(hd), arrays, h->stream);
+    if (rc != SNK_OK) return rc;
+    EnvState s;
+    void *p[7], *q[7];
+    size_t b[7];
+    uint8_t *src = sc.data();
+    for (int k = 0; k < 7; k++) { q[k] = src; src += (k < 6 ? 8 : 4) * (size_t)h->n; }
+    s.occ = (u64 *)q[0]; s.pocc = (u64 *)q[1]; s.clo = (u64 *)q[2]; s.chi = (u64 *)q[3]; s.cons = (u64 *)q[4]; s.misc = (u64 *)q[5];
+    s.ret = (float *)q[6];
+    k_env_validate<<<nblocks(h->n, 256), 256, 0, h->stream>>>(s, h->n, ft.mask(), sc.first());
+    long long bad = -1;
+    int rule = 0;
+    if ((rc = load_verdict(sc, h->stream, &bad, &rule)) != SNK_OK) return rc;
+    if (bad >= 0) {
+        if (first_bad_env != nullptr) *first_bad_env = bad;
+        return fail(SNK_ERR_INVALID, "%s: env %lld of the checkpoint: %s", __func__, bad,
+                    rule < (int)(sizeof(kEnvRuleText) / sizeof(kEnvRuleText[0])) ? kEnvRuleText[rule] : "?");
+    }
+    env_arrays(h->s, p, b);
+    for (int k = 0; k < 7; k++) SNK_CUDA(cudaMemcpyAsync(p[k], q[k], b[k] * (size_t)h->n, cudaMemcpyDeviceToDevice, h->stream));
+    SNK_CUDA(cudaStreamSynchronize(h->stream));
+    h->seed = hd.seed;
+    h->step_counter = hd.step_counter;
+    h->food = ft;
+    return SNK_OK;
+}
+
+int snk_replay_checkpoint_bytes(snk_replay r, size_t *bytes) {
+    if (r == nullptr || bytes == nullptr) return fail(SNK_ERR_INVALID, "%s: null argument", __func__);
+    const long long filled = r->total < r->capacity ? r->total : r->capacity;
+    *bytes = sizeof(ReplayCkptHeader) + (size_t)filled * 128;
+    return SNK_OK;
+}
+
+int snk_replay_save_host(snk_replay r, void *blob_host, size_t bytes) {
+    SNK_REQUIRE(r != nullptr && blob_host != nullptr, "null argument");
+    size_t need = 0;
+    snk_replay_checkpoint_bytes(r, &need);
+    if (bytes != need) return fail(SNK_ERR_INVALID, "%s: blob of %zu bytes, the checkpoint has %zu", __func__, bytes, need);
+    DeviceGuard guard(r->device);
+    ReplayCkptHeader hd;
+    memset(&hd, 0, sizeof(hd));
+    memcpy(hd.magic, kReplayMagic, 8);
+    hd.version = CKPT_VERSION; hd.record_bytes = 128; hd.capacity = r->capacity; hd.total = r->total; hd.draws = r->draws;
+    memcpy(blob_host, &hd, sizeof(hd));
+    SNK_CUDA(cudaDeviceSynchronize());                     // the steps that store into the ring run on the env's stream
+    if (bytes > sizeof(hd)) SNK_CUDA(cudaMemcpy((uint8_t *)blob_host + sizeof(hd), r->ring, bytes - sizeof(hd), cudaMemcpyDeviceToHost));
+    return SNK_OK;
+}
+
+int snk_replay_load_host(snk_replay r, const void *blob_host, size_t bytes, int64_t *first_bad_slot) {
+    if (first_bad_slot != nullptr) *first_bad_slot = -1;
+    SNK_REQUIRE(r != nullptr && blob_host != nullptr, "null argument");
+    ReplayCkptHeader hd;
+    if (bytes < sizeof(hd))
+        return fail(SNK_ERR_INVALID, "%s: truncated blob: %zu bytes, the header alone has %zu", __func__, bytes, sizeof(hd));
+    memcpy(&hd, blob_host, sizeof(hd));
+    if (memcmp(hd.magic, kReplayMagic, 8) != 0) return fail(SNK_ERR_INVALID, "%s: not a replay checkpoint (wrong magic)", __func__);
+    if (hd.version != CKPT_VERSION || hd.record_bytes != 128)
+        return fail(SNK_ERR_INVALID, "%s: checkpoint format version %u (records of %u bytes), this library reads %u (128)", __func__,
+                    hd.version, hd.record_bytes, CKPT_VERSION);
+    if (hd.capacity != r->capacity)
+        return fail(SNK_ERR_INVALID, "%s: checkpoint of a ring of %lld, this ring holds %lld", __func__, (long long)hd.capacity, r->capacity);
+    if (hd.total < 0) return fail(SNK_ERR_INVALID, "%s: negative count of stored transitions", __func__);
+    const long long filled = hd.total < hd.capacity ? hd.total : hd.capacity;
+    const size_t recs = (size_t)filled * 128;
+    if (bytes != sizeof(hd) + recs)
+        return fail(SNK_ERR_INVALID, "%s: blob of %zu bytes, a checkpoint of %lld records has %zu", __func__, bytes, filled, sizeof(hd) + recs);
+    DeviceGuard guard(r->device);
+    LoadScratch sc;
+    int rc = load_scratch(sc, (const uint8_t *)blob_host + sizeof(hd), recs, nullptr);
+    if (rc != SNK_OK) return rc;
+    const uint4 *ring = reinterpret_cast<const uint4 *>(sc.data());
+    if (filled > 0) k_replay_validate<<<nblocks(filled, 256), 256>>>(ring, filled, sc.first());
+    long long bad = -1;
+    int rule = 0;
+    if ((rc = load_verdict(sc, nullptr, &bad, &rule)) != SNK_OK) return rc;
+    if (bad >= 0) {
+        if (first_bad_slot != nullptr) *first_bad_slot = bad;
+        return fail(SNK_ERR_INVALID, "%s: record %lld of the checkpoint: %s", __func__, bad,
+                    rule < (int)(sizeof(kReplayRuleText) / sizeof(kReplayRuleText[0])) ? kReplayRuleText[rule] : "?");
+    }
+    SNK_CUDA(cudaDeviceSynchronize());                     // nothing in flight reads or writes the ring any more
+    if (recs) SNK_CUDA(cudaMemcpy(r->ring, sc.data(), recs, cudaMemcpyDeviceToDevice));
+    r->total = hd.total;
+    r->draws = hd.draws;
     return SNK_OK;
 }
 

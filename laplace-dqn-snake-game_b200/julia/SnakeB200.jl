@@ -17,7 +17,7 @@ export BatchedSnakeGame, available_actions, step!, step_fused!, virtual_step, as
        GramShard, export_handle, connect!, run!, planes,
        step_device!, step_abs_device!, step_fused_device!, rollout_device!, state_device!, losing_mask_device!,
        lost_device!, steps_device!, error_flags_device!, count_errors, seed!, set_stream!, num_envs, library_version,
-       default_food_list, device_alloc, device_free, compression_supported
+       default_food_list, device_alloc, device_free, compression_supported, checkpoint, restore!
 
 const lib = get(ENV, "SNAKE_B200_LIB", joinpath(@__DIR__, "..", "libsnake_b200.so"))
 
@@ -295,6 +295,40 @@ stack_exp(r::DeviceReplayBuffer, d_idx::Ptr{Int64}, B::Integer, d_states::Ptr{Fl
                 (Ptr{Cvoid}, Ptr{Int64}, Int64, Ptr{Float32}, Ptr{Float32}, Ptr{UInt8}, Ptr{Float32}, Ptr{UInt8}, Ptr{UInt8},
                  Ptr{Float32}, Ptr{Int32}, Ptr{Cvoid}),
                 r.handle, d_idx, B, d_states, d_next, d_actions, d_rewards, d_dones, d_mask, C_NULL, C_NULL, C_NULL))
+
+# ---- checkpoints: save_trainer / load_trainer (utils.jl:408-418), save_buffer / load_buffer (utils.jl:316-340) -----------
+"""The library's checkpoint of the games (seed, generator counter, food list, every game's state) as bytes: write them
+anywhere; `restore!` continues bit for bit."""
+function checkpoint(g::BatchedSnakeGame)
+    n = Ref{Csize_t}(0)
+    check(ccall((:snk_env_checkpoint_bytes, lib), Cint, (Ptr{Cvoid}, Ref{Csize_t}), g.handle, n))
+    blob = Vector{UInt8}(undef, n[])
+    check(ccall((:snk_env_save_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Csize_t), g.handle, blob, length(blob)))
+    return blob
+end
+"""Load a `checkpoint(g)` of games with the same N and auto-reset flag; a refused blob (SnakeB200Error naming the cause and
+the first failing game) leaves `g` as it was.  The host mirrors are refreshed from the device."""
+function restore!(g::BatchedSnakeGame, blob::Vector{UInt8})
+    bad = Ref{Int64}(-1)
+    check(ccall((:snk_env_load_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Csize_t, Ref{Int64}), g.handle, blob, length(blob), bad))
+    virtual_step(g)
+    assemble_state!(g)
+    return g
+end
+"""The ring's checkpoint (the filled records, the stored count, the sampler's call count) as bytes."""
+function checkpoint(r::DeviceReplayBuffer)
+    n = Ref{Csize_t}(0)
+    check(ccall((:snk_replay_checkpoint_bytes, lib), Cint, (Ptr{Cvoid}, Ref{Csize_t}), r.handle, n))
+    blob = Vector{UInt8}(undef, n[])
+    check(ccall((:snk_replay_save_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Csize_t), r.handle, blob, length(blob)))
+    return blob
+end
+"""Load a `checkpoint(r)` of a ring of the same capacity; a refused blob leaves `r` as it was."""
+function restore!(r::DeviceReplayBuffer, blob::Vector{UInt8})
+    bad = Ref{Int64}(-1)
+    check(ccall((:snk_replay_load_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Csize_t, Ref{Int64}), r.handle, blob, length(blob), bad))
+    return r
+end
 
 # ---- Q-net forward (structs.jl:127-139) from Flux.destructure(q_net) ------------------------------------------
 mutable struct DeviceQNet

@@ -169,6 +169,28 @@ class QNet:
         _check(lib().snk_qnet_set_params(self._q, p, st))
         self._updated = True
 
+    def load_params(self, theta):
+        """θ = theta: (181,395) float32, a tensor on any device or a numpy array, in Flux.destructure order; every layout
+        re-derived on the device (snk_qnet_set_params), enqueued on the current stream."""
+        from . import _check, _ptr, lib
+        t = torch.as_tensor(theta)
+        if t.dtype != torch.float32 or t.numel() != N_PARAMS:
+            raise ValueError("load_params: theta must be %d float32 values, got %d %s" % (N_PARAMS, t.numel(), t.dtype))
+        t = t.reshape(-1).to(self.device).contiguous()
+        st = C.c_void_p(torch.cuda.current_stream(self.device).cuda_stream)
+        _check(lib().snk_qnet_set_params(self._q, _ptr(t, torch.float32, N_PARAMS, self.device), st))
+        self._updated = True
+
+    def state_dict(self):
+        """{'theta': (181,395) f32 CPU tensor, 'precision'}"""
+        return {"theta": self.theta_device.cpu(), "precision": self.precision}
+
+    def load_state_dict(self, d):
+        """θ of a state_dict(); the precision must be this net's"""
+        if not isinstance(d, dict) or "theta" not in d or d.get("precision") != self.precision:
+            raise ValueError("a QNet state_dict of precision %r with 'theta' is required" % self.precision)
+        self.load_params(d["theta"])
+
     def overflow(self):
         """f32 mode: True if an activation left the fp16 range of the split operands since the last call (synchronises)."""
         from . import _check, lib
@@ -199,3 +221,17 @@ class RMSProp:
         if self.acc is None:
             self.acc = torch.zeros(N_PARAMS, dtype=torch.float32, device=device)
         return self.acc
+
+    def state_dict(self):
+        """{'eta', 'rho', 'epsilon', 'acc': (181,395) f32 CPU tensor, or None before the first update}"""
+        return {"eta": self.eta, "rho": self.rho, "epsilon": self.epsilon, "acc": None if self.acc is None else self.acc.cpu()}
+
+    def load_state_dict(self, d, device):
+        """the hyper-parameters and `acc` of a state_dict(); acc goes to `device` (the net's)"""
+        if not isinstance(d, dict) or not all(isinstance(d.get(k), float) for k in ("eta", "rho", "epsilon")) or "acc" not in d:
+            raise ValueError("an RMSProp state_dict holds the floats 'eta', 'rho', 'epsilon' and 'acc'")
+        acc = d["acc"]
+        if acc is not None and (not isinstance(acc, torch.Tensor) or acc.dtype != torch.float32 or acc.numel() != N_PARAMS):
+            raise ValueError("RMSProp acc must be None or %d float32 values" % N_PARAMS)
+        self.eta, self.rho, self.epsilon = d["eta"], d["rho"], d["epsilon"]
+        self.acc = None if acc is None else acc.reshape(-1).to(device, copy=True).contiguous()
