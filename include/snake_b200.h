@@ -60,7 +60,7 @@ extern "C" {
 #define SNK_ERR_CUDA (-2)      /* a CUDA runtime call failed */
 #define SNK_ERR_NODEVICE (-3)  /* no CUDA device / not a Blackwell part */
 #define SNK_ERR_UNSUPPORTED (-4)
-#define SNK_ERR_TIMEOUT (-5)   /* a peer of the row-sharded Gram did not reach a barrier */
+#define SNK_ERR_TIMEOUT (-5)   /* a peer of the row-sharded Gram or of a learner group did not arrive in time */
 
 /* snk_create flags */
 #define SNK_AUTO_RESET 1u      /* a lost env is re-initialised (a fresh SnakeGame(), utils.jl:199) after its terminal outputs */
@@ -324,6 +324,33 @@ SNK_API int snk_qnet_train_step(snk_qnet q, const float *states, const uint8_t *
                                 void *cuda_stream);
 SNK_API int snk_qnet_set_params(snk_qnet q, const float *theta_dev, void *cuda_stream);   /* update_target_net!, utils.jl:469-472 */
 SNK_API int snk_qnet_params(snk_qnet q, const float **theta_dev);
+/* ---- the data-parallel learner: one Q-net trained on every GPU of a box (DESIGN §5f) ----------------------------------
+ * A group has `world` ranks (1 .. 16), one snk_qnet_group per rank, each wrapping a Q-net handle; all ranks' handles hold the
+ * same θ.  snk_qnet_group_train_step(g, states, actions, targets, B_local, ...) takes the arguments of snk_qnet_train_step
+ * with this rank's own B_local >= 1 transitions.  Rank r computes its per-sample rows, continues the Float64 running sum
+ * rank r - 1 published (rank 0 starts from 0) with its rows in sample order and publishes the sum and the running sample
+ * count; every rank then applies the final sum of rank world - 1 with B = the chained count.  So after every update every
+ * rank holds the same θ, acc, g and loss, and they equal snk_qnet_train_step on the ranks' minibatches concatenated in rank
+ * order, bit for bit, for any world (world = 1 is snk_qnet_train_step).  Ranks wait for each other on the device (flags over
+ * peer memory, no host synchronisation); a wait that gives up after ~20 s sets the flag snk_qnet_group_status_host reports.
+ * Every rank must call train_step the same number of times.  A rank keeps all B_local rows resident: B_local x 0.73 MB of
+ * device memory, plus 2.9 MB of peer memory.
+ * Set-up, once: create -> export_host (64 bytes) -> [the host language moves every rank's 64 bytes to every rank: MPI,
+ * Distributed.jl, torch.distributed, a file ...] -> connect_host(world x 64 bytes in rank order, own entry ignored).
+ * connect_local wires the groups of ONE process (virtual ranks on one GPU, each driven from its own stream).  The Q-net must
+ * outlive its group. */
+#define SNK_QNET_GROUP_HANDLE_BYTES 64
+typedef struct snk_qnet_group_s *snk_qnet_group;
+SNK_API int snk_qnet_group_create(snk_qnet_group *out, snk_qnet q, int world, int rank);
+SNK_API int snk_qnet_group_destroy(snk_qnet_group g);
+SNK_API int snk_qnet_group_export_host(snk_qnet_group g, uint8_t *handle64);
+SNK_API int snk_qnet_group_connect_host(snk_qnet_group g, const uint8_t *handles_world_x_64, int n_handles);
+SNK_API int snk_qnet_group_connect_local(snk_qnet_group g, const snk_qnet_group *peers, int n_peers);
+SNK_API int snk_qnet_group_train_step(snk_qnet_group g, const float *states, const uint8_t *actions, const double *targets,
+                                      int64_t B_local, float *acc, double eta, double rho, double epsilon, float *grad_out,
+                                      float *loss_out, void *cuda_stream);
+/* SNK_ERR_TIMEOUT if a wait gave up on a peer (synchronises) */
+SNK_API int snk_qnet_group_status_host(snk_qnet_group g, int *timed_out);
 /* profiling aid (SNK_QNET_BF16): device buffer of 512 int64 that receives clock64 stamps of the conv phases of CTA 0 on every
  * later forward (64 slots for each of its first 8 iterations, tools/qnet_phases17.py); NULL switches it off */
 SNK_API int snk_qnet_debug_timing(snk_qnet q, long long *device_buf);

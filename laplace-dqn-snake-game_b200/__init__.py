@@ -154,6 +154,11 @@ def lib():
         "snk_qnet_sample_grads": [vp, vp, vp, vp, i64, vp, vp, i64, vp, i64, vp, vp],
         "snk_qnet_train_step": [vp, vp, vp, vp, i64, vp, f64, f64, f64, vp, vp, vp],
         "snk_qnet_set_params": [vp, vp, vp], "snk_qnet_params": [vp, C.POINTER(vp)],
+        "snk_qnet_group_create": [C.POINTER(vp), vp, i32, i32], "snk_qnet_group_destroy": [vp],
+        "snk_qnet_group_export_host": [vp, vp], "snk_qnet_group_connect_host": [vp, vp, i32],
+        "snk_qnet_group_connect_local": [vp, vp, i32],
+        "snk_qnet_group_train_step": [vp, vp, vp, vp, i64, vp, f64, f64, f64, vp, vp, vp],
+        "snk_qnet_group_status_host": [vp, C.POINTER(i32)],
         "snk_gram_workspace_bytes": [i64, i64, i32, C.POINTER(C.c_size_t)],
         "snk_gram_pack": [vp, i32, i64, i64, vp, vp],
         "snk_gram": [vp, i64, i64, i32, i32, i32, vp, vp],

@@ -23,37 +23,23 @@
 #include <vector>
 
 #include "common.h"
+#include "peer.h"
 
 namespace snk {
 namespace gram_shard {
-
-constexpr int MAX_WORLD = 16;
 
 struct PeerFlags {
     unsigned long long *p[MAX_WORLD];
 };
 
 // thread r: publish my arrival at `epoch` in slot [rank] of rank r's flag array, then wait for rank r's arrival in my
-// slot [r].  Everything this stream did before the barrier is visible to a peer that has passed it (release at system
-// scope before the flag store, acquire on the flag load).  Bounded spin: a missing peer sets *timed_out, never hangs.
+// slot [r] (peer.h).  Everything this stream did before the barrier is visible to a peer that has passed it.
 __global__ void k_peer_barrier(PeerFlags peers, unsigned long long *mine, int world, int rank, unsigned long long epoch,
                                int *timed_out) {
     const int r = threadIdx.x;
     if (r >= world) return;
-    __threadfence_system();
-    asm volatile("st.release.sys.global.u64 [%0], %1;" ::"l"(peers.p[r] + rank), "l"(epoch) : "memory");
-    const long long t0 = clock64();
-    for (;;) {
-        unsigned long long v;
-        asm volatile("ld.acquire.sys.global.u64 %0, [%1];" : "=l"(v) : "l"(mine + r) : "memory");
-        if (v >= epoch) break;
-        if (clock64() - t0 > 40000000000ll) {        // ~20 s at 2 GHz
-            *timed_out = 1;
-            break;
-        }
-        __nanosleep(200);
-    }
-    __threadfence_system();
+    peer_signal(peers.p[r] + rank, epoch);
+    peer_wait(mine + r, epoch, timed_out);
 }
 
 // the ring schedule of one rank (see snk_gram_shard_schedule in the header)

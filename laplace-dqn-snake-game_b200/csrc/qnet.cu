@@ -39,6 +39,7 @@
 #include <new>
 
 #include "common.h"
+#include "peer.h"
 #include "qnet_theta.h"
 #include "sm100.h"
 
@@ -1108,14 +1109,17 @@ __device__ __forceinline__ void scatter_param(float w, int p, float *theta, uint
     }
 }
 
+// A running sum: [NP] Float64 sums of the rows, [NP] the loss, [NP + 1] the number of samples summed so far (exact in Float64).
+constexpr int SUM_LEN = qgrad::NP + 2;
+
 struct ApplyArgs {
-    const float *rows;           // [nrows][NP] per-sample gradient rows of one chunk of the minibatch (k_sample_grads), or NULL:
-    const float *losses;         //   no update, theta_src is the new theta (snk_qnet_set_params);  [nrows] per-sample losses
-    int nrows;
-    int first, last;             // the chunk is the first / the last of the minibatch
-    double *gsum;                // [NP + 1] Float64 running sums carried between chunks; [NP] = the loss
-    long long B;
-    const float *theta_src;
+    const float *theta_src;      // non-NULL: no update, theta_src is the new theta (snk_qnet_set_params)
+    const float *rows;           // [nrows][NP] per-sample gradient rows of one chunk of the minibatch (k_sample_grads)
+    const float *losses;         // [nrows] per-sample losses
+    int nrows;                   // 0 in the last pass of a learner group: the chain's final sum is the whole minibatch
+    const double *sum_in;        // [SUM_LEN] the running sum this chunk continues (a peer's in a learner group), NULL: 0
+    double *sum_out;             // [SUM_LEN] where a pass that is not the last leaves its running sum
+    int last;                    // the sum is complete: apply it, B = its sample count
     float *acc;                  // RMSProp state of theta
     double eta, rho, one_m_rho, eps;
     float *grad_out, *loss_out;  // optional
@@ -1124,26 +1128,30 @@ struct ApplyArgs {
     int *overflow;               // SNK_QNET_F32: a parameter left the fp16 range of the split operands; NULL in bf16 mode
 };
 
-// One thread per parameter (thread NP: the loss).  g = Float32(sum_i J_i / B), the sum a Float64 running sum in sample order,
-// rounded once: the order depends on B only.  Then Flux.Optimise's RMSProp (apply! + update!, utils.jl:466) with Julia's
-// promotions: Float64 hyper-parameters, Float32 arrays, every operation rounded on its own (no FMA contraction).
+// One thread per parameter (thread NP: the loss and the sample count).  g = Float32(sum_i J_i / B), the sum a Float64 running
+// sum in sample order, rounded once: the order depends on B only, wherever the chunks of the sum were added (one handle's
+// scratch chunks, or the ranks of a learner group, each continuing its predecessor's sum).  Then Flux.Optimise's RMSProp
+// (apply! + update!, utils.jl:466) with Julia's promotions: Float64 hyper-parameters, Float32 arrays, every operation rounded
+// on its own (no FMA contraction).
 constexpr int APPLY_THREADS = 256;
 __global__ void __launch_bounds__(APPLY_THREADS) k_qnet_train_apply(const ApplyArgs a) {
     using qgrad::NP;
     const int p = blockIdx.x * APPLY_THREADS + threadIdx.x;
     if (p > NP) return;
     float w;
-    if (a.rows != nullptr) {
+    if (a.theta_src == nullptr) {
         const float *src = p < NP ? a.rows + p : a.losses;
         const long long ld = p < NP ? NP : 1;
-        double s = a.first ? 0.0 : a.gsum[p];
+        double s = a.sum_in != nullptr ? a.sum_in[p] : 0.0;
 #pragma unroll 8
         for (int r = 0; r < a.nrows; r++) s = __dadd_rn(s, (double)src[r * ld]);
+        const double count = (a.sum_in != nullptr ? a.sum_in[NP + 1] : 0.0) + (double)a.nrows;
         if (!a.last) {
-            a.gsum[p] = s;
+            a.sum_out[p] = s;
+            if (p == NP) a.sum_out[NP + 1] = count;
             return;
         }
-        const float g = (float)__ddiv_rn(s, (double)a.B);
+        const float g = (float)__ddiv_rn(s, count);
         if (p == NP) {
             if (a.loss_out != nullptr) *a.loss_out = g;
             return;
@@ -1161,6 +1169,31 @@ __global__ void __launch_bounds__(APPLY_THREADS) k_qnet_train_apply(const ApplyA
     }
     if (a.overflow != nullptr && !(fabsf(w) <= 65504.0f)) *a.overflow = 1;
     scatter_param(w, p, a.theta, a.params);
+}
+
+// ---- the data-parallel learner group (snk_qnet_group_*, DESIGN §5f) ----------------------------------------------------
+// Rank r of R continues the running sum rank r - 1 published with its own rows and publishes the result; every rank then
+// applies the sum of rank R - 1.  The peer memory of a rank is ONE snk_ipc_alloc allocation (one 64-byte handle):
+//   [0, 8 MAX_WORLD)                   flags: slot q = the last update (epoch) whose running sum rank q has published
+//   GROUP_OFF_SUM + k GROUP_SUM_BYTES   the running sum (SUM_LEN doubles) this rank published at an update of parity k
+// Double buffering by parity is enough: a rank overwrites its sum of update e at update e + 2, and before that (in update
+// e + 1) it has waited for rank R - 1's sum of e + 1.  Rank R - 1 published e + 1 only after every rank had, and each rank
+// published e + 1 only after its last reads of update e (its predecessor's sum, rank R - 1's final sum) had finished.
+constexpr size_t GROUP_OFF_SUM = 256, GROUP_SUM_BYTES = (size_t)SUM_LEN * 8;
+constexpr size_t GROUP_PEER_BYTES = GROUP_OFF_SUM + 2 * GROUP_SUM_BYTES;
+
+struct GroupFlags {
+    unsigned long long *p[MAX_WORLD];
+};
+
+// One CTA, run on the rank's stream between the kernels of an update (a spinning kernel of one CTA leaves the GPU to the
+// other virtual ranks of one process, whatever stream each of them is on).  signal: thread q tells rank q that this rank has
+// published its sum of `epoch`; then thread 0 waits until rank `wait_for` (>= 0) has published its sum of `epoch`.
+__global__ void k_group_sync(GroupFlags peers, const unsigned long long *mine, int world, int rank, int signal, int wait_for,
+                             unsigned long long epoch, int *timed_out) {
+    const int q = threadIdx.x;
+    if (signal && q < world) peer_signal(peers.p[q] + rank, epoch);
+    if (q == 0 && wait_for >= 0) peer_wait(mine + wait_for, epoch, timed_out);
 }
 
 }  // namespace qnet
@@ -1184,7 +1217,7 @@ struct snk_qnet_s {
     // learner (snk_qnet_train_step): per-sample gradient rows of one chunk of the minibatch, grown on demand up to 2 * sms samples
     float *rows;
     float *row_loss;
-    double *gsum;                // NP + 1 running sums carried between chunks
+    double *gsum;                // the running sum (SUM_LEN) carried between chunks
     long long rows_cap;          // in samples
     // conv1's weights are kernel parameters read from w1h / b1h / w1f / b1f (DESIGN §5b): every write of the weights on the device
     // copies them into conv1_host and records conv1_ready; create, and after an update the next forward, waits for that event and
@@ -1192,6 +1225,21 @@ struct snk_qnet_s {
     float *conv1_host;           // pinned: P_W1 (288) then b1 (16)
     cudaEvent_t conv1_ready;
     int conv1_pending;
+};
+
+// one rank of a data-parallel learner (DESIGN §5f); the layout of `mem` is described at k_group_sync
+struct snk_qnet_group_s {
+    snk_qnet_s *q;
+    int world, rank, device;
+    bool connected;
+    unsigned long long epoch;    // updates so far
+    uint8_t *mem;                // this rank's flags and published sums (snk_ipc_alloc)
+    uint8_t *peer_mem[MAX_WORLD];
+    void *opened[MAX_WORLD];     // snk_ipc_import mappings to close
+    int *d_timed_out;
+    // ALL of this rank's rows stay resident (B_local x 0.73 MB): it cannot reduce a chunk before its predecessor's sum arrives
+    float *rows, *row_loss;
+    long long rows_cap;          // in samples
 };
 
 static void set_conv1(snk_qnet_s *q, const float *w1f, const float *b1f) {
@@ -1215,6 +1263,13 @@ static int fetch_conv1(snk_qnet_s *q) {
     set_conv1(q, q->conv1_host, q->conv1_host + 288);
     q->conv1_pending = 0;
     return SNK_OK;
+}
+
+static ApplyArgs rmsprop_args(float *acc, double eta, double rho, double epsilon, float *grad_out, float *loss_out) {
+    ApplyArgs a = {};
+    a.acc = acc; a.eta = eta; a.rho = rho; a.one_m_rho = 1.0 - rho; a.eps = epsilon;
+    a.grad_out = grad_out; a.loss_out = loss_out;
+    return a;
 }
 
 static int launch_apply(snk_qnet_s *q, ApplyArgs &a, cudaStream_t st) {
@@ -1308,19 +1363,17 @@ int snk_qnet_train_step(snk_qnet q, const float *states, const uint8_t *actions,
         q->rows_cap = 0;
         SNK_CUDA(cudaMalloc((void **)&q->rows, (size_t)need * qgrad::NP * 4));
         SNK_CUDA(cudaMalloc((void **)&q->row_loss, (size_t)need * 4));
-        if (q->gsum == nullptr) SNK_CUDA(cudaMalloc((void **)&q->gsum, (qgrad::NP + 1) * sizeof(double)));
+        if (q->gsum == nullptr) SNK_CUDA(cudaMalloc((void **)&q->gsum, SUM_LEN * sizeof(double)));
         q->rows_cap = need;
     }
-    ApplyArgs a = {};
-    a.rows = q->rows; a.losses = q->row_loss; a.gsum = q->gsum; a.B = B;
-    a.acc = acc; a.eta = eta; a.rho = rho; a.one_m_rho = 1.0 - rho; a.eps = epsilon;
-    a.grad_out = grad_out; a.loss_out = loss_out;
+    ApplyArgs a = rmsprop_args(acc, eta, rho, epsilon, grad_out, loss_out);
+    a.rows = q->rows; a.losses = q->row_loss; a.sum_out = q->gsum;
     for (long long s0 = 0; s0 < B; s0 += chunk) {
         const long long n = B - s0 < chunk ? B - s0 : chunk;
         int rc = qgrad::launch_sample_grads(q->theta, states + s0 * 200, actions + s0, targets + s0, n, nullptr, nullptr, 0, q->rows,
                                             qgrad::NP, q->row_loss, q->sms, st);
         if (rc != SNK_OK) return rc;
-        a.nrows = (int)n; a.first = s0 == 0; a.last = s0 + n == B;
+        a.nrows = (int)n; a.sum_in = s0 == 0 ? nullptr : q->gsum; a.last = s0 + n == B;
         if ((rc = launch_apply(q, a, st)) != SNK_OK) return rc;
     }
     return enqueue_conv1_refresh(q, st);
@@ -1449,6 +1502,140 @@ int snk_qnet_forward(snk_qnet q, const float *obs_f32, int64_t N, float *q_out_3
         k_qnet_head<false><<<grid, HB_THREADS, HeadCfg<false>::SMEM, st>>>(mx, mw, ha);
     }
     SNK_CUDA(cudaGetLastError());
+    return SNK_OK;
+}
+
+// ---- data-parallel learner group (DESIGN §5f) ----------------------------------------------------------------------------
+int snk_qnet_group_create(snk_qnet_group *out, snk_qnet q, int world, int rank) {
+    SNK_REQUIRE(out != nullptr, "null argument");
+    *out = nullptr;
+    SNK_REQUIRE(world >= 1 && world <= MAX_WORLD, "world must be 1 .. 16");
+    SNK_REQUIRE(rank >= 0 && rank < world, "rank must be 0 .. world - 1");
+    SNK_REQUIRE(q != nullptr, "null qnet");
+    DeviceGuard guard(q->device);
+    snk_qnet_group_s *g = new (std::nothrow) snk_qnet_group_s();
+    if (g == nullptr) return fail(SNK_ERR_INVALID, "out of host memory");
+    g->q = q; g->world = world; g->rank = rank; g->device = q->device;
+    auto build = [&]() -> int {
+        int rc;
+        if ((rc = snk_ipc_alloc((void **)&g->mem, GROUP_PEER_BYTES)) != SNK_OK) return rc;
+        SNK_CUDA(cudaMemset(g->mem, 0, GROUP_OFF_SUM));
+        SNK_CUDA(cudaMalloc((void **)&g->d_timed_out, sizeof(int)));
+        SNK_CUDA(cudaMemset(g->d_timed_out, 0, sizeof(int)));
+        return SNK_OK;
+    };
+    const int rc = build();
+    if (rc != SNK_OK) {
+        snk_qnet_group_destroy(g);
+        return rc;
+    }
+    g->peer_mem[rank] = g->mem;
+    g->connected = world == 1;
+    *out = g;
+    return SNK_OK;
+}
+
+int snk_qnet_group_destroy(snk_qnet_group g) {
+    if (g == nullptr) return SNK_OK;
+    DeviceGuard guard(g->device);
+    cudaDeviceSynchronize();
+    for (void *p : g->opened) if (p) snk_ipc_close(p);
+    if (g->mem) snk_ipc_free(g->mem);
+    if (g->d_timed_out) cudaFree(g->d_timed_out);
+    if (g->rows) cudaFree(g->rows);
+    if (g->row_loss) cudaFree(g->row_loss);
+    delete g;
+    return SNK_OK;
+}
+
+int snk_qnet_group_export_host(snk_qnet_group g, uint8_t *handle64) {
+    SNK_REQUIRE(g != nullptr && handle64 != nullptr, "null argument");
+    DeviceGuard guard(g->device);
+    return snk_ipc_export(g->mem, handle64);
+}
+
+int snk_qnet_group_connect_host(snk_qnet_group g, const uint8_t *handles, int n_handles) {
+    SNK_REQUIRE(g != nullptr && handles != nullptr, "null argument");
+    SNK_REQUIRE(n_handles == g->world, "one handle per rank is needed");
+    SNK_REQUIRE(!g->connected || g->world == 1, "already connected");
+    DeviceGuard guard(g->device);
+    for (int r = 0; r < g->world; r++) {
+        if (r == g->rank) continue;
+        void *p = nullptr;
+        int rc = snk_ipc_import(handles + (size_t)r * SNK_QNET_GROUP_HANDLE_BYTES, &p);
+        if (rc != SNK_OK) return rc;
+        g->opened[r] = p;
+        g->peer_mem[r] = (uint8_t *)p;
+    }
+    g->connected = true;
+    return SNK_OK;
+}
+
+int snk_qnet_group_connect_local(snk_qnet_group g, const snk_qnet_group *peers, int n_peers) {
+    SNK_REQUIRE(g != nullptr && peers != nullptr, "null argument");
+    SNK_REQUIRE(n_peers == g->world, "one group per rank is needed");
+    for (int r = 0; r < g->world; r++)
+        SNK_REQUIRE(peers[r] != nullptr && peers[r]->rank == r && peers[r]->world == g->world && peers[r]->device == g->device,
+                    "peer list does not match");
+    SNK_REQUIRE(peers[g->rank] == g, "peer list does not match");
+    for (int r = 0; r < g->world; r++) g->peer_mem[r] = peers[r]->mem;
+    g->connected = true;
+    return SNK_OK;
+}
+
+// k_sample_grads into the resident rows -> wait for rank - 1's sum -> continue it with my rows and publish -> wait for rank
+// world - 1's sum -> apply it (RMSProp + every layout) -> conv1 refresh.  No host synchronisation.
+int snk_qnet_group_train_step(snk_qnet_group g, const float *states, const uint8_t *actions, const double *targets,
+                              int64_t B_local, float *acc, double eta, double rho, double epsilon, float *grad_out,
+                              float *loss_out, void *cuda_stream) {
+    SNK_REQUIRE(g != nullptr, "null group");
+    SNK_REQUIRE(g->connected, "group not connected (snk_qnet_group_connect_host / connect_local)");
+    SNK_REQUIRE(B_local >= 1 && B_local <= (1ll << 30), "B_local must be 1 .. 2^30");
+    SNK_REQUIRE(eta > 0.0 && rho >= 0.0 && rho < 1.0 && epsilon >= 0.0, "RMSProp needs eta > 0, 0 <= rho < 1 and epsilon >= 0");
+    SNK_REQUIRE(states != nullptr && actions != nullptr && targets != nullptr && acc != nullptr, "null argument");
+    DeviceGuard guard(g->device);
+    snk_qnet_s *q = g->q;
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    if (g->rows_cap < B_local) {
+        SNK_CUDA(cudaStreamSynchronize(st));
+        if (g->rows) { SNK_CUDA(cudaFree(g->rows)); g->rows = nullptr; }
+        if (g->row_loss) { SNK_CUDA(cudaFree(g->row_loss)); g->row_loss = nullptr; }
+        g->rows_cap = 0;
+        SNK_CUDA(cudaMalloc((void **)&g->rows, (size_t)B_local * qgrad::NP * 4));
+        SNK_CUDA(cudaMalloc((void **)&g->row_loss, (size_t)B_local * 4));
+        g->rows_cap = B_local;
+    }
+    int rc = qgrad::launch_sample_grads(q->theta, states, actions, targets, B_local, nullptr, nullptr, 0, g->rows, qgrad::NP,
+                                        g->row_loss, q->sms, st);
+    if (rc != SNK_OK) return rc;
+    const unsigned long long e = ++g->epoch;
+    const size_t sum_off = GROUP_OFF_SUM + (e & 1) * GROUP_SUM_BYTES;
+    GroupFlags peers;
+    for (int r = 0; r < g->world; r++) peers.p[r] = (unsigned long long *)g->peer_mem[r];
+    const unsigned long long *mine = (const unsigned long long *)g->mem;
+    auto sync = [&](int signal, int wait_for) -> int {
+        k_group_sync<<<1, 32, 0, st>>>(peers, mine, g->world, g->rank, signal, wait_for, e, g->d_timed_out);
+        SNK_CUDA(cudaGetLastError());
+        return SNK_OK;
+    };
+    if (g->rank > 0 && (rc = sync(0, g->rank - 1)) != SNK_OK) return rc;
+    ApplyArgs a = rmsprop_args(acc, eta, rho, epsilon, grad_out, loss_out);
+    a.rows = g->rows; a.losses = g->row_loss; a.nrows = (int)B_local;
+    a.sum_in = g->rank > 0 ? (const double *)(g->peer_mem[g->rank - 1] + sum_off) : nullptr;
+    a.sum_out = (double *)(g->mem + sum_off);
+    if ((rc = launch_apply(q, a, st)) != SNK_OK) return rc;
+    if ((rc = sync(1, g->world - 1)) != SNK_OK) return rc;
+    a.rows = a.losses = nullptr; a.nrows = 0;
+    a.sum_in = (const double *)(g->peer_mem[g->world - 1] + sum_off); a.sum_out = nullptr; a.last = 1;
+    if ((rc = launch_apply(q, a, st)) != SNK_OK) return rc;
+    return enqueue_conv1_refresh(q, st);
+}
+
+int snk_qnet_group_status_host(snk_qnet_group g, int *timed_out) {
+    SNK_REQUIRE(g != nullptr && timed_out != nullptr, "null argument");
+    DeviceGuard guard(g->device);
+    SNK_CUDA(cudaMemcpy(timed_out, g->d_timed_out, 4, cudaMemcpyDeviceToHost));
+    if (*timed_out) return fail(SNK_ERR_TIMEOUT, "snk_qnet_group: a peer did not publish its running sum within ~20 s");
     return SNK_OK;
 }
 

@@ -14,7 +14,7 @@ export BatchedSnakeGame, available_actions, step!, step_fused!, virtual_step, as
        epsilon_greedy, masked_target, center_columns!, reset!, set_food_list!, score, lost,
        DeviceReplayBuffer, store_step!, store_step_host!, store_step_host_bits!, stack_exp, sample_indices, DeviceQNet, forward!, overflowed,
        sample_grads!, RMSPropState, train_step!, update_target_net!, params_device, store_snapshot!, gram!, sample_model_weights!, empty_buffer!, patch_reset_obs!,
-       GramShard, export_handle, connect!, run!, planes,
+       GramShard, export_handle, connect!, run!, planes, LearnerGroup, check_peers,
        step_device!, step_abs_device!, step_fused_device!, rollout_device!, state_device!, losing_mask_device!,
        lost_device!, steps_device!, error_flags_device!, count_errors, seed!, set_stream!, num_envs, library_version,
        default_food_list, device_alloc, device_free, compression_supported, checkpoint, restore!
@@ -524,6 +524,45 @@ function planes(g::GramShard)
     hi = Ref{Ptr{Cvoid}}(C_NULL); lo = Ref{Ptr{Cvoid}}(C_NULL); pitch = Ref{Int64}(0)
     check(ccall((:snk_gram_shard_planes, lib), Cint, (Ptr{Cvoid}, Ref{Ptr{Cvoid}}, Ref{Ptr{Cvoid}}, Ref{Int64}), g.handle, hi, lo, pitch))
     return hi[], lo[], Int(pitch[])
+end
+
+# ---- data-parallel learner: one process (Distributed.jl worker / MPI rank) per GPU, one Q-net trained on all of them ---------
+"""Rank `rank` of a learner group of `world` ranks around `q` (DESIGN §5f).  Every rank's `q` holds the same θ; after each
+`train_step!` every rank holds θ, acc, g and loss of `train_step!(q, ...)` on the ranks' minibatches concatenated in rank
+order, bit for bit.  `q` must outlive the group."""
+mutable struct LearnerGroup
+    handle::Ptr{Cvoid}
+    world::Int
+    q::DeviceQNet
+    function LearnerGroup(q::DeviceQNet, world::Integer, rank::Integer)
+        h = Ref{Ptr{Cvoid}}(C_NULL)
+        check(ccall((:snk_qnet_group_create, lib), Cint, (Ref{Ptr{Cvoid}}, Ptr{Cvoid}, Cint, Cint), h, q.handle, world, rank))
+        g = new(h[], world, q)
+        finalizer(x -> ccall((:snk_qnet_group_destroy, lib), Cint, (Ptr{Cvoid},), x.handle), g)
+        return g
+    end
+end
+"""64 bytes to send to every other rank"""
+function export_handle(g::LearnerGroup)
+    h = Vector{UInt8}(undef, 64)
+    check(ccall((:snk_qnet_group_export_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}), g.handle, h))
+    return h
+end
+"""`handles` = the 64-byte handles of ALL ranks, concatenated in rank order"""
+connect!(g::LearnerGroup, handles::Vector{UInt8}) =
+    check(ccall((:snk_qnet_group_connect_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Cint), g.handle, handles, length(handles) ÷ 64))
+"""This rank's part of one group update: its own B_local transitions (device pointers as for `train_step!`).  Enqueued on
+the default stream; every rank must call it the same number of times."""
+train_step!(g::LearnerGroup, opt::RMSPropState, d_states::Ptr{Float32}, d_actions::Ptr{UInt8}, d_targets::Ptr{Float64},
+            B_local::Integer; d_grad::Ptr{Float32} = Ptr{Float32}(C_NULL), d_loss::Ptr{Float32} = Ptr{Float32}(C_NULL)) =
+    check(ccall((:snk_qnet_group_train_step, lib), Cint,
+                (Ptr{Cvoid}, Ptr{Float32}, Ptr{UInt8}, Ptr{Float64}, Int64, Ptr{Float32}, Cdouble, Cdouble, Cdouble, Ptr{Float32},
+                 Ptr{Float32}, Ptr{Cvoid}),
+                g.handle, d_states, d_actions, d_targets, B_local, opt.d_acc, opt.eta, opt.rho, opt.epsilon, d_grad, d_loss, C_NULL))
+"""throws if a wait of this rank gave up on a peer (synchronises)"""
+function check_peers(g::LearnerGroup)
+    t = Ref{Cint}(0)
+    check(ccall((:snk_qnet_group_status_host, lib), Cint, (Ptr{Cvoid}, Ref{Cint}), g.handle, t))
 end
 
 """`bytes` of device memory on `device` for the outputs of the fused step; with `compressible`, memory with generic L2

@@ -199,6 +199,118 @@ class QNet:
         return bool(f.value)
 
 
+GROUP_HANDLE_BYTES = 64          # SNK_QNET_GROUP_HANDLE_BYTES
+
+
+class LearnerGroup:
+    """One rank of a data-parallel learner (snk_qnet_group, DESIGN §5f): R ranks, each with its own QNet holding the same θ and
+    its own local minibatch.  train_step continues the Float64 running sum of the gradient rows that rank - 1 published and
+    every rank applies the sum of rank R - 1, so after each update every rank holds the same θ, acc, g and loss, equal bit for
+    bit to QNet.train_step on the ranks' minibatches concatenated in rank order.  The ranks wait for each other on the
+    device.  Set-up: handle() on every rank, then connect(every rank's handle, in rank order)."""
+
+    def __init__(self, net, world, rank):
+        from . import _check, lib
+        self.net, self.world, self.rank = net, int(world), int(rank)
+        self._g = C.c_void_p()
+        _check(lib().snk_qnet_group_create(C.byref(self._g), net._q, self.world, self.rank))
+
+    def handle(self):
+        """this rank's 64-byte handle (bytes), to be sent to every other rank"""
+        from . import _check, lib
+        h = (C.c_uint8 * GROUP_HANDLE_BYTES)()
+        _check(lib().snk_qnet_group_export_host(self._g, h))
+        return bytes(h)
+
+    def connect(self, handles):
+        """handles: every rank's handle() in rank order (this rank's own entry is ignored)"""
+        from . import _check, lib
+        blob = b"".join(bytes(h) for h in handles)
+        _check(lib().snk_qnet_group_connect_host(self._g, (C.c_uint8 * len(blob)).from_buffer_copy(blob),
+                                                 len(handles)))
+
+    def train_step(self, states, actions, targets, opt, want_grad=False):
+        """QNet.train_step of this rank's B_r transitions as part of the group's update; (loss, g) are the whole update's
+        (the same on every rank).  Enqueued on the current stream; every rank must call it the same number of times."""
+        from . import _check, _ptr, lib
+        net, dev = self.net, self.net.device
+        B = states.shape[0]
+        acc = opt.state(dev)
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        g = torch.empty(N_PARAMS, dtype=torch.float32, device=dev) if want_grad else None
+        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _check(lib().snk_qnet_group_train_step(self._g, _ptr(states, torch.float32, B * 200, dev), _ptr(actions, torch.uint8, B, dev),
+                                               _ptr(targets, torch.float64, B, dev), B, _ptr(acc, torch.float32, N_PARAMS, dev),
+                                               opt.eta, opt.rho, opt.epsilon, _ptr(g), _ptr(loss), st))
+        net._updated = True
+        return loss, g
+
+    def check(self):
+        """raises if a wait of this rank gave up on a peer (synchronises)"""
+        from . import _check, lib
+        t = C.c_int(0)
+        _check(lib().snk_qnet_group_status_host(self._g, C.byref(t)))
+
+    def close(self):
+        if getattr(self, "_g", None):
+            try:
+                from . import lib
+                lib().snk_qnet_group_destroy(self._g)
+            except Exception:          # interpreter shutdown
+                pass
+            self._g = None
+
+    __del__ = close
+
+
+class LocalLearnerGroup:
+    """R virtual ranks of a LearnerGroup in ONE process on ONE GPU (connect_local), each driven from its own stream: the
+    ranks order themselves on the device, so the host may enqueue them in any order.  For tests on a single B200."""
+
+    def __init__(self, nets):
+        from . import _check, lib
+        world = len(nets)
+        self.groups = [LearnerGroup(n, world, r) for r, n in enumerate(nets)]
+        self.streams = [torch.cuda.Stream(n.device) for n in nets]
+        arr = (C.c_void_p * world)(*[g._g.value for g in self.groups])
+        for g in self.groups:
+            _check(lib().snk_qnet_group_connect_local(g._g, arr, world))
+
+    def train_step(self, batches, opts, want_grad=False, order=None):
+        """batches[r] = (states, actions, targets) of rank r, opts[r] its RMSProp; the ranks are enqueued in `order` (default
+        0 .. R-1).  Returns [(loss, g)] per rank; the current stream waits for all of them."""
+        cur = torch.cuda.current_stream(self.groups[0].net.device)
+        out = [None] * len(self.groups)
+        for r in (range(len(self.groups)) if order is None else order):
+            s = self.streams[r]
+            s.wait_stream(cur)
+            with torch.cuda.stream(s):
+                out[r] = self.groups[r].train_step(*batches[r], opts[r], want_grad)
+        for s in self.streams:
+            cur.wait_stream(s)
+        return out
+
+    def check(self):
+        for g in self.groups:
+            g.check()
+
+    def close(self):
+        for g in self.groups:
+            g.close()
+
+
+class DistributedLearnerGroup(LearnerGroup):
+    """This process's rank of a LearnerGroup over torch.distributed (one process per GPU): the 64-byte handles travel through
+    all_gather_object once, the only thing torch.distributed is used for; updates need no communicator."""
+
+    def __init__(self, net, group=None):
+        import torch.distributed as dist
+        super().__init__(net, dist.get_world_size(group), dist.get_rank(group))
+        handles = [None] * self.world
+        dist.all_gather_object(handles, self.handle(), group=group)
+        self.connect(handles)
+
+
 class _ParamsView:
     """__cuda_array_interface__ of a QNet's device theta; keeps the net alive as long as a tensor views it."""
 
