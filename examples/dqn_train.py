@@ -9,8 +9,9 @@ utils.jl:408-412); --resume PATH continues a saved run bit for bit (load_trainer
 
 Started under torchrun (one process per GPU: python -m torch.distributed.run --nproc-per-node 8 examples/dqn_train.py) it
 trains one Q-net data-parallel (DESIGN §5f): every rank plays its own --envs games into its own replay ring and samples 64
-transitions from it, and every update is the update of all ranks' minibatches together.  Rank 0 reports; --save and
---resume take one file per rank (PATH.rank<r>).
+transitions from it, and every update is the update of all ranks' minibatches together.  With --shared-replay the ranks'
+minibatches are instead drawn together, uniformly without replacement from the union of all rings (DESIGN §5g), as the
+reference samples its one buffer.  Rank 0 reports; --save and --resume take one file per rank (PATH.rank<r>).
 """
 import argparse
 import os
@@ -30,8 +31,13 @@ def main():
     ap.add_argument("--precision", default="f32", choices=["f32", "bf16"])
     ap.add_argument("--report", type=int, default=1000)
     ap.add_argument("--window", type=int, default=1000, help="episodes in the moving average of the returns")
+    ap.add_argument("--capacity", type=int, default=50000, help="replay ring capacity per rank (the reference's 50,000)")
+    ap.add_argument("--shared-replay", action="store_true",
+                    help="under torchrun: draw each update's minibatch uniformly from the union of every rank's ring instead of "
+                         "64 from each rank's own; with R ranks, --capacity C/R per rank keeps the reference's C transitions in "
+                         "the union")
     ap.add_argument("--save", metavar="PATH", help="write a checkpoint of the run here at the end")
-    ap.add_argument("--resume", metavar="PATH", help="continue the run saved here (its --envs and --precision are the checkpoint's)")
+    ap.add_argument("--resume", metavar="PATH", help="continue the run saved here (its --envs, --capacity, --precision and --shared-replay are the checkpoint's)")
     args = ap.parse_args()
     S = graft.load_package()
     world, rank, dev = 1, 0, 0
@@ -46,8 +52,8 @@ def main():
         tr = S.train.Trainer.load(args.resume + suffix, device=dev, world=world, rank=rank)
         say("resumed %s: %d updates, %d transitions stored" % (args.resume, tr.n_updates, tr.stored))
     else:
-        tr = S.train.Trainer(n_envs=args.envs, device=dev, precision=args.precision, updates_per_step=args.updates_per_step,
-                             world=world, rank=rank)
+        tr = S.train.Trainer(n_envs=args.envs, device=dev, precision=args.precision, capacity=args.capacity,
+                             updates_per_step=args.updates_per_step, world=world, rank=rank, shared_replay=args.shared_replay)
     if world > 1:
         handles = [None] * world
         dist.all_gather_object(handles, tr.handle())
@@ -68,8 +74,10 @@ def main():
         tr.save(args.save + suffix)
         say("saved %s" % (args.save + suffix))
     if world > 1:
-        dist.barrier()                                   # no rank still waits on a peer's published sums
+        dist.barrier()                                   # no rank still waits on a peer's published sums or reads its ring
         tr.learner.check()
+        if tr.sampler is not None:
+            tr.sampler.check()
         dist.destroy_process_group()
 
 

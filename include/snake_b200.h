@@ -60,7 +60,7 @@ extern "C" {
 #define SNK_ERR_CUDA (-2)      /* a CUDA runtime call failed */
 #define SNK_ERR_NODEVICE (-3)  /* no CUDA device / not a Blackwell part */
 #define SNK_ERR_UNSUPPORTED (-4)
-#define SNK_ERR_TIMEOUT (-5)   /* a peer of the row-sharded Gram or of a learner group did not arrive in time */
+#define SNK_ERR_TIMEOUT (-5)   /* a peer of the row-sharded Gram, a learner group or a replay group did not arrive in time */
 
 /* snk_create flags */
 #define SNK_AUTO_RESET 1u      /* a lost env is re-initialised (a fresh SnakeGame(), utils.jl:199) after its terminal outputs */
@@ -270,6 +270,43 @@ SNK_API int snk_replay_bad_index_host(snk_replay r, int *flag);
 SNK_API int snk_replay_checkpoint_bytes(snk_replay r, size_t *bytes);
 SNK_API int snk_replay_save_host(snk_replay r, void *blob_host, size_t bytes);
 SNK_API int snk_replay_load_host(snk_replay r, const void *blob_host, size_t bytes, int64_t *first_bad_slot);
+/* ---- the replay group: one minibatch drawn uniformly from the union of the rings of a box (DESIGN §5g) ----------------
+ * A group has `world` ranks (1 .. 16), one snk_replay_group per rank, each wrapping that rank's ring.  batch_all[world]: every
+ * rank's share B_q >= 1 of the minibatch, fixed at create and the same on every rank, as is `seed`.
+ *   The union: the ranks' filled slots concatenated in rank order; union index u is slot u - (n_0 + ... + n_{q-1}) of rank q,
+ *   with n_q = min(stored, capacity) of ring q when its stream reaches the call.  n = n_0 + ... + n_{R-1}.
+ *   Call e (the group's draw counter, 0 at create) draws with key splitmix64(seed ^ splitmix64(e)), the key
+ *   snk_replay_sample_indices derives from a ring's draw counter, and rank r takes the counters [off_r, off_r + B_r) of that
+ *   permutation of [0, n), off_r = B_0 + ... + B_{r-1}.
+ * So the ranks' outputs concatenated in rank order equal, bit for bit, snk_replay_sample_indices(seed, B_0 + ... + B_{R-1})
+ * and snk_replay_gather on ONE full ring of capacity n that holds the ranks' filled records concatenated and whose draw counter
+ * is e; world = 1 is snk_replay_sample_indices + snk_replay_gather on the ring itself.
+ * snk_replay_group_sample writes this rank's B_r transitions in snk_replay_gather's layout, and idx_out (B_r int64) its global
+ * union indices; every output may be NULL.  Ranks order themselves on the device, on cuda_stream (no host synchronisation):
+ * the call waits until every ring is complete for call e, reads the records over peer memory, then waits until every rank has
+ * read, so the rank's next store into its ring cannot overwrite a slot a peer still reads.  Every rank must call sample the same
+ * number of times, and store into its ring only on the stream it samples on.  A call with B_0 + ... + B_{R-1} > n writes no
+ * output and sets the flag status_host reports as SNK_ERR_INVALID; a wait that gives up after ~20 s sets SNK_ERR_TIMEOUT
+ * (both flags stay set).  draws / set_draws: the draw counter, the only state of the group a checkpoint needs.
+ * Set-up as for snk_qnet_group: create -> export_host (128 bytes: the ring's IPC handle and the flag block's) -> [every rank's
+ * 128 bytes to every rank] -> connect_host(world x 128 bytes in rank order, own entry ignored); connect_local wires the groups
+ * of ONE process (virtual ranks on one GPU, each on its own stream).  The ring must outlive its group. */
+#define SNK_REPLAY_GROUP_HANDLE_BYTES 128
+typedef struct snk_replay_group_s *snk_replay_group;
+SNK_API int snk_replay_group_create(snk_replay_group *out, snk_replay r, int world, int rank, const int64_t *batch_all,
+                                    uint64_t seed);
+SNK_API int snk_replay_group_destroy(snk_replay_group g);
+SNK_API int snk_replay_group_export_host(snk_replay_group g, uint8_t *handle128);
+SNK_API int snk_replay_group_connect_host(snk_replay_group g, const uint8_t *handles_world_x_128, int n_handles);
+SNK_API int snk_replay_group_connect_local(snk_replay_group g, const snk_replay_group *peers, int n_peers);
+SNK_API int snk_replay_group_sample(snk_replay_group g, int64_t *idx_out, float *states, float *next_states, uint8_t *actions,
+                                    float *rewards, uint8_t *dones, uint8_t *mask, float *ep_return, int32_t *score,
+                                    void *cuda_stream);
+SNK_API int snk_replay_group_draws(snk_replay_group g, uint64_t *draws);
+SNK_API int snk_replay_group_set_draws(snk_replay_group g, uint64_t draws);
+/* *timed_out: a wait gave up on a peer (SNK_ERR_TIMEOUT); *too_few: a call found B_0 + ... + B_{R-1} > n (SNK_ERR_INVALID).
+ * Synchronises. */
+SNK_API int snk_replay_group_status_host(snk_replay_group g, int *timed_out, int *too_few);
 
 /* ---- Q-network forward  structs.jl:127-139; call sites utils.jl:165 (acting), 448 (t_net targets) -------------
  * Conv(3x3,2=>16,relu,pad 1) -> Conv(3x3,16=>32,relu,pad 1) -> Conv(6x6,32=>64,relu) -> flatten -> Dense(1600,64,relu)

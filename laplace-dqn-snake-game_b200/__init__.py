@@ -148,6 +148,12 @@ def lib():
         "snk_replay_gather": [vp, vp, i64, vp, vp, vp, vp, vp, vp, vp, vp, vp],
         "snk_replay_sample_indices": [vp, C.c_uint64, i64, vp, vp],
         "snk_replay_bad_index_host": [vp, C.POINTER(i32)],
+        "snk_replay_group_create": [C.POINTER(vp), vp, i32, i32, vp, C.c_uint64], "snk_replay_group_destroy": [vp],
+        "snk_replay_group_export_host": [vp, vp], "snk_replay_group_connect_host": [vp, vp, i32],
+        "snk_replay_group_connect_local": [vp, vp, i32],
+        "snk_replay_group_sample": [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp],
+        "snk_replay_group_draws": [vp, C.POINTER(C.c_uint64)], "snk_replay_group_set_draws": [vp, C.c_uint64],
+        "snk_replay_group_status_host": [vp, C.POINTER(i32), C.POINTER(i32)],
         "snk_qnet_create": [C.POINTER(vp), vp, i64, i32, i32], "snk_qnet_destroy": [vp],
         "snk_qnet_forward": [vp, vp, i64, vp, vp], "snk_qnet_precision": [vp, C.POINTER(i32)],
         "snk_qnet_overflow_host": [vp, C.POINTER(i32)], "snk_qnet_debug_timing": [vp, vp],
@@ -622,6 +628,20 @@ def gram(A, terms=3, block_k=0, splits=0):
     return GramPlan(A.shape[0], A.shape[1], A.device, splits).pack(A).gram(terms, block_k)
 
 
+def _stack_exp_out(B, dev, ep_stats):
+    """the output dict of stack_exp for B transitions"""
+    out = {"states": torch.empty(B, 2, 10, 10, dtype=torch.float32, device=dev),
+           "next_states": torch.empty(B, 2, 10, 10, dtype=torch.float32, device=dev),
+           "actions": torch.empty(B, dtype=torch.uint8, device=dev),
+           "rewards": torch.empty(B, dtype=torch.float32, device=dev),
+           "dones": torch.empty(B, dtype=torch.uint8, device=dev),
+           "mask": torch.empty(B, 3, dtype=torch.uint8, device=dev)}
+    if ep_stats:
+        out["ep_return"] = torch.empty(B, dtype=torch.float32, device=dev)
+        out["score"] = torch.empty(B, dtype=torch.int32, device=dev)
+    return out
+
+
 class ReplayBuffer:
     """ReplayBuffer (structs.jl:104-116) on the device: capacity 50,000, batch_size 64 by default.
 
@@ -679,15 +699,7 @@ class ReplayBuffer:
         """utils.jl:343-383 for the transitions at idx: dict(states, actions, rewards, next_states, dones, mask)"""
         B = idx.numel()
         dev = self.device
-        out = {"states": torch.empty(B, 2, 10, 10, dtype=torch.float32, device=dev),
-               "next_states": torch.empty(B, 2, 10, 10, dtype=torch.float32, device=dev),
-               "actions": torch.empty(B, dtype=torch.uint8, device=dev),
-               "rewards": torch.empty(B, dtype=torch.float32, device=dev),
-               "dones": torch.empty(B, dtype=torch.uint8, device=dev),
-               "mask": torch.empty(B, 3, dtype=torch.uint8, device=dev)}
-        if ep_stats:
-            out["ep_return"] = torch.empty(B, dtype=torch.float32, device=dev)
-            out["score"] = torch.empty(B, dtype=torch.int32, device=dev)
+        out = _stack_exp_out(B, dev, ep_stats)
         st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
         _check(lib().snk_replay_gather(self._r, _ptr(idx, torch.int64, B, dev), B, _ptr(out["states"]),
                                        _ptr(out["next_states"]), _ptr(out["actions"]), _ptr(out["rewards"]),
@@ -732,6 +744,140 @@ class ReplayBuffer:
             raise ValueError("batch_size cannot be greater than the capacity of the buffer.")
         _load_blob(lib().snk_replay_load_host, self._r, d)
         self.seed, self.batch_size = d["seed"], d["batch_size"]
+
+
+REPLAY_GROUP_HANDLE_BYTES = 128          # SNK_REPLAY_GROUP_HANDLE_BYTES
+
+
+class ReplayGroup:
+    """One rank of a replay group (snk_replay_group, DESIGN §5g): R ranks, each with its own ReplayBuffer, draw one minibatch
+    of batch_all[0] + ... + batch_all[R-1] transitions uniformly without replacement from the union of their rings, and rank r
+    receives its batch_all[r] of them.  The ranks' samples concatenated in rank order are, bit for bit, ReplayBuffer.sample() of
+    one full ring holding the ranks' records concatenated, with the group's seed and draw counter.  The ranks wait for each other
+    on the device.  Set-up: handle() on every rank, then connect(every rank's handle, in rank order).  The ring must outlive
+    the group."""
+
+    def __init__(self, replay, world, rank, batch_all, seed):
+        self.replay, self.world, self.rank, self.seed = replay, int(world), int(rank), int(seed)
+        self.batch_all = [int(b) for b in batch_all]
+        if len(self.batch_all) != self.world:
+            raise ValueError("batch_all needs one entry per rank")
+        self._g = C.c_void_p()
+        arr = (C.c_int64 * self.world)(*self.batch_all)
+        _check(lib().snk_replay_group_create(C.byref(self._g), replay._r, self.world, self.rank, arr, self.seed % 2 ** 64))
+
+    def handle(self):
+        """this rank's 128-byte handle (bytes), to be sent to every other rank"""
+        h = (C.c_uint8 * REPLAY_GROUP_HANDLE_BYTES)()
+        _check(lib().snk_replay_group_export_host(self._g, h))
+        return bytes(h)
+
+    def connect(self, handles):
+        """handles: every rank's handle() in rank order (this rank's own entry is ignored)"""
+        blob = b"".join(bytes(h) for h in handles)
+        _check(lib().snk_replay_group_connect_host(self._g, (C.c_uint8 * max(len(blob), 1)).from_buffer_copy(blob or b"\0"),
+                                                   len(handles)))
+
+    def sample(self, want_idx=False, ep_stats=False):
+        """this rank's batch_all[rank] transitions of the group's minibatch as stack_exp's dict (+ 'idx': their union indices,
+        int64, if want_idx).  Enqueued on the current stream; every rank must call it the same number of times."""
+        dev = self.replay.device
+        B = self.batch_all[self.rank]
+        out = _stack_exp_out(B, dev, ep_stats)
+        if want_idx:
+            out["idx"] = torch.empty(B, dtype=torch.int64, device=dev)
+        st = C.c_void_p(torch.cuda.current_stream(dev).cuda_stream)
+        _check(lib().snk_replay_group_sample(self._g, _ptr(out.get("idx")), _ptr(out["states"]), _ptr(out["next_states"]),
+                                             _ptr(out["actions"]), _ptr(out["rewards"]), _ptr(out["dones"]), _ptr(out["mask"]),
+                                             _ptr(out.get("ep_return")), _ptr(out.get("score")), st))
+        return out
+
+    @property
+    def draws(self):
+        """sample calls so far: call e draws with the key ReplayBuffer.sample_indices derives from a ring's e-th call"""
+        d = C.c_uint64(0)
+        _check(lib().snk_replay_group_draws(self._g, C.byref(d)))
+        return d.value
+
+    def check(self):
+        """raises if a wait of this rank gave up on a peer, or a call asked for more transitions than the union held
+        (synchronises)"""
+        t, f = C.c_int(0), C.c_int(0)
+        _check(lib().snk_replay_group_status_host(self._g, C.byref(t), C.byref(f)))
+
+    def state_dict(self):
+        """{'draws', 'seed', 'batch_all'}: the group's only state is its draw counter"""
+        return {"draws": self.draws, "seed": self.seed, "batch_all": list(self.batch_all)}
+
+    def load_state_dict(self, d):
+        """the draw counter of a state_dict() of a group with this seed and batch_all"""
+        if not isinstance(d, dict) or not isinstance(d.get("draws"), int) or d.get("seed") != self.seed \
+                or d.get("batch_all") != self.batch_all:
+            raise ValueError("a ReplayGroup state_dict of seed %d and batch_all %s with 'draws' is required" % (self.seed, self.batch_all))
+        if not 0 <= d["draws"] < 2 ** 64:
+            raise ValueError("draws must be 0 .. 2^64 - 1")
+        _check(lib().snk_replay_group_set_draws(self._g, d["draws"]))
+
+    def close(self):
+        if getattr(self, "_g", None):
+            try:
+                lib().snk_replay_group_destroy(self._g)
+            except Exception:          # interpreter shutdown
+                pass
+            self._g = None
+
+    __del__ = close
+
+
+def connect_local_replay(groups):
+    """wire the ReplayGroups of ONE process together as virtual ranks 0 .. R-1 (snk_replay_group_connect_local)"""
+    arr = (C.c_void_p * len(groups))(*[g._g.value for g in groups])
+    for g in groups:
+        _check(lib().snk_replay_group_connect_local(g._g, arr, len(groups)))
+
+
+class LocalReplayGroup:
+    """R virtual ranks of a ReplayGroup in ONE process on ONE GPU, each driven from its own stream: the ranks order themselves
+    on the device, so the host may enqueue them in any order.  For tests on a single B200."""
+
+    def __init__(self, replays, batch_all, seed):
+        world = len(replays)
+        self.groups = [ReplayGroup(rb, world, r, batch_all, seed) for r, rb in enumerate(replays)]
+        self.streams = [torch.cuda.Stream(rb.device) for rb in replays]
+        connect_local_replay(self.groups)
+
+    def sample(self, want_idx=False, ep_stats=False, order=None):
+        """every rank's sample(), enqueued in `order` (default 0 .. R-1); the current stream waits for all of them"""
+        cur = torch.cuda.current_stream(self.groups[0].replay.device)
+        out = [None] * len(self.groups)
+        for r in (range(len(self.groups)) if order is None else order):
+            s = self.streams[r]
+            s.wait_stream(cur)
+            with torch.cuda.stream(s):
+                out[r] = self.groups[r].sample(want_idx, ep_stats)
+        for s in self.streams:
+            cur.wait_stream(s)
+        return out
+
+    def check(self):
+        for g in self.groups:
+            g.check()
+
+    def close(self):
+        for g in self.groups:
+            g.close()
+
+
+class DistributedReplayGroup(ReplayGroup):
+    """This process's rank of a ReplayGroup over torch.distributed (one process per GPU): the 128-byte handles travel through
+    all_gather_object once; sample calls need no communicator."""
+
+    def __init__(self, replay, batch_all, seed, group=None):
+        import torch.distributed as dist
+        super().__init__(replay, dist.get_world_size(group), dist.get_rank(group), batch_all, seed)
+        handles = [None] * self.world
+        dist.all_gather_object(handles, self.handle(), group=group)
+        self.connect(handles)
 
 
 from . import shard  # noqa: E402,F401

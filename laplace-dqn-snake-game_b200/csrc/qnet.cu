@@ -45,6 +45,7 @@
 
 namespace snk {
 namespace qgrad {       // qnet_grads.cu
+int preload_sample_grads();
 int launch_sample_grads(const float *theta_dev, const float *states, const uint8_t *actions, const double *targets, long long B,
                         void *hi, void *lo, long long pitch, float *J, long long ldJ, float *loss, int sms, cudaStream_t st);
 }
@@ -1522,7 +1523,12 @@ int snk_qnet_group_create(snk_qnet_group *out, snk_qnet q, int world, int rank) 
         SNK_CUDA(cudaMemset(g->mem, 0, GROUP_OFF_SUM));
         SNK_CUDA(cudaMalloc((void **)&g->d_timed_out, sizeof(int)));
         SNK_CUDA(cudaMemset(g->d_timed_out, 0, sizeof(int)));
-        return SNK_OK;
+        // load the update's kernels now (module loading is lazy): a first launch while a peer wait of this process spins
+        // would block the host until that wait gives up
+        cudaFuncAttributes fa;
+        SNK_CUDA(cudaFuncGetAttributes(&fa, k_group_sync));
+        SNK_CUDA(cudaFuncGetAttributes(&fa, k_qnet_train_apply));
+        return qgrad::preload_sample_grads();
     };
     const int rc = build();
     if (rc != SNK_OK) {
@@ -1597,7 +1603,9 @@ int snk_qnet_group_train_step(snk_qnet_group g, const float *states, const uint8
     snk_qnet_s *q = g->q;
     cudaStream_t st = (cudaStream_t)cuda_stream;
     if (g->rows_cap < B_local) {
-        SNK_CUDA(cudaStreamSynchronize(st));
+        // only a buffer in use needs the wait: the first call must not block the host, whose stream may already wait on the
+        // device for a peer's call the same host thread has yet to enqueue (a replay group's sample, DESIGN §5g)
+        if (g->rows != nullptr) SNK_CUDA(cudaStreamSynchronize(st));
         if (g->rows) { SNK_CUDA(cudaFree(g->rows)); g->rows = nullptr; }
         if (g->row_loss) { SNK_CUDA(cudaFree(g->row_loss)); g->row_loss = nullptr; }
         g->rows_cap = 0;

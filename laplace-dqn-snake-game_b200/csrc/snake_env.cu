@@ -32,6 +32,7 @@
 #include <cuda.h>
 
 #include "common.h"
+#include "peer.h"
 #include "sm100.h"
 
 // how phase B stores the observation: 0 = st.global.cs (streaming), 1 = plain st.global (default), 2 = st.global.wt.
@@ -1077,39 +1078,27 @@ __global__ void k_masked_target(const float *q, const uint8_t *mask, const float
 
 // ---- replay ring: stack_exp (utils.jl:343-383) of the records at idx[0..B) ------------------------------
 // One CTA per 32 samples; the records' planes go to shared memory, then states (10,10,2,B) and next_states are
-// streamed out with the same nibble->float4 table as the step kernel.
+// streamed out with the same nibble->float4 table as the step kernel.  stage_record and expand_staged are the one definition
+// of the expansion, for one ring (k_replay_gather) and for the union of a replay group's rings (k_replay_group_gather).
 constexpr int GATHER_S = 32;
-__global__ void __launch_bounds__(128) k_replay_gather(const uint4 *__restrict__ ring, long long cap, const long long *__restrict__ idx,
-                                                       long long B, float *states, float *next_states, uint8_t *actions,
-                                                       float *rewards, uint8_t *dones, uint8_t *mask, float *ep_return,
-                                                       int32_t *score, int *bad_index) {
-    __shared__ __align__(16) uint32_t s_pl[GATHER_S * 24];        // per sample: 3 boards x (P0[4], P1[4])
-    __shared__ ObsTables s_tb;
-    const int tid = threadIdx.x;
-    const long long b0 = (long long)blockIdx.x * GATHER_S;
-    const int n_local = (B - b0) < GATHER_S ? (int)(B - b0) : GATHER_S;
-    fill_tables<SNK_OBS_F32>(s_tb, tid, 128);
-    // 4 threads per sample copy the 6 plane vectors + scalars
-    if (tid < n_local * 4) {
-        const int sl = tid >> 2, part = tid & 3;
-        long long i = idx[b0 + sl];
-        if (i < 0 || i >= cap) { *bad_index = 1; i = 0; }
-        const uint4 *rec = ring + i * REC_U4;
-        uint4 *dst = reinterpret_cast<uint4 *>(s_pl + sl * 24);
-        if (part < 3) { dst[2 * part] = rec[2 * part]; dst[2 * part + 1] = rec[2 * part + 1]; }
-        else {
-            const uint4 sc = rec[6];
-            const long long o = b0 + sl;
-            if (rewards) rewards[o] = __uint_as_float(sc.x);
-            if (actions) actions[o] = (uint8_t)(sc.y & 0xFF);
-            if (dones) dones[o] = (uint8_t)((sc.y >> 8) & 0xFF);
-            if (mask) { mask[3 * o] = (sc.y >> 16) & 1; mask[3 * o + 1] = (sc.y >> 17) & 1; mask[3 * o + 2] = (sc.y >> 18) & 1; }
-            if (ep_return) ep_return[o] = __uint_as_float(sc.z);
-            if (score) score[o] = (int32_t)sc.w;
-        }
+// 4 threads per sample (part 0..3) copy the 6 plane vectors of record `rec` to shared memory and write its scalars
+__device__ __forceinline__ void stage_record(uint32_t *s_pl, const uint4 *rec, int sl, int part, long long o, uint8_t *actions,
+                                             float *rewards, uint8_t *dones, uint8_t *mask, float *ep_return, int32_t *score) {
+    uint4 *dst = reinterpret_cast<uint4 *>(s_pl + sl * 24);
+    if (part < 3) { dst[2 * part] = rec[2 * part]; dst[2 * part + 1] = rec[2 * part + 1]; }
+    else {
+        const uint4 sc = rec[6];
+        if (rewards) rewards[o] = __uint_as_float(sc.x);
+        if (actions) actions[o] = (uint8_t)(sc.y & 0xFF);
+        if (dones) dones[o] = (uint8_t)((sc.y >> 8) & 0xFF);
+        if (mask) { mask[3 * o] = (sc.y >> 16) & 1; mask[3 * o + 1] = (sc.y >> 17) & 1; mask[3 * o + 2] = (sc.y >> 18) & 1; }
+        if (ep_return) ep_return[o] = __uint_as_float(sc.z);
+        if (score) score[o] = (int32_t)sc.w;
     }
-    __syncthreads();
-    // two outputs: states uses boards (0,1), next_states boards (1,2); 50 float4 units per sample each
+}
+// after the barrier: states uses boards (0,1), next_states boards (1,2); 50 float4 units per sample each
+__device__ __forceinline__ void expand_staged(const uint32_t *s_pl, const ObsTables &s_tb, int tid, long long b0, int n_local,
+                                              float *states, float *next_states) {
     const int total = n_local * 50;
 #pragma unroll 2
     for (int which = 0; which < 2; which++) {
@@ -1128,6 +1117,25 @@ __global__ void __launch_bounds__(128) k_replay_gather(const uint4 *__restrict__
         }
     }
 }
+__global__ void __launch_bounds__(128) k_replay_gather(const uint4 *__restrict__ ring, long long cap, const long long *__restrict__ idx,
+                                                       long long B, float *states, float *next_states, uint8_t *actions,
+                                                       float *rewards, uint8_t *dones, uint8_t *mask, float *ep_return,
+                                                       int32_t *score, int *bad_index) {
+    __shared__ __align__(16) uint32_t s_pl[GATHER_S * 24];        // per sample: 3 boards x (P0[4], P1[4])
+    __shared__ ObsTables s_tb;
+    const int tid = threadIdx.x;
+    const long long b0 = (long long)blockIdx.x * GATHER_S;
+    const int n_local = (B - b0) < GATHER_S ? (int)(B - b0) : GATHER_S;
+    fill_tables<SNK_OBS_F32>(s_tb, tid, 128);
+    if (tid < n_local * 4) {
+        const int sl = tid >> 2, part = tid & 3;
+        long long i = idx[b0 + sl];
+        if (i < 0 || i >= cap) { *bad_index = 1; i = 0; }
+        stage_record(s_pl, ring + i * REC_U4, sl, part, b0 + sl, actions, rewards, dones, mask, ep_return, score);
+    }
+    __syncthreads();
+    expand_staged(s_pl, s_tb, tid, b0, n_local, states, next_states);
+}
 
 // B distinct slots in [0, n): a keyed bijection of [0, 2^k) (4-round Feistel on k bits, k even) cycle-walked
 // into [0, n) and evaluated at counters 0..B-1 — sampling without replacement with no state and no rejection set.
@@ -1143,14 +1151,89 @@ __device__ __forceinline__ unsigned long long feistel_perm(unsigned long long x,
     }
     return (l << half_bits) | r;
 }
-__global__ void k_replay_sample(long long n, long long B, u64 key, long long *out) {
-    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= B) return;
+// the permutation of [0, n) keyed by `key`, at counter i
+__device__ __forceinline__ long long uniform_slot(long long n, long long i, u64 key) {
     int bits = 2;
     while ((1ll << bits) < n) bits += 2;
     unsigned long long x = (unsigned long long)i;
     do { x = feistel_perm(x, bits / 2, key); } while (x >= (unsigned long long)n);
-    out[i] = (long long)x;
+    return (long long)x;
+}
+__global__ void k_replay_sample(long long n, long long B, u64 key, long long *out) {
+    long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= B) return;
+    out[i] = uniform_slot(n, i, key);
+}
+
+// ---- replay group: one uniform minibatch over the union of R rings (snk_replay_group_*, DESIGN §5g) ----------------------
+// The flag block of a rank (one snk_ipc_alloc allocation, 64-bit words; rank q writes only the words of slot q):
+//   [RG_STORED + q]  the last sample call for which rank q's ring was complete (everything q's stream stored before the call)
+//   [RG_READ + q]    the last sample call rank q finished reading every ring for
+//   [RG_N + q]       n_q = the filled slots of rank q's ring at its last call (written before RG_STORED + q)
+// Call e on rank r's stream, three kernels:
+//   1. k_replay_group_flags(RG_STORED): store n_r into slot r of every rank's block, then e into RG_STORED + r (release, system
+//      scope, after everything the stream did before, including the step kernels that stored into the ring); wait until all R
+//      slots of the own block hold e (acquire).  Every record of every ring that the union of call e covers is then visible.
+//   2. k_replay_group_gather: the rank's counters of the permutation of the union, mapped to (rank, slot), read with peer loads.
+//   3. k_replay_group_flags(RG_READ): signal e into RG_READ + r of every block, wait for all R.  A rank's stream stores into its
+//      ring (the next step_fused_store) only after every rank has finished reading the rings for call e.
+// The n slots need no second buffer: rank q overwrites n_q (call e + 1) only after its step 3 of call e, so after every rank's
+// gather of call e has read it.
+constexpr int RG_STORED = 0, RG_READ = MAX_WORLD, RG_N = 2 * MAX_WORLD;
+constexpr size_t RG_FLAG_BYTES = 3 * MAX_WORLD * 8;
+
+struct RgPeers {
+    unsigned long long *flags[MAX_WORLD];
+    const uint4 *ring[MAX_WORLD];
+};
+
+// One CTA (see k_group_sync in qnet.cu: a spinning kernel of one CTA leaves the GPU to the other virtual ranks of a process).
+__global__ void k_replay_group_flags(RgPeers peers, const unsigned long long *mine, int world, int rank, int which, long long n_r,
+                                     unsigned long long epoch, int *timed_out) {
+    const int q = threadIdx.x;
+    if (q < world) {
+        if (which == RG_STORED) peers.flags[q][RG_N + rank] = (unsigned long long)n_r;
+        peer_signal(peers.flags[q] + which + rank, epoch);
+    }
+    __syncwarp();
+    if (q < world) peer_wait(mine + which + q, epoch, timed_out);
+}
+
+// Counters [off, off + B) of the permutation of the union (n = Σ n_q, as k_replay_sample for one ring of n), each union index
+// mapped to (rank q, slot) and its record expanded as k_replay_gather does.  A call with sum_B > n sets *too_few and writes
+// nothing (every thread sees the same n).
+__global__ void __launch_bounds__(128) k_replay_group_gather(RgPeers peers, const unsigned long long *mine, int world, long long off,
+                                                             long long B, long long sum_B, u64 key, long long *idx_out,
+                                                             float *states, float *next_states, uint8_t *actions,
+                                                             float *rewards, uint8_t *dones, uint8_t *mask, float *ep_return,
+                                                             int32_t *score, int *too_few) {
+    const long long *n_all = reinterpret_cast<const long long *>(mine + RG_N);
+    long long n = 0;
+    for (int q = 0; q < world; q++) n += n_all[q];
+    if (sum_B > n) {
+        if (blockIdx.x == 0 && threadIdx.x == 0) *too_few = 1;
+        return;
+    }
+    __shared__ __align__(16) uint32_t s_pl[GATHER_S * 24];
+    __shared__ ObsTables s_tb;
+    const int tid = threadIdx.x;
+    const long long b0 = (long long)blockIdx.x * GATHER_S;
+    const int n_local = (B - b0) < GATHER_S ? (int)(B - b0) : GATHER_S;
+    fill_tables<SNK_OBS_F32>(s_tb, tid, 128);
+    if (tid < n_local * 4) {
+        const int sl = tid >> 2, part = tid & 3;
+        long long s = uniform_slot(n, off + b0 + sl, key);
+        if (part == 3 && idx_out != nullptr) idx_out[b0 + sl] = s;
+        int q = 0;
+        while (s >= n_all[q]) s -= n_all[q++];
+        const uint4 *ring = peers.ring[0];
+#pragma unroll
+        for (int k = 1; k < MAX_WORLD; k++)      // a select, not an indexed read of the parameter (which would copy it to the stack)
+            if (k == q) ring = peers.ring[k];
+        stage_record(s_pl, ring + s * REC_U4, sl, part, b0 + sl, actions, rewards, dones, mask, ep_return, score);
+    }
+    __syncthreads();
+    expand_staged(s_pl, s_tb, tid, b0, n_local, states, next_states);
 }
 
 // ---- checkpoint validation (snk_env_load_host, snk_replay_load_host; DESIGN §5e) ----------------------------------------
@@ -1267,6 +1350,21 @@ struct snk_replay_s {
     int *d_bad;
     uint8_t *stage;          // device staging of snk_replay_gather_host
     size_t stage_bytes;
+};
+
+// one rank of a replay group (DESIGN §5g); the layout of `flags` is described at k_replay_group_flags
+struct snk_replay_group_s {
+    snk_replay_s *r;
+    int world, rank, device;
+    bool connected;
+    long long batch_all[MAX_WORLD];
+    long long off, sum_B;        // this rank's first counter, Σ batch_all
+    u64 seed, draws;             // the key of call e is splitmix64(seed ^ splitmix64(e)), e = draws before the call
+    unsigned long long calls;    // sample calls of this group object: the epoch of the flags (draws may be set back, calls not)
+    unsigned long long *flags;   // this rank's flag block (snk_ipc_alloc)
+    RgPeers peers;
+    void *opened[2 * MAX_WORLD]; // snk_ipc_import mappings to close
+    int *d_status;               // [0] a wait timed out, [1] a call asked for more transitions than the union held
 };
 
 static const uint8_t kDefaultFoodRC[100] = {  // Xoshiro(42) list, structs.jl:70 (pinned by tests/test_oracle_golden.py)
@@ -2006,6 +2104,153 @@ int snk_replay_bad_index_host(snk_replay r, int *flag) {
     SNK_REQUIRE(r != nullptr && flag != nullptr, "bad argument");
     DeviceGuard guard(r->device);
     SNK_CUDA(cudaMemcpy(flag, r->d_bad, sizeof(int), cudaMemcpyDeviceToHost));
+    return SNK_OK;
+}
+
+// ---- replay group: a uniform minibatch over the union of the rings of R ranks (DESIGN §5g) ------------------------------
+int snk_replay_group_create(snk_replay_group *out, snk_replay r, int world, int rank, const int64_t *batch_all, uint64_t seed) {
+    SNK_REQUIRE(out != nullptr, "null argument");
+    *out = nullptr;
+    SNK_REQUIRE(world >= 1 && world <= MAX_WORLD, "world must be 1 .. 16");
+    SNK_REQUIRE(rank >= 0 && rank < world, "rank must be 0 .. world - 1");
+    SNK_REQUIRE(r != nullptr && batch_all != nullptr, "null argument");
+    for (int q = 0; q < world; q++) SNK_REQUIRE(batch_all[q] >= 1 && batch_all[q] <= (1ll << 30), "batch_all entries must be 1 .. 2^30");
+    DeviceGuard guard(r->device);
+    snk_replay_group_s *g = new (std::nothrow) snk_replay_group_s();
+    if (g == nullptr) return fail(SNK_ERR_INVALID, "out of host memory");
+    g->r = r; g->world = world; g->rank = rank; g->device = r->device; g->seed = seed;
+    for (int q = 0; q < world; q++) {
+        g->batch_all[q] = batch_all[q];
+        if (q < rank) g->off += batch_all[q];
+        g->sum_B += batch_all[q];
+    }
+    auto build = [&]() -> int {
+        int rc;
+        if ((rc = snk_ipc_alloc((void **)&g->flags, RG_FLAG_BYTES)) != SNK_OK) return rc;
+        SNK_CUDA(cudaMemset(g->flags, 0, RG_FLAG_BYTES));
+        SNK_CUDA(cudaMalloc((void **)&g->d_status, 2 * sizeof(int)));
+        SNK_CUDA(cudaMemset(g->d_status, 0, 2 * sizeof(int)));
+        // load the call's kernels now (module loading is lazy): a first launch of the gather behind this rank's spinning flag
+        // kernel would block the host until the wait gives up
+        cudaFuncAttributes fa;
+        SNK_CUDA(cudaFuncGetAttributes(&fa, k_replay_group_flags));
+        SNK_CUDA(cudaFuncGetAttributes(&fa, k_replay_group_gather));
+        return SNK_OK;
+    };
+    const int rc = build();
+    if (rc != SNK_OK) {
+        snk_replay_group_destroy(g);
+        return rc;
+    }
+    g->peers.flags[rank] = g->flags;
+    g->peers.ring[rank] = r->ring;
+    g->connected = world == 1;
+    *out = g;
+    return SNK_OK;
+}
+
+int snk_replay_group_destroy(snk_replay_group g) {
+    if (g == nullptr) return SNK_OK;
+    DeviceGuard guard(g->device);
+    cudaDeviceSynchronize();
+    for (void *p : g->opened) if (p) snk_ipc_close(p);
+    if (g->flags) snk_ipc_free(g->flags);
+    if (g->d_status) cudaFree(g->d_status);
+    delete g;
+    return SNK_OK;
+}
+
+int snk_replay_group_export_host(snk_replay_group g, uint8_t *handle128) {
+    SNK_REQUIRE(g != nullptr && handle128 != nullptr, "null argument");
+    DeviceGuard guard(g->device);
+    int rc = snk_ipc_export(g->r->ring, handle128);
+    return rc != SNK_OK ? rc : snk_ipc_export(g->flags, handle128 + 64);
+}
+
+int snk_replay_group_connect_host(snk_replay_group g, const uint8_t *handles, int n_handles) {
+    SNK_REQUIRE(g != nullptr && handles != nullptr, "null argument");
+    SNK_REQUIRE(n_handles == g->world, "one handle per rank is needed");
+    SNK_REQUIRE(!g->connected || g->world == 1, "already connected");
+    DeviceGuard guard(g->device);
+    for (int q = 0; q < g->world; q++) {
+        if (q == g->rank) continue;
+        const uint8_t *h = handles + (size_t)q * SNK_REPLAY_GROUP_HANDLE_BYTES;
+        void *ring = nullptr, *flags = nullptr;
+        int rc = snk_ipc_import(h, &ring);
+        if (rc != SNK_OK) return rc;
+        g->opened[2 * q] = ring;
+        if ((rc = snk_ipc_import(h + 64, &flags)) != SNK_OK) return rc;
+        g->opened[2 * q + 1] = flags;
+        g->peers.ring[q] = (const uint4 *)ring;
+        g->peers.flags[q] = (unsigned long long *)flags;
+    }
+    g->connected = true;
+    return SNK_OK;
+}
+
+int snk_replay_group_connect_local(snk_replay_group g, const snk_replay_group *peers, int n_peers) {
+    SNK_REQUIRE(g != nullptr && peers != nullptr, "null argument");
+    SNK_REQUIRE(n_peers == g->world, "one group per rank is needed");
+    for (int q = 0; q < g->world; q++) {
+        const snk_replay_group_s *p = peers[q];
+        SNK_REQUIRE(p != nullptr && p->rank == q && p->world == g->world && p->device == g->device && p->seed == g->seed &&
+                        memcmp(p->batch_all, g->batch_all, sizeof(g->batch_all)) == 0,
+                    "peer list does not match");
+    }
+    SNK_REQUIRE(peers[g->rank] == g, "peer list does not match");
+    for (int q = 0; q < g->world; q++) {
+        g->peers.ring[q] = peers[q]->r->ring;
+        g->peers.flags[q] = peers[q]->flags;
+    }
+    g->connected = true;
+    return SNK_OK;
+}
+
+// publish n_r and wait for every ring -> draw and gather -> wait until every rank has read.  No host synchronisation.
+int snk_replay_group_sample(snk_replay_group g, int64_t *idx_out, float *states, float *next_states, uint8_t *actions,
+                            float *rewards, uint8_t *dones, uint8_t *mask, float *ep_return, int32_t *score, void *cuda_stream) {
+    SNK_REQUIRE(g != nullptr, "null group");
+    SNK_REQUIRE(g->connected, "group not connected (snk_replay_group_connect_host / connect_local)");
+    SNK_REQUIRE((((uintptr_t)states | (uintptr_t)next_states) & 15u) == 0, "state buffers must be 16-byte aligned");
+    DeviceGuard guard(g->device);
+    cudaStream_t st = (cudaStream_t)cuda_stream;
+    const snk_replay_s *r = g->r;
+    const long long n_r = r->total < r->capacity ? r->total : r->capacity;
+    const unsigned long long e = ++g->calls;
+    const u64 key = splitmix64(g->seed ^ splitmix64(g->draws++));
+    const long long B = g->batch_all[g->rank];
+    k_replay_group_flags<<<1, 32, 0, st>>>(g->peers, g->flags, g->world, g->rank, RG_STORED, n_r, e, g->d_status);
+    SNK_CUDA(cudaGetLastError());
+    k_replay_group_gather<<<nblocks(B, GATHER_S), 128, 0, st>>>(g->peers, g->flags, g->world, g->off, B, g->sum_B, key,
+                                                               (long long *)idx_out, states, next_states, actions, rewards,
+                                                               dones, mask, ep_return, score, g->d_status + 1);
+    SNK_CUDA(cudaGetLastError());
+    k_replay_group_flags<<<1, 32, 0, st>>>(g->peers, g->flags, g->world, g->rank, RG_READ, 0, e, g->d_status);
+    SNK_CUDA(cudaGetLastError());
+    return SNK_OK;
+}
+
+int snk_replay_group_draws(snk_replay_group g, uint64_t *draws) {
+    SNK_REQUIRE(g != nullptr && draws != nullptr, "null argument");
+    *draws = g->draws;
+    return SNK_OK;
+}
+
+int snk_replay_group_set_draws(snk_replay_group g, uint64_t draws) {
+    SNK_REQUIRE(g != nullptr, "null group");
+    g->draws = draws;
+    return SNK_OK;
+}
+
+int snk_replay_group_status_host(snk_replay_group g, int *timed_out, int *too_few) {
+    SNK_REQUIRE(g != nullptr && timed_out != nullptr && too_few != nullptr, "null argument");
+    DeviceGuard guard(g->device);
+    int st[2];
+    SNK_CUDA(cudaMemcpy(st, g->d_status, sizeof(st), cudaMemcpyDeviceToHost));
+    *timed_out = st[0];
+    *too_few = st[1];
+    if (st[0]) return fail(SNK_ERR_TIMEOUT, "snk_replay_group: a peer did not reach a sample call within ~20 s");
+    if (st[1]) return fail(SNK_ERR_INVALID, "snk_replay_group: a sample call asked for more transitions than the union of the rings held");
     return SNK_OK;
 }
 

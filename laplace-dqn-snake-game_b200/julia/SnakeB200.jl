@@ -14,7 +14,7 @@ export BatchedSnakeGame, available_actions, step!, step_fused!, virtual_step, as
        epsilon_greedy, masked_target, center_columns!, reset!, set_food_list!, score, lost,
        DeviceReplayBuffer, store_step!, store_step_host!, store_step_host_bits!, stack_exp, sample_indices, DeviceQNet, forward!, overflowed,
        sample_grads!, RMSPropState, train_step!, update_target_net!, params_device, store_snapshot!, gram!, sample_model_weights!, empty_buffer!, patch_reset_obs!,
-       GramShard, export_handle, connect!, run!, planes, LearnerGroup, check_peers,
+       GramShard, export_handle, connect!, run!, planes, LearnerGroup, check_peers, ReplayGroup, sample!,
        step_device!, step_abs_device!, step_fused_device!, rollout_device!, state_device!, losing_mask_device!,
        lost_device!, steps_device!, error_flags_device!, count_errors, seed!, set_stream!, num_envs, library_version,
        default_food_list, device_alloc, device_free, compression_supported, checkpoint, restore!
@@ -563,6 +563,49 @@ train_step!(g::LearnerGroup, opt::RMSPropState, d_states::Ptr{Float32}, d_action
 function check_peers(g::LearnerGroup)
     t = Ref{Cint}(0)
     check(ccall((:snk_qnet_group_status_host, lib), Cint, (Ptr{Cvoid}, Ref{Cint}), g.handle, t))
+end
+
+# ---- replay group: one minibatch drawn uniformly from the union of every rank's ring (DESIGN §5g) -------------------------
+"""Rank `rank` of a replay group of `world` ranks around the ring `r`.  `batch_all` (one share B_q >= 1 per rank) and `seed` are
+the same on every rank.  The ranks' `sample!` outputs concatenated in rank order are `sample_indices` + `stack_exp` of one
+full ring holding every rank's filled records, bit for bit.  `r` must outlive the group."""
+mutable struct ReplayGroup
+    handle::Ptr{Cvoid}
+    world::Int
+    r::DeviceReplayBuffer
+    function ReplayGroup(r::DeviceReplayBuffer, world::Integer, rank::Integer, batch_all::Vector{Int64}, seed::Integer)
+        length(batch_all) == world || throw(ArgumentError("batch_all needs one entry per rank"))
+        h = Ref{Ptr{Cvoid}}(C_NULL)
+        check(ccall((:snk_replay_group_create, lib), Cint, (Ref{Ptr{Cvoid}}, Ptr{Cvoid}, Cint, Cint, Ptr{Int64}, UInt64),
+                    h, r.handle, world, rank, batch_all, UInt64(seed)))
+        g = new(h[], world, r)
+        finalizer(x -> ccall((:snk_replay_group_destroy, lib), Cint, (Ptr{Cvoid},), x.handle), g)
+        return g
+    end
+end
+"""128 bytes to send to every other rank"""
+function export_handle(g::ReplayGroup)
+    h = Vector{UInt8}(undef, 128)
+    check(ccall((:snk_replay_group_export_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}), g.handle, h))
+    return h
+end
+"""`handles` = the 128-byte handles of ALL ranks, concatenated in rank order"""
+connect!(g::ReplayGroup, handles::Vector{UInt8}) =
+    check(ccall((:snk_replay_group_connect_host, lib), Cint, (Ptr{Cvoid}, Ptr{UInt8}, Cint), g.handle, handles, length(handles) ÷ 128))
+"""This rank's share of one group minibatch into device buffers in `stack_exp`'s layout (states / next_states (10,10,2,B)
+Float32, actions B UInt8 0-based, rewards B Float32, dones B UInt8, mask (3,B) UInt8; d_idx: the union indices, Int64).  Any
+may be C_NULL.  Enqueued on the default stream; every rank must call it the same number of times."""
+sample!(g::ReplayGroup, d_states::Ptr{Float32}, d_next_states::Ptr{Float32}, d_actions::Ptr{UInt8}, d_rewards::Ptr{Float32},
+        d_dones::Ptr{UInt8}, d_mask::Ptr{UInt8}; d_idx::Ptr{Int64} = Ptr{Int64}(C_NULL)) =
+    check(ccall((:snk_replay_group_sample, lib), Cint,
+                (Ptr{Cvoid}, Ptr{Int64}, Ptr{Float32}, Ptr{Float32}, Ptr{UInt8}, Ptr{Float32}, Ptr{UInt8}, Ptr{UInt8}, Ptr{Float32},
+                 Ptr{Int32}, Ptr{Cvoid}),
+                g.handle, d_idx, d_states, d_next_states, d_actions, d_rewards, d_dones, d_mask, Ptr{Float32}(C_NULL),
+                Ptr{Int32}(C_NULL), C_NULL))
+"""throws if a wait of this rank gave up on a peer, or a call asked for more transitions than the rings held (synchronises)"""
+function check_peers(g::ReplayGroup)
+    t = Ref{Cint}(0); f = Ref{Cint}(0)
+    check(ccall((:snk_replay_group_status_host, lib), Cint, (Ptr{Cvoid}, Ref{Cint}, Ref{Cint}), g.handle, t, f))
 end
 
 """`bytes` of device memory on `device` for the outputs of the fused step; with `compressible`, memory with generic L2

@@ -14,8 +14,11 @@ Data parallelism (DESIGN §5f): Trainer(world=R, rank=r) is rank r of R trainers
 games into its own replay ring (the ring's and the games' seeds are derived from (seed, rank)) and samples batch_size
 transitions from it; the update goes through a LearnerGroup, so every rank applies the same update: QNet.train_step of the
 R minibatches concatenated in rank order.  epsilon, the target-sync counter and the target net stay per rank and agree
-everywhere because θ does.  Deviation: the global minibatch is stratified over the ranks' rings, not uniform over their
-union.  Before the first update the ranks are connected: connect(every rank's handle()) or Trainer.connect_local.
+everywhere because θ does.  Deviation, unless shared_replay: the global minibatch is stratified over the ranks' rings, not
+uniform over their union.  With shared_replay=True (DESIGN §5g) the R x batch_size transitions of an update are drawn
+uniformly without replacement from the union of all ranks' rings (a ReplayGroup seeded with `seed`), as the reference's
+sample(rpb) draws from its one buffer, and rank r trains on its batch_size slice of them; at world 1 this is the run without
+it, bit for bit.  Before the first update the ranks are connected: connect(every rank's handle()) or Trainer.connect_local.
 
 Deviation from the reference: it plays one whole episode of one game per update; here one play is one Rollout.step(), which
 advances each of the N games by one step (and stores N transitions), followed by `updates_per_step` updates.  The ratio of
@@ -25,7 +28,7 @@ import ctypes as C
 
 import torch
 
-from . import ReplayBuffer, SnakeGame, _check, lib, masked_target
+from . import ReplayBuffer, ReplayGroup, SnakeGame, _check, connect_local_replay, lib, masked_target
 from .qnet import LearnerGroup, QNet, RMSProp, glorot_layers
 from .rollout import Rollout
 
@@ -40,7 +43,8 @@ def rank_seed(seed, rank):
 class Trainer:
     def __init__(self, n_envs=4096, device=0, layers=None, precision="f32", capacity=50000, batch_size=64, gamma=0.97,
                  eta=5e-4, rho=0.9, opt_epsilon=1e-8, epsilon=1.0, epsilon_min=0.05, epsilon_decay=1e-6,
-                 target_sync=1000, fill=50000, fill_epsilon=1.0, updates_per_step=1, seed=0, world=1, rank=0):
+                 target_sync=1000, fill=50000, fill_epsilon=1.0, updates_per_step=1, seed=0, world=1, rank=0,
+                 shared_replay=False):
         dev = torch.device("cuda", device)
         self.precision = precision
         self.world, self.rank = int(world), int(rank)
@@ -52,6 +56,9 @@ class Trainer:
         self.learner = LearnerGroup(self.q_net, self.world, self.rank) if self.world > 1 else None
         self.env = SnakeGame(n_envs, device=device, auto_reset=True, seed=rank_seed(ENV_SEED, self.rank))
         self.replay = ReplayBuffer(capacity, device, batch_size, rank_seed(seed, self.rank))
+        # shared_replay: the minibatch of an update is drawn from the union of every rank's ring, keyed by the run's seed
+        self.shared_replay = bool(shared_replay)
+        self.sampler = ReplayGroup(self.replay, self.world, self.rank, [batch_size] * self.world, seed) if self.shared_replay else None
         self.opt = RMSProp(eta, rho, opt_epsilon)
         self.rollout = Rollout(self.env, self.q_net, self.t_net, self.replay, epsilon=fill_epsilon)
         self.gamma, self.epsilon, self.epsilon_min, self.epsilon_decay = float(gamma), float(epsilon), float(epsilon_min), float(epsilon_decay)
@@ -63,21 +70,26 @@ class Trainer:
         self.returns = []              # per play: the returns (f32, device) of the episodes that finished in it
 
     def handle(self):
-        """this rank's learner-group handle (64 bytes), for connect() on every rank"""
-        return self.learner.handle()
+        """this rank's learner-group handle (64 bytes), followed with shared_replay by its replay-group handle (128 bytes), for
+        connect() on every rank"""
+        return self.learner.handle() + (self.sampler.handle() if self.sampler is not None else b"")
 
     def connect(self, handles):
         """every rank's handle() in rank order"""
-        self.learner.connect(handles)
+        self.learner.connect([h[:64] for h in handles])
+        if self.sampler is not None:
+            self.sampler.connect([h[64:] for h in handles])
 
     @staticmethod
     def connect_local(trainers):
         """wire the trainers of ONE process together as virtual ranks 0 .. R-1 on one GPU.  Each must be built and run with
-        its own stream current, and the host must not wait on one rank's stream before every rank has enqueued its update
-        (e.g. all ranks play, then all ranks update)."""
+        its own stream current, and the host must not wait on one rank's stream before every rank has enqueued its update and,
+        with shared_replay, its sample call (e.g. all ranks play, then all ranks update)."""
         arr = (C.c_void_p * len(trainers))(*[t.learner._g.value for t in trainers])
         for t in trainers:
             _check(lib().snk_qnet_group_connect_local(t.learner._g, arr, len(trainers)))
+        if trainers[0].sampler is not None:
+            connect_local_replay([t.sampler for t in trainers])
 
     def _play(self, epsilon):
         self.rollout.epsilon = epsilon
@@ -93,7 +105,7 @@ class Trainer:
 
     def update(self):
         """one minibatch update (utils.jl:442-480)"""
-        b = self.replay.sample()
+        b = self.sampler.sample() if self.sampler is not None else self.replay.sample()
         y = masked_target(self.t_net(b["next_states"]), b["mask"], b["rewards"], b["dones"], gamma=self.gamma)
         learner = self.learner if self.learner is not None else self.q_net
         loss, _ = learner.train_step(b["states"], b["actions"], y, self.opt)
@@ -131,7 +143,8 @@ class Trainer:
         dev = self.q_net.device
         return {
             "n_envs": self.env.n, "capacity": self.replay.capacity, "batch_size": self.replay.batch_size, "precision": self.precision,
-            "world": self.world, "rank": self.rank,
+            "world": self.world, "rank": self.rank, "shared_replay": self.shared_replay,
+            **({"replay_group": self.sampler.state_dict()} if self.sampler is not None else {}),
             **{k: getattr(self, k) for k in self._HYPER},
             "n_updates": self.n_updates, "stored": self.stored, "epsilon": self.epsilon,
             "losses": (torch.stack(self.losses) if self.losses else torch.empty(0, dtype=torch.float32, device=dev)).cpu(),
@@ -153,12 +166,18 @@ class Trainer:
         for k, default in self._RANK:
             if d.get(k, default) != getattr(self, k):
                 raise ValueError("checkpoint has %s = %r, this trainer %r" % (k, d.get(k, default), getattr(self, k)))
+        if bool(d.get("shared_replay", False)) != self.shared_replay:
+            raise ValueError("checkpoint has shared_replay = %r, this trainer %r" % (bool(d.get("shared_replay", False)), self.shared_replay))
+        if self.shared_replay and not isinstance(d.get("replay_group"), dict):
+            raise ValueError("a shared_replay checkpoint holds 'replay_group'")
         for k in ("losses", "returns"):
             if not isinstance(d[k], torch.Tensor) or d[k].dtype != torch.float32 or d[k].dim() != 1:
                 raise ValueError("%s must be a 1-d float32 tensor" % k)
         dev = self.q_net.device
         self.env.load_state_dict(d["env"])
         self.replay.load_state_dict(d["replay"])
+        if self.sampler is not None:
+            self.sampler.load_state_dict(d["replay_group"])
         self.q_net.load_state_dict(d["q_net"])
         self.t_net.load_state_dict(d["t_net"])
         self.opt.load_state_dict(d["opt"], dev)
@@ -175,19 +194,23 @@ class Trainer:
         torch.save(self.state_dict(), path)
 
     @classmethod
-    def load(cls, path, device=0, n_envs=None, capacity=None, batch_size=None, precision=None, world=None, rank=None):
+    def load(cls, path, device=0, n_envs=None, capacity=None, batch_size=None, precision=None, world=None, rank=None,
+             shared_replay=None):
         """A Trainer continuing the run saved at path (torch.load with weights_only=True).  n_envs, capacity, batch_size,
-        precision, world, rank: when given, a checkpoint with other values is refused (ValueError).  A rank of a group run
-        must then be connected again before its next update."""
+        precision, world, rank, shared_replay: when given, a checkpoint with other values is refused (ValueError).  A rank of a
+        group run must then be connected again before its next update."""
         d = torch.load(path, map_location="cpu", weights_only=True)
         if not isinstance(d, dict) or any(k not in d for k in cls._SHAPE):
             raise ValueError("%s is not a Trainer checkpoint" % path)
         got = {k: d[k] for k in cls._SHAPE}
-        got.update({k: d.get(k, default) for k, default in cls._RANK})
-        for k, want in zip(cls._SHAPE + ("world", "rank"), (n_envs, capacity, batch_size, precision, world, rank)):
+        got.update({k: d.get(k, default) for k, default in cls._RANK + (("shared_replay", False),)})
+        for k, want in zip(cls._SHAPE + ("world", "rank", "shared_replay"),
+                           (n_envs, capacity, batch_size, precision, world, rank, shared_replay)):
             if want is not None and got[k] != want:
                 raise ValueError("checkpoint has %s = %r, %r was asked for" % (k, got[k], want))
+        # the replay group's seed is fixed at create: the run's seed (everything else seed chose is replaced by the load)
+        seed = d["replay_group"].get("seed", 0) if got["shared_replay"] and isinstance(d.get("replay_group"), dict) else 0
         tr = cls(n_envs=d["n_envs"], device=device, precision=d["precision"], capacity=d["capacity"], batch_size=d["batch_size"],
-                 world=got["world"], rank=got["rank"])
+                 world=got["world"], rank=got["rank"], shared_replay=bool(got["shared_replay"]), seed=seed)
         tr.load_state_dict(d)
         return tr
